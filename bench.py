@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the NOVIC decoder hot path: labels/sec, greedy decode, batch 4096 per GPU (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A step = one greedy decode (prefix prefill + 15 autoregressive steps, KV-cached) of one batch of 4096 synthetic
@@ -41,7 +41,8 @@ UNIT = "labels/s"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="K: timed steps of the headline greedy decode and of each of its three end-to-end "
+                                                          "passes; the beam-search and training workloads time K clamped to 2..5 and 5..20 steps")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=("b200", "reference"))
     ap.add_argument("--batch", type=int, default=BATCH_PER_GPU, help="embeddings per GPU per step")
@@ -49,7 +50,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads (beam k=3, training step, image encoder + decoder)")
     ap.add_argument("--encoder-images", type=int, default=1024, help="images per GPU of the encoder + decoder workload (BASELINE config #5)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed greedy step returned (target ids, padding, scores; "
+                                                          "with one GPU also loss_sum, loss_basis) as DIR/<name>.npy, to compare two builds "
+                                                          "output for output; GPU arm only (not with --impl reference)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 def workload_config(args, world):
@@ -358,6 +367,28 @@ def traffic_entry(name: str):
     return json.load(open(path)).get(name)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Writes each tensor as path/<name>.npy: per-sequence arrays (leading dimension = the first array's) in float32, where token ids
+    below 2^24 and 0/1 padding flags are exact, and scalars in float64.  Outputs larger than DUMP_BYTES in all keep a fixed, seeded
+    sample of the sequences, whose indices go to path/rows.npy."""
+    import numpy as np
+    arrays = {name: t.cpu().to(torch.float32 if t.ndim else torch.float64).numpy() for name, t in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    per_seq = [name for name, a in arrays.items() if a.ndim and a.shape[0] == n]
+    row_bytes = sum(arrays[name].nbytes for name in per_seq) // n
+    fixed_bytes = sum(a.nbytes for name, a in arrays.items() if name not in per_seq)
+    if row_bytes * n + fixed_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=(DUMP_BYTES - fixed_bytes) // (row_bytes + 8), replace=False))
+        arrays.update({name: arrays[name][rows] for name in per_seq})
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def main():
     args = parse_args()
     if args.impl == "reference":
@@ -409,8 +440,8 @@ def main():
 
         def step_device():
             if world == 1:
-                tok, pad, _, _, _, score = model.generate(embed, False, True, 1.0, 0.0, None, None, False)
-                return tok, pad, score
+                tok, pad, _, loss_sum, loss_basis, score = model.generate(embed, False, True, 1.0, 0.0, None, None, False)
+                return tok, pad, score, loss_sum, loss_basis
             # sharded: decode and gather are enqueued without a host synchronisation; the one sync of the step reads the global early-exit length
             tok, pad, score, T = model.generate_async(embed, 1.0, 0.0)
             tok, pad, score, T = gather_generation_async(tok.unsqueeze(1), pad.unsqueeze(1), score.unsqueeze(1), B * world, G, T)
@@ -467,6 +498,8 @@ def main():
             sampler.wait_started()
             sampler.mark()
         total_ms, launches, out, dev_steps = timed(step_device, args.steps)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, dict(zip(("target", "target_padding", "target_score", "loss_sum", "loss_basis"), out)))
         # three passes of exactly K steps each; the median pass is reported (all three are in e2e.runs_ms): one host hiccup in a 60 ms
         # loop (page-in after the previous process, a scheduler tick) otherwise decides the headline
         e2e_runs = [run_e2e(args.steps) for _ in range(3)]

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA sm_100 device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the reference tree at /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: runs the unmodified reference itself; skips unless its source tree is found (oracle/refload.py)")
 
 
 def pytest_collection_modifyitems(config, items):

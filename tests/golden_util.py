@@ -10,6 +10,7 @@ import dataclasses
 
 GOLDEN_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_outputs.npz")
 VARIANTS_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_variants.npz")
+TWINS_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "live_twins.npz")
 B_GOLD = 32
 
 
@@ -22,6 +23,18 @@ class Golden:
 
     def has(self, key: str) -> bool:
         return key.replace("/", "__") in self._z.files
+
+
+def check_twin(prefix: str, got: dict) -> None:
+    """Compare values computed now with the `prefix__*` arrays of tests/golden/live_twins.npz (oracle/make_twin_golden.py): the same
+    keys, shapes and dtypes; floating-point arrays within 1e-6, everything else exactly."""
+    z = np.load(TWINS_PATH)
+    want = {k[len(prefix) + 2:]: z[k] for k in z.files if k.startswith(prefix + "__")}
+    assert want and set(got) == set(want), sorted(set(got) ^ set(want))[:10]
+    for k, v in got.items():
+        w = want[k]
+        assert v.shape == w.shape and v.dtype == w.dtype, (k, v.shape, w.shape, v.dtype, w.dtype)
+        assert np.allclose(v, w, rtol=0, atol=1e-6) if v.dtype.kind == "f" else np.array_equal(v, w), k
 
 
 def weight_case(tag: str, dims: synth.DecoderDims = synth.DecoderDims()) -> dict:

@@ -42,6 +42,38 @@ def test_gpu_arm_refuses_to_run_without_a_gpu():
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
 
 
+def test_dump_outputs_writes_float32_and_samples_large_outputs(tmp_path, monkeypatch):
+    """bench.dump_outputs: one .npy per output, per-sequence arrays in float32 and scalars (the loss totals) in float64; above
+    DUMP_BYTES the same seeded sequences of every per-sequence array, their indices, and the scalars whole."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    tok = torch.arange(40 * 15, dtype=torch.int64).view(40, 15)
+    pad = tok % 3 == 0
+    score = -torch.arange(40, dtype=torch.float32) / 7
+    loss_sum, loss_basis = torch.tensor(123.456, dtype=torch.float32), torch.tensor(401, dtype=torch.int64)
+    outputs = {"target": tok, "target_padding": pad, "target_score": score, "loss_sum": loss_sum, "loss_basis": loss_basis}
+    bench.dump_outputs(str(tmp_path / "all"), outputs)
+    got = {n: np.load(tmp_path / "all" / f"{n}.npy") for n in outputs}
+    assert {n: a.dtype for n, a in got.items()} == {"target": np.float32, "target_padding": np.float32, "target_score": np.float32,
+                                                    "loss_sum": np.float64, "loss_basis": np.float64}
+    assert not (tmp_path / "all" / "rows.npy").exists()
+    for n, t in outputs.items():
+        assert np.array_equal(got[n], t.to(torch.float64).numpy()), n
+    monkeypatch.setattr(bench, "DUMP_BYTES", 10 * (31 * 4 + 8) + 16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outputs)
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.dtype == np.float64 and len(rows) == 10 and np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    r = rows.astype(np.int64)
+    for n in ("target", "target_padding", "target_score"):
+        assert np.array_equal(np.load(tmp_path / "a" / f"{n}.npy"), outputs[n].to(torch.float32).numpy()[r]), n
+    for n in ("loss_sum", "loss_basis"):
+        assert np.load(tmp_path / "a" / f"{n}.npy") == outputs[n].item(), n
+    assert sum(os.path.getsize(tmp_path / "a" / f"{n}.npy") - 128 for n in (*outputs, "rows")) <= bench.DUMP_BYTES
+
+
 def test_roofline_entry_reports_the_binding_roof():
     """bench.roof_entry: a GEMM class is measured against the roof that takes longer for its algorithmic work; an HBM class against
     the HBM roof; fractions are work / time / peak."""

@@ -119,6 +119,25 @@ def test_header_struct_and_offsets_match_the_reference(tmp_path):
                                                                          rm.embed_stride, rm.total_size)
 
 
+def header_values() -> dict:
+    """What test_header_struct_and_offsets_match_the_reference compares: the header struct format, the magic bytes and, per cache file,
+    the eight section offsets / sizes of its layout."""
+    out = {"struct_format": np.array(cache.HEADER_STRUCT.format), "magic": np.frombuffer(cache.MAGIC, dtype=np.uint8).copy()}
+    for name in CASES:
+        raw = open(os.path.join(GOLDEN, f"cache_{name}.bin"), "rb").read(128)
+        lay = cache.CacheLayout.from_header(cache.CacheHeader.unpack(raw))
+        out[f"{name}__layout"] = np.array([lay.target_nouns_offset, lay.target_offset, lay.target_mask_offset, lay.embed_targets_offset,
+                                           lay.embed_target_weights_offset, lay.embed_offset, lay.embed_stride, lay.total_size], dtype=np.int64)
+    return out
+
+
+def test_header_struct_and_offsets_match_committed_reference_values():
+    """test_header_struct_and_offsets_match_the_reference without the reference tree: against the stored values that test asserts
+    equal to the reference's Header / Meta (tests/golden/live_twins.npz)."""
+    from tests.golden_util import check_twin
+    check_twin("cache", header_values())
+
+
 # ------------------------------------------------------------------------------------------------------------
 # GPU
 # ------------------------------------------------------------------------------------------------------------

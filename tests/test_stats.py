@@ -3,10 +3,12 @@ GenerationTask.update (infer.py:613-644) run on strings.  The reference detokeni
 test gives it an injective stand-in (the ids up to the end token, joined), for which string membership and id membership coincide."""
 import types
 
+import numpy as np
 import pytest
 import torch
 
 from novic_b200 import stats, synth
+from tests.golden_util import check_twin
 
 DIMS = synth.DecoderDims()
 G = DIMS.token_length - 1
@@ -63,6 +65,31 @@ def test_stats_match_reference_generation_task(use_classes):
         for name in ("topk", "topk_guide", "topk_vocab", "topk_invalid", "topk_valid"):
             assert torch.allclose(getattr(mine, name), getattr(task, name)), name
     assert mine.valid_guide.any() and mine.valid_vocab.any() and mine.invalid.any() and (not use_classes or mine.correct.any())
+
+
+STATS_FIELDS = ("valid_vocab", "valid_guide", "correct", "invalid", "result", "topk_counts", "topk", "topk_guide", "topk_vocab", "topk_invalid",
+                "topk_valid")
+
+
+def stats_values(use_classes: bool) -> dict:
+    """The counters test_stats_match_reference_generation_task compares, after each of its two batches: {"<batch>__<field>": array}."""
+    guide_t, vocab_t, classes, target, padding, class_idx = make_case()
+    K = target.shape[1]
+    mine = stats.GenerationStats(K, vocab_t, guide_t, G, DIMS.vocab_size, device="cpu", class_targets=classes if use_classes else None)
+    score = torch.zeros(target.shape[:2])
+    out = {}
+    for j, (lo, hi) in enumerate(((0, 16), (16, 40))):
+        mine.update(target[lo:hi], padding[lo:hi], score[lo:hi], class_indices=class_idx[lo:hi] if use_classes else None)
+        out.update({f"{j}__{f}": getattr(mine, f).numpy() for f in STATS_FIELDS})
+        out[f"{j}__num_samples"] = np.array(mine.num_samples, dtype=np.int64)
+    return out
+
+
+@pytest.mark.parametrize("use_classes", (False, True))
+def test_stats_match_committed_reference_values(use_classes):
+    """test_stats_match_reference_generation_task without the reference tree: the same inputs against the stored values of the
+    counters that test asserts equal to the reference's (tests/golden/live_twins.npz)."""
+    check_twin(f"stats__{int(use_classes)}", stats_values(use_classes))
 
 
 def test_membership_semantics_without_reference():

@@ -157,6 +157,52 @@ def test_formats_match_committed_reference_vectors(name):
             assert np.array_equal(decode_targets(out, tok, fmt).numpy(), z[f"{key}__b{bi}__raw"]), (sw, batch)
 
 
+def random_cases():
+    """The cases of test_random_vocabularies_match_the_reference_embedder, drawn from the same seeded stream in the same order:
+    (trial, case within the trial, tokenizer name, nouns, switch index, batch)."""
+    import random
+    rng = random.Random(1234)
+    for trial in range(25):
+        name = rng.choice(sorted(TOKENIZERS))
+        alphabet = rng.sample("abcdefghijklmnopqrstuvwxyz", rng.randint(1, 26))
+        nouns = tuple(dict.fromkeys("".join(rng.choice(alphabet) for _ in range(rng.randint(1, 12))) for _ in range(rng.randint(1, 30))))
+        for k, sw in enumerate(rng.sample(SWITCHES, 6)):
+            batch = tuple(rng.sample(nouns, rng.randint(1, len(nouns))))
+            yield trial, k, name, nouns, SWITCHES.index(sw), batch
+
+
+def random_vocabulary_values() -> dict:
+    """Per trial of random_cases(): the format fields, compact maps, encoded ids / mask and decoded ids that the live test asserts
+    equal to the reference Embedder's, packed into one int64 vector per trial (each case: switch index, vocab_size, start, end,
+    pad, token_length with None as -2^31, then map, unmap, ids, mask, decoded ids, each as ndim, shape, values or as -1 when
+    absent), and the trial's nouns and batches as words ("|" before each batch)."""
+    import numpy as np
+    none = -(2 ** 31)
+    ints, words = {}, {}
+    for trial, k, name, nouns, si, batch in random_cases():
+        spec = TOKENIZERS[name]
+        tok = _tok(spec)
+        fmt = make_target_format(*_raw(nouns, spec["start"], spec["end"], spec["pad"]), tok, **SWITCHES[si])
+        ids, mask = encode_targets(*_raw(batch, spec["start"], spec["end"], spec["pad"]), tok, fmt)
+        parts = [[si, fmt.vocab_size, none if fmt.start_token_id is None else fmt.start_token_id,
+                  none if fmt.end_token_id is None else fmt.end_token_id, fmt.pad_token_id, fmt.token_length]]
+        for t in (fmt.compact_map if fmt.compact_ids else None, fmt.compact_unmap if fmt.compact_ids else None, ids, mask,
+                  decode_targets(ids, tok, fmt)):
+            parts += [[-1]] if t is None else [[t.ndim, *t.shape], t.flatten().tolist()]
+        ints.setdefault(trial, []).extend(v for p in parts for v in p)
+        words.setdefault(trial, list(nouns)).extend(("|",) + batch)
+    out = {f"{t}__ints": np.array(v, dtype=np.int64) for t, v in ints.items()}
+    out.update({f"{t}__words": np.array(v) for t, v in words.items()})
+    return out
+
+
+def test_random_vocabularies_match_committed_reference_values():
+    """test_random_vocabularies_match_the_reference_embedder without the reference tree: the same seeded cases against the stored
+    values that test asserts equal to the reference Embedder's (tests/golden/live_twins.npz)."""
+    from tests.golden_util import check_twin
+    check_twin("rand", random_vocabulary_values())
+
+
 def test_random_vocabularies_match_the_reference_embedder(ref):
     """Seeded random noun lists (1-12 letters from random alphabets, duplicates of letters, single-noun lists) and random switch
     choices against the live reference."""

@@ -260,6 +260,47 @@ size_t novic_vit_workspace_bytes(const NovicVitHandle* h, int64_t images_per_chu
 int novic_vit_encode(NovicVitHandle* h, const float* images, int64_t B, float* embed_out, int32_t normalize, int64_t images_per_chunk,
                      void* ws, size_t ws_bytes, void* stream);
 
+/* The reference's default embedder, open_clip `ViT-B-16-SigLIP` (config/train.yaml:126; architecture assumed as in DESIGN.md §5d):
+ * timm `vit_base_patch16_siglip_224` - patch convolution with bias, learned positions, no class token, `layers` pre-LN blocks (heads
+ * of 64 channels, exact erf GELU), final LayerNorm on all tokens, MAP attention-pool head; out_dim = width.  novic_siglip_create and
+ * novic_siglip_set_weights fill the same NovicVitHandle, so novic_vit_destroy / _weight_bytes / _workspace_bytes / _encode serve both
+ * models.  All parameters fp32 device pointers named after open_clip's state dict (`visual.trunk.*`). */
+typedef struct NovicSiglipCfg {
+  int32_t image_size;   /* 224 */
+  int32_t patch_size;   /* 16  */
+  int32_t width;        /* 768 = heads * 64 = out_dim */
+  int32_t layers;       /* 12 */
+  int32_t heads;        /* 12 */
+  int32_t mlp_dim;      /* 3072 (blocks and head MLP) */
+  float ln_eps;         /* 1e-6 */
+} NovicSiglipCfg;
+typedef struct NovicSiglipWeights {
+  const float *patch_w, *patch_b;     /* visual.trunk.patch_embed.proj.{weight,bias}  [width, 3, patch, patch], [width] */
+  const float* pos_embed;             /* visual.trunk.pos_embed                       [1, tokens, width] */
+  const float *norm_w, *norm_b;       /* visual.trunk.norm.{weight,bias} */
+  const float* pool_latent;           /* visual.trunk.attn_pool.latent                [1, 1, width] */
+  const float *pool_q_w, *pool_q_b;   /* ...attn_pool.q.{weight,bias}                 [width, width], [width] */
+  const float *pool_kv_w, *pool_kv_b; /* ...attn_pool.kv.{weight,bias}                [2 width, width], [2 width] (k first) */
+  const float *pool_proj_w, *pool_proj_b;   /* ...attn_pool.proj.{weight,bias}        [width, width], [width] */
+  const float *pool_norm_w, *pool_norm_b;   /* ...attn_pool.norm.{weight,bias} */
+  const float *pool_fc1_w, *pool_fc1_b;     /* ...attn_pool.mlp.fc1.{weight,bias}     [mlp_dim, width], [mlp_dim] */
+  const float *pool_fc2_w, *pool_fc2_b;     /* ...attn_pool.mlp.fc2.{weight,bias}     [width, mlp_dim], [width] */
+  const float* norm1_w[NOVIC_VIT_MAX_LAYERS];    /* visual.trunk.blocks.i.norm1.weight */
+  const float* norm1_b[NOVIC_VIT_MAX_LAYERS];
+  const float* qkv_w[NOVIC_VIT_MAX_LAYERS];      /* ...attn.qkv.weight       [3 width, width] */
+  const float* qkv_b[NOVIC_VIT_MAX_LAYERS];      /* ...attn.qkv.bias         [3 width] */
+  const float* proj_w[NOVIC_VIT_MAX_LAYERS];     /* ...attn.proj.weight      [width, width] */
+  const float* proj_b[NOVIC_VIT_MAX_LAYERS];
+  const float* norm2_w[NOVIC_VIT_MAX_LAYERS];    /* ...norm2.weight */
+  const float* norm2_b[NOVIC_VIT_MAX_LAYERS];
+  const float* fc1_w[NOVIC_VIT_MAX_LAYERS];      /* ...mlp.fc1.weight        [mlp_dim, width] */
+  const float* fc1_b[NOVIC_VIT_MAX_LAYERS];
+  const float* fc2_w[NOVIC_VIT_MAX_LAYERS];      /* ...mlp.fc2.weight        [width, mlp_dim] */
+  const float* fc2_b[NOVIC_VIT_MAX_LAYERS];
+} NovicSiglipWeights;
+int novic_siglip_create(const NovicSiglipCfg* cfg, NovicVitHandle** out);
+int novic_siglip_set_weights(NovicVitHandle* h, const NovicSiglipWeights* w, void* wbuf, size_t wbuf_bytes, void* stream);
+
 /* Building-block check used by the test-suite: out[M, N] fp32 = A[M, K] (bf16) * W[N, K]^T (bf16) through the
  * same tcgen05 / TMA kernel the decoder uses.  K % 64 == 0. */
 int novic_debug_gemm(const void* a_bf16, const void* w_bf16, float* out, int32_t M, int32_t N, int32_t K,

@@ -58,6 +58,19 @@ class NovicVitWeights(C.Structure):
                                                         "fc_w", "fc_b", "cproj_w", "cproj_b")]
 
 
+class NovicSiglipCfg(C.Structure):
+    _fields_ = [("image_size", C.c_int32), ("patch_size", C.c_int32), ("width", C.c_int32), ("layers", C.c_int32), ("heads", C.c_int32),
+                ("mlp_dim", C.c_int32), ("ln_eps", C.c_float)]
+
+
+class NovicSiglipWeights(C.Structure):
+    _fields_ = [(name, _FP) for name in ("patch_w", "patch_b", "pos_embed", "norm_w", "norm_b", "pool_latent", "pool_q_w", "pool_q_b",
+                                         "pool_kv_w", "pool_kv_b", "pool_proj_w", "pool_proj_b", "pool_norm_w", "pool_norm_b",
+                                         "pool_fc1_w", "pool_fc1_b", "pool_fc2_w", "pool_fc2_b")] + [
+        (name, _FP * NOVIC_VIT_MAX_LAYERS) for name in ("norm1_w", "norm1_b", "qkv_w", "qkv_b", "proj_w", "proj_b", "norm2_w", "norm2_b",
+                                                        "fc1_w", "fc1_b", "fc2_w", "fc2_b")]
+
+
 class NovicAdamW(C.Structure):
     _fields_ = [("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float), ("weight_decay", C.c_float),
                 ("max_grad_norm", C.c_float), ("step", C.c_int64)]
@@ -103,6 +116,8 @@ SIGNATURES = {
     "novic_vit_set_weights": (C.c_int, [C.c_void_p, C.POINTER(NovicVitWeights), C.c_void_p, C.c_size_t, C.c_void_p]),
     "novic_vit_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int64]),
     "novic_vit_encode": (C.c_int, [C.c_void_p, _FP, C.c_int64, _FP, C.c_int32, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "novic_siglip_create": (C.c_int, [C.POINTER(NovicSiglipCfg), C.POINTER(C.c_void_p)]),
+    "novic_siglip_set_weights": (C.c_int, [C.c_void_p, C.POINTER(NovicSiglipWeights), C.c_void_p, C.c_size_t, C.c_void_p]),
     "novic_set_dropout": (C.c_int, [C.c_void_p, C.c_float, C.c_float, C.c_uint64]),
     "novic_noise_apply": (C.c_int, [C.POINTER(NovicNoiseCfg), _FP, C.c_int64, C.c_uint64, C.c_uint64, C.c_void_p]),
     "novic_noise_apply_predrawn": (C.c_int, [C.POINTER(NovicNoiseCfg), _FP, C.c_int64, _FP, _FP, _FP, _FP, C.c_void_p]),

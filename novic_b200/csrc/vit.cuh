@@ -5,6 +5,16 @@
 // QuickGELU MLP, biases on every linear, LayerNorm (weight + bias, eps 1e-5) before the blocks and on the class token after them,
 // bias-free 1280 -> 1024 projection.  Parity is pinned only on an independent torch restatement (oracle/vit_oracle.py).
 //
+// The same kernels also run the reference's DEFAULT embedder, open_clip `ViT-B-16-SigLIP` (config/train.yaml:126), whose definition is
+// equally un-vendored, so its architecture is an ASSUMPTION too (open_clip's TimmModel around timm `vit_base_patch16_siglip_224`,
+// timm_pool 'map', timm_proj 'none', as remembered): a 16 x 16 patch convolution WITH bias on 224 x 224 images (14 x 14 = 196 tokens, no
+// class token) plus a learned pos_embed, no ln_pre; 12 pre-LN blocks of width 768 (qkv [2304, 768] + bias laid out q; k; v, 12 heads of 64,
+// scale 1/8, no mask; MLP 768 -> 3072 -> 768 with biases and the exact erf GELU of timm's nn.GELU - big_vision's original uses the tanh
+// approximation); LayerNorm with weight + bias, eps 1e-6; the final `norm` on all tokens; then the MAP head (timm AttentionPoolLatent):
+// q = q_proj(latent) (image independent), k, v = kv(x) ([1536, 768] + bias, k first), o = softmax(q k^T / 8) v per head (one query over
+// the 196 keys), y = proj(o), y += fc2(GELU(fc1(norm(y)))); the output is y (768), no projection after it.  Parameter names follow
+// open_clip (`visual.trunk.*`); parity is pinned only on tests/siglip_oracle.py:encode_image_siglip.
+//
 // The dense contractions (patch embedding, QKV, out-proj, both MLP layers: 99 % of the FLOPs outside attention) run on the persistent
 // tcgen05 / TMEM / TMA GEMM of gemm.cuh through the epilogues below; attention (730 keys x 80 channels per head) runs on
 // mma.sync.m16n8k16 tiles with an online softmax (flash-style: scores never leave the registers).
@@ -15,20 +25,25 @@
 
 namespace novic {
 
-constexpr int kVitHeadDim = 80;
+constexpr int kVitHeadDim = 80;       // open_clip ViT-H/14 heads (the legacy mma.sync attention is built for this one)
+constexpr int kSiglipHeadDim = 64;    // SigLIP ViT-B/16 heads
+
+// activation of EpiVitBias
+constexpr int kVitActNone = 0, kVitActQuickGelu = 1, kVitActGelu = 2;
 
 // ---------------------------------------------------------------------------------------------------------
 // GEMM epilogues (persistent gemm_kernel: 8 epilogue warps, thread = output row, 64 columns per thread)
 // ---------------------------------------------------------------------------------------------------------
 
-// out[row, n] = act(acc + bias[n]) as bf16 (QKV: no activation; MLP c_fc: QuickGELU x * sigmoid(1.702 x))
+// out[row, n] = act(acc + bias[n]) as bf16 (QKV: no activation; MLP c_fc: QuickGELU x * sigmoid(1.702 x) for open_clip's ViT-H,
+// the erf GELU for SigLIP)
 struct EpiVitBias {
   struct Params {
     __nv_bfloat16* out;
     int ld;                 // elements per output row
     const float* bias;      // [N] or nullptr
     int n_valid;            // N (columns >= N of the last tile are not stored)
-    int quick_gelu;
+    int act;                // kVitActNone / kVitActQuickGelu / kVitActGelu
     int direct;             // != 0: rows stored straight from the registers with 256-bit stores (ld must be a multiple of 16 elements)
   };
   template <class Release>
@@ -51,9 +66,12 @@ struct EpiVitBias {
             v[q * 4] += b.x; v[q * 4 + 1] += b.y; v[q * 4 + 2] += b.z; v[q * 4 + 3] += b.w;
           }
         }
-        if (p.quick_gelu) {
+        if (p.act == kVitActQuickGelu) {
 #pragma unroll
           for (int j = 0; j < 32; ++j) v[j] = v[j] * __fdividef(1.0f, 1.0f + __expf(-1.702f * v[j]));
+        } else if (p.act == kVitActGelu) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) v[j] = gelu_fast(v[j]);
         }
         if (p.direct) {
           // thread = row: 32 columns are 64 contiguous bytes of the row = two full 32-byte sectors (st.global.v8.b32); no staging tile
@@ -86,8 +104,9 @@ struct EpiVitBias {
 
 // Residual / patch-embedding epilogue on the fp32 token stream x [images * T, W] (row-major):
 //   residual mode (table == nullptr):  x[row, n] += acc + bias[n]                                  (attention out-proj, MLP c_proj)
-//   patch mode    (table != nullptr):  x[img * T + 1 + p, n] = acc + table[(1 + p) * W + n]        (conv1 as a GEMM over patches + positions;
-//                                      GEMM row = img * (T - 1) + p)
+//   patch mode    (table != nullptr):  x[img * T + tok0 + p, n] = acc + table[(tok0 + p) * W + n] + bias[n]
+//                                      (conv1 as a GEMM over patches + positions; GEMM row = img * (T - tok0) + p; tok0 = 1 behind a
+//                                      class token, 0 without one)
 // The thread = row accumulator chunk goes through a warp-private XOR-swizzled fp32 tile so that every global access covers 4 rows x 128
 // contiguous bytes.
 struct EpiVitResid {
@@ -96,8 +115,9 @@ struct EpiVitResid {
     int ld;                 // W
     const float* bias;      // [W] or nullptr
     const float* table;     // patch mode: positional embedding [T, W]
-    int patches;            // patch mode: T - 1
+    int patches;            // patch mode: T - tok0
     int n_valid;            // W (columns >= W of a ragged last tile are not touched)
+    int tok0;               // patch mode: token index of the first patch (1 with a class token, 0 without)
   };
   template <class Release>
   __device__ static __forceinline__ void run(const Params& p, const EpiCtx& c, Release release) {
@@ -124,8 +144,8 @@ struct EpiVitResid {
           if (row < c.M) {
             if (p.table != nullptr) {
               const int img = row / p.patches, pp = row - img * p.patches;
-              dst[i] = p.x + (static_cast<size_t>(img) * (p.patches + 1) + 1 + pp) * p.ld + col;
-              base[i] = __ldg(reinterpret_cast<const float4*>(p.table + static_cast<size_t>(1 + pp) * p.ld + col));
+              dst[i] = p.x + (static_cast<size_t>(img) * (p.patches + p.tok0) + p.tok0 + pp) * p.ld + col;
+              base[i] = __ldg(reinterpret_cast<const float4*>(p.table + static_cast<size_t>(p.tok0 + pp) * p.ld + col));
             } else {
               dst[i] = p.x + static_cast<size_t>(row) * p.ld + col;
               base[i] = *reinterpret_cast<const float4*>(dst[i]);
@@ -155,11 +175,13 @@ struct EpiVitResid {
   }
 };
 
-// out[row, n] = acc (fp32, row-major): the final 1280 -> 1024 projection of the class-token rows (B rows only)
+// out[row, n] = acc (+ bias[n]) (fp32, row-major): ViT-H's final 1280 -> 1024 projection of the class-token rows, SigLIP's MAP-head
+// `proj` (B rows only)
 struct EpiVitStoreF32 {
   struct Params {
     float* out;
     int ld;
+    const float* bias;      // [ld] or nullptr
   };
   template <class Release>
   __device__ static __forceinline__ void run(const Params& p, const EpiCtx& c, Release release) {
@@ -169,8 +191,16 @@ struct EpiVitStoreF32 {
       float v[32];
       tmem_ld_32x32(c.tmem_row + ch * 32, v);
       if (ch == nch - 1) release();
-      if (c.row < c.M && c.n0 + ch * 32 < p.ld) {
-        float4* d = reinterpret_cast<float4*>(p.out + static_cast<size_t>(c.row) * p.ld + c.n0 + ch * 32);
+      const int col0 = c.n0 + ch * 32;
+      if (c.row < c.M && col0 < p.ld) {
+        if (p.bias != nullptr) {
+#pragma unroll
+          for (int q = 0; q < 8; ++q) {
+            const float4 b = __ldg(reinterpret_cast<const float4*>(p.bias + col0) + q);
+            v[q * 4] += b.x; v[q * 4 + 1] += b.y; v[q * 4 + 2] += b.z; v[q * 4 + 3] += b.w;
+          }
+        }
+        float4* d = reinterpret_cast<float4*>(p.out + static_cast<size_t>(c.row) * p.ld + col0);
 #pragma unroll
         for (int q = 0; q < 8; ++q) d[q] = make_float4(v[q * 4], v[q * 4 + 1], v[q * 4 + 2], v[q * 4 + 3]);
       }
@@ -472,13 +502,17 @@ __global__ void __launch_bounds__(kVaWarps * 32, 2) vit_attention_kernel(const V
 // so the tensor core computes the next scores while the softmax warps work), warps 2..9 = softmax / correction / epilogue (two warps per
 // scheduler: with one, every dependent instruction of the exponential chain waits out its own latency - 473 us against ... for this kernel).
 // ---------------------------------------------------------------------------------------------------------
+//
+// The kernel is a template on the head dimension D: D = 80 (ViT-H) as above; D = 64 (SigLIP) takes Q and K as one 64-channel k-block each,
+// S in four k-slices, Vᵀ tiles of 64 rows, O with N = 64, and the four 16-column O chunks split 2 / 2 between the two softmax halves.
 constexpr int kTaQ = 128, kTaK = 128;
 constexpr int kTaStages = 3;                              // K / V^T ring: a tile's load (~2 k cycles) overlaps two tiles of work
-constexpr int kTaQBytes = 2 * kABytes;                    // Q: two k-blocks of 128 rows x 128 B
-constexpr int kTaKBytes = 2 * kABytes;                    // K tile: the same
-constexpr int kTaVBytes = 2 * kVitHeadDim * 128;          // V^T tile: two k-blocks (64 keys each) of 80 rows x 128 B
+template <int D> constexpr int kTaQBytes = ((D + 63) / 64) * kABytes;   // Q: 128 rows x 128 B per 64-channel k-block (D = 80: two)
+template <int D> constexpr int kTaKBytes = kTaQBytes<D>;                // K tile: the same
+template <int D> constexpr int kTaVBytes = 2 * D * 128;                 // V^T tile: two k-blocks (64 keys each) of D rows x 128 B
 constexpr int kTaPBytes = 2 * kABytes;                    // P: 128 rows x 128 keys bf16
-constexpr int kTaSmemBytes = kTaQBytes + kTaStages * (kTaKBytes + kTaVBytes) + kTaPBytes + 1024 /*align*/ + 256 /*barriers*/ + 3 * 2 * 128 * 4 /*row exchange*/;   // 224.3 KB
+template <int D>
+constexpr int kTaSmemBytes = kTaQBytes<D> + kTaStages * (kTaKBytes<D> + kTaVBytes<D>) + kTaPBytes + 1024 /*align*/ + 256 /*barriers*/ + 3 * 2 * 128 * 4 /*row exchange*/;   // D = 80: 224.3 KB
 constexpr int kTaSoftWarps = 8;                            // two per TMEM lane quadrant: each thread owns one query row x 64 of the tile's 128 keys
 constexpr int kTaThreads = 64 + 32 * kTaSoftWarps;
 
@@ -508,14 +542,16 @@ __global__ void __launch_bounds__(256) vit_vt_kernel(const __nv_bfloat16* __rest
   }
 }
 
+template <int D>
 __global__ void __launch_bounds__(kTaThreads, 1)
 vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_vt, const VitAttnTcParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;
-  uint8_t* sK = sQ + kTaQBytes;                            // [kTaStages]
-  uint8_t* sV = sK + kTaStages * kTaKBytes;                // [kTaStages]
-  uint8_t* sP = sV + kTaStages * kTaVBytes;
+  constexpr int kQBytes = kTaQBytes<D>, kKBytes = kTaKBytes<D>, kVBytes = kTaVBytes<D>;
+  uint8_t* sK = sQ + kQBytes;                              // [kTaStages]
+  uint8_t* sV = sK + kTaStages * kKBytes;                  // [kTaStages]
+  uint8_t* sP = sV + kTaStages * kVBytes;
   uint64_t* bars = reinterpret_cast<uint64_t*>(sP + kTaPBytes);
   uint64_t* q_full = bars;                                 // 1
   uint64_t* q_empty = bars + 1;                            // 1: every Q K^T of the item has been executed
@@ -560,38 +596,38 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       int g = 0, it = 0;
       for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++it) {
         const int qt = item % qtiles, head = (item / qtiles) % p.heads, img = item / (qtiles * p.heads);
-        // Q: channels [head * 80, +128) of the image's token rows (rows >= T are out of bounds: zero)
+        // Q: channels [head * D, +64 per k-block) of the image's token rows (rows >= T are out of bounds: zero)
         mbar_wait(q_empty, (it & 1) ^ 1, 1);
-        mbar_arrive_expect_tx(q_full, kTaQBytes);
-        tma_load_3d_at(sQ, &tm_qkv, q_full, head * kVitHeadDim, qt * kTaQ, img, kEvictNormal);
-        tma_load_3d_at(sQ + kABytes, &tm_qkv, q_full, head * kVitHeadDim + 64, qt * kTaQ, img, kEvictNormal);
+        mbar_arrive_expect_tx(q_full, kQBytes);
+        tma_load_3d_at(sQ, &tm_qkv, q_full, head * D, qt * kTaQ, img, kEvictNormal);
+        if (D > 64) tma_load_3d_at(sQ + kABytes, &tm_qkv, q_full, head * D + 64, qt * kTaQ, img, kEvictNormal);
         for (int t = 0; t < ntiles; ++t, ++g) {
           const int st = g % kTaStages;
           mbar_wait(&kv_empty[st], ((g / kTaStages) & 1) ^ 1, 1);
-          mbar_arrive_expect_tx(&kv_full[st], kTaKBytes + kTaVBytes);
-          uint8_t* k = sK + st * kTaKBytes;
-          uint8_t* v = sV + st * kTaVBytes;
-          tma_load_3d_at(k, &tm_qkv, &kv_full[st], W + head * kVitHeadDim, t * kTaK, img, kEvictLast);
-          tma_load_3d_at(k + kABytes, &tm_qkv, &kv_full[st], W + head * kVitHeadDim + 64, t * kTaK, img, kEvictLast);
-          tma_load_3d_at(v, &tm_vt, &kv_full[st], t * kTaK, head * kVitHeadDim, img, kEvictLast);
-          tma_load_3d_at(v + kVitHeadDim * 128, &tm_vt, &kv_full[st], t * kTaK + 64, head * kVitHeadDim, img, kEvictLast);
+          mbar_arrive_expect_tx(&kv_full[st], kKBytes + kVBytes);
+          uint8_t* k = sK + st * kKBytes;
+          uint8_t* v = sV + st * kVBytes;
+          tma_load_3d_at(k, &tm_qkv, &kv_full[st], W + head * D, t * kTaK, img, kEvictLast);
+          if (D > 64) tma_load_3d_at(k + kABytes, &tm_qkv, &kv_full[st], W + head * D + 64, t * kTaK, img, kEvictLast);
+          tma_load_3d_at(v, &tm_vt, &kv_full[st], t * kTaK, head * D, img, kEvictLast);
+          tma_load_3d_at(v + D * 128, &tm_vt, &kv_full[st], t * kTaK + 64, head * D, img, kEvictLast);
         }
       }
     }
   } else if (warp == 1) {
     if (elect_one()) {
       constexpr uint32_t kIdescS = umma_idesc_bf16_f32(kTaQ, kTaK);
-      constexpr uint32_t kIdescO = umma_idesc_bf16_f32(kTaQ, kVitHeadDim);
+      constexpr uint32_t kIdescO = umma_idesc_bf16_f32(kTaQ, D);
       // Q K^T of global tile gq (scores buffer gq & 1)
       auto issue_qk = [&](int gq) {
         const int st = gq % kTaStages, sb = gq & 1;
         mbar_wait(&kv_full[st], (gq / kTaStages) & 1, 2);
         mbar_wait(&s_empty[sb], ((gq >> 1) & 1) ^ 1, 3);           // the softmax warps have read the previous scores of this buffer
         tc_fence_after_sync();
-        const uint32_t a = smem_u32(sQ), b = smem_u32(sK + st * kTaKBytes);
+        const uint32_t a = smem_u32(sQ), b = smem_u32(sK + st * kKBytes);
         const uint32_t d = tmem_base + kColS + sb * kTaK;
 #pragma unroll
-        for (int k = 0; k < kVitHeadDim / kUmmaK; ++k) {            // 4 slices of k-block 0, 1 of k-block 1
+        for (int k = 0; k < D / kUmmaK; ++k) {                      // 4 slices of k-block 0 (D = 80: and 1 of k-block 1)
           const uint32_t off = (k >> 2) * kABytes + (k & 3) * (kUmmaK * 2);
           umma_bf16_ss(d, umma_desc_sw128_kmajor(a + off), umma_desc_sw128_kmajor(b + off), kIdescS, k != 0 ? 1u : 0u);
         }
@@ -607,11 +643,11 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
           else umma_commit(q_empty);                                // the item's last Q K^T has been issued: Q may be replaced once they are done
           mbar_wait(p_full, g & 1, 5);                              // P(t) is in shared memory, O has been rescaled
           tc_fence_after_sync();
-          const uint32_t a = smem_u32(sP), b = smem_u32(sV + st * kTaVBytes);
+          const uint32_t a = smem_u32(sP), b = smem_u32(sV + st * kVBytes);
 #pragma unroll
           for (int k = 0; k < kTaK / kUmmaK; ++k) {
             const uint32_t offa = (k >> 2) * kABytes + (k & 3) * (kUmmaK * 2);
-            const uint32_t offb = (k >> 2) * (kVitHeadDim * 128) + (k & 3) * (kUmmaK * 2);
+            const uint32_t offb = (k >> 2) * (D * 128) + (k & 3) * (kUmmaK * 2);
             umma_bf16_ss(tmem_base + kColO, umma_desc_sw128_kmajor(a + offa), umma_desc_sw128_kmajor(b + offb), kIdescO, (t | k) != 0 ? 1u : 0u);
           }
           umma_commit(&kv_empty[st]);
@@ -626,7 +662,8 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
     const int r = quad * 32 + lane;                                 // query row inside the tile
     const uint32_t tlane = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
     const float c = p.scale_log2e;
-    const int oc0 = half == 0 ? 0 : 3, oc1 = half == 0 ? 3 : kVitHeadDim / 16;   // 16-column chunks of O this warp rescales / stores
+    constexpr int kOSplit = (D / 16 + 1) / 2;                       // D = 80: chunks 0-2 | 3-4; D = 64: 0-1 | 2-3
+    const int oc0 = half == 0 ? 0 : kOSplit, oc1 = half == 0 ? kOSplit : D / 16;   // 16-column chunks of O this warp rescales / stores
     int g = 0, it = 0;
     for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++it) {
       const int qt = item % qtiles, head = (item / qtiles) % p.heads, img = item / (qtiles * p.heads);
@@ -711,7 +748,7 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       tc_fence_after_sync();
       asm volatile("bar.sync 2, 256;\n" ::: "memory");
       const float inv = 1.0f / (l_run + xl[(half ^ 1) * 128 + r]);
-      __nv_bfloat16* so = reinterpret_cast<__nv_bfloat16*>(sP) + r * (kVitHeadDim + 8);
+      __nv_bfloat16* so = reinterpret_cast<__nv_bfloat16*>(sP) + r * (D + 8);
 #pragma unroll 1
       for (int ch = oc0; ch < oc1; ++ch) {
         float ov[16];
@@ -722,15 +759,15 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
                                                                  pack_bf16x2(ov[12] * inv, ov[13] * inv), pack_bf16x2(ov[14] * inv, ov[15] * inv));
       }
       asm volatile("bar.sync 1, 256;\n" ::: "memory");                 // both halves of every row are staged
-      // each warp copies 16 rows: 16 rows x 10 chunks of 16 B
-      constexpr int kChunks = kVitHeadDim / 8;
-      __nv_bfloat16* dst = p.out + static_cast<size_t>(img) * T * W + head * kVitHeadDim;
+      // each warp copies 16 rows: 16 rows x D / 8 chunks of 16 B
+      constexpr int kChunks = D / 8;
+      __nv_bfloat16* dst = p.out + static_cast<size_t>(img) * T * W + head * D;
       const int row0 = quad * 32 + half * 16;
-      const __nv_bfloat16* sw = reinterpret_cast<const __nv_bfloat16*>(sP) + row0 * (kVitHeadDim + 8);
+      const __nv_bfloat16* sw = reinterpret_cast<const __nv_bfloat16*>(sP) + row0 * (D + 8);
       for (int i = lane; i < 16 * kChunks; i += 32) {
         const int rr = i / kChunks, cc = i - rr * kChunks;
         const int row = q0 + row0 + rr;
-        if (row < T) *reinterpret_cast<uint4*>(dst + static_cast<size_t>(row) * W + cc * 8) = *reinterpret_cast<const uint4*>(sw + rr * (kVitHeadDim + 8) + cc * 8);
+        if (row < T) *reinterpret_cast<uint4*>(dst + static_cast<size_t>(row) * W + cc * 8) = *reinterpret_cast<const uint4*>(sw + rr * (D + 8) + cc * 8);
       }
       // the staging rows overlap the P rows of other warps: nobody writes the next item's P before everyone has copied
       asm volatile("bar.sync 1, 256;\n" ::: "memory");
@@ -739,6 +776,95 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
   tc_fence_before_sync();
   __syncthreads();
   if (warp == 1) tmem_dealloc<512>(tmem_base);
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// SigLIP MAP head (timm AttentionPoolLatent)
+// ---------------------------------------------------------------------------------------------------------
+// q[n] = latent . Wq[n, :] + bq[n] (fp32, once per set of weights: the latent query is the same for every image).  One warp per output.
+__global__ void __launch_bounds__(256) siglip_latent_q_kernel(const float* __restrict__ latent, const float* __restrict__ wq, const float* __restrict__ bq,
+                                                              float* __restrict__ q, int W) {
+  const int n = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (n >= W) return;
+  const float* wr = wq + static_cast<size_t>(n) * W;
+  float s = 0.f;
+  for (int k = lane; k < W; k += 32) s = fmaf(__ldg(latent + k), __ldg(wr + k), s);
+  s = warp_sum(s);
+  if (lane == 0) q[n] = s + __ldg(bq + n);
+}
+
+// out[img, h * 64 + c] = softmax_t(q_h . k_t / 8) v_t[c] over the T tokens of one image (bf16 out, fp32 throughout).
+// kv: bf16 [images * T, 2 W] (k | v, head h at columns h * 64).  One warp per (image, head): lanes in four groups of eight, each group
+// one key (or value) row per step = 128 contiguous bytes, each lane 8 channels; scores go through the warp's T floats of shared memory.
+constexpr int kMapWarps = 4;
+constexpr int kMapMaxTokens = 3072;       // the scores of kMapWarps warps stay within the 48 KB of default dynamic shared memory
+__global__ void __launch_bounds__(kMapWarps * 32) siglip_map_attention_kernel(const __nv_bfloat16* __restrict__ kv, const float* __restrict__ q,
+                                                                              __nv_bfloat16* __restrict__ out, int T, int W, int heads, int items, float scale_log2e) {
+  extern __shared__ float sm_map[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int item = blockIdx.x * kMapWarps + warp;
+  if (item >= items) return;
+  const int img = item / heads, head = item - img * heads;
+  const int grp = lane >> 3, c0 = (lane & 7) * 8;
+  float* sc = sm_map + warp * T;
+  const __nv_bfloat16* krow = kv + static_cast<size_t>(img) * T * 2 * W + head * kSiglipHeadDim + c0;
+  const __nv_bfloat16* vrow = krow + W;
+  float qv[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) qv[j] = __ldg(q + head * kSiglipHeadDim + c0 + j) * scale_log2e;   // scores in log2 units
+  for (int t0 = 0; t0 < T; t0 += 4) {
+    const int t = t0 + grp;
+    float s = 0.f;
+    if (t < T) {
+      const uint4 u = __ldg(reinterpret_cast<const uint4*>(krow + static_cast<size_t>(t) * 2 * W));
+      const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float2 f = __bfloat1622float2(h2[j]);
+        s = fmaf(qv[2 * j], f.x, fmaf(qv[2 * j + 1], f.y, s));
+      }
+    }
+    s += __shfl_xor_sync(0xffffffffu, s, 1);
+    s += __shfl_xor_sync(0xffffffffu, s, 2);
+    s += __shfl_xor_sync(0xffffffffu, s, 4);
+    if ((lane & 7) == 0 && t < T) sc[t] = s;
+  }
+  __syncwarp();
+  float m = -INFINITY;
+  for (int t = lane; t < T; t += 32) m = fmaxf(m, sc[t]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  float l = 0.f;
+  for (int t = lane; t < T; t += 32) {
+    const float e = exp2f(sc[t] - m);
+    sc[t] = e;
+    l += e;
+  }
+  l = warp_sum(l);
+  __syncwarp();
+  float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int t = grp; t < T; t += 4) {
+    const float pt = sc[t];
+    const uint4 u = __ldg(reinterpret_cast<const uint4*>(vrow + static_cast<size_t>(t) * 2 * W));
+    const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float2 f = __bfloat1622float2(h2[j]);
+      acc[2 * j] = fmaf(pt, f.x, acc[2 * j]);
+      acc[2 * j + 1] = fmaf(pt, f.y, acc[2 * j + 1]);
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], 8);
+    acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], 16);
+  }
+  if (grp == 0) {
+    const float inv = 1.0f / l;
+    *reinterpret_cast<uint4*>(out + static_cast<size_t>(img) * W + head * kSiglipHeadDim + c0) =
+        make_uint4(pack_bf16x2(acc[0] * inv, acc[1] * inv), pack_bf16x2(acc[2] * inv, acc[3] * inv), pack_bf16x2(acc[4] * inv, acc[5] * inv),
+                   pack_bf16x2(acc[6] * inv, acc[7] * inv));
+  }
 }
 
 // embed[b, :] /= ||embed[b, :]|| (fp32; embedders.py:764).  One warp per row.

@@ -262,16 +262,20 @@ int novic_vit_encode(NovicVitHandle* h, const float* images, int64_t B, float* e
 
 /* The reference's default embedder, open_clip `ViT-B-16-SigLIP` (config/train.yaml:126; architecture assumed as in DESIGN.md §5d):
  * timm `vit_base_patch16_siglip_224` - patch convolution with bias, learned positions, no class token, `layers` pre-LN blocks (heads
- * of 64 channels, exact erf GELU), final LayerNorm on all tokens, MAP attention-pool head; out_dim = width.  novic_siglip_create and
+ * of 64 channels, exact erf GELU), final LayerNorm on all tokens, MAP attention-pool head; out_dim = width.  The same structs describe
+ * open_clip `ViT-SO400M-14-SigLIP` (timm `vit_so400m_patch14_siglip_224`, the F = 1152 checkpoints' embedder, assumed to be the same
+ * architecture): patch 14, width 1152, 27 blocks, 16 heads of 72, mlp_dim 4304.  Accepted: width / heads = 64 or 72, width 640, 768,
+ * 1024, 1152 or 1280, mlp_dim a multiple of 16 (the library pads the MLPs to whole 128-channel k-stages with zero weights; the
+ * weight and workspace sizes include the padding).  novic_siglip_create and
  * novic_siglip_set_weights fill the same NovicVitHandle, so novic_vit_destroy / _weight_bytes / _workspace_bytes / _encode serve both
  * models.  All parameters fp32 device pointers named after open_clip's state dict (`visual.trunk.*`). */
 typedef struct NovicSiglipCfg {
   int32_t image_size;   /* 224 */
   int32_t patch_size;   /* 16  */
-  int32_t width;        /* 768 = heads * 64 = out_dim */
-  int32_t layers;       /* 12 */
-  int32_t heads;        /* 12 */
-  int32_t mlp_dim;      /* 3072 (blocks and head MLP) */
+  int32_t width;        /* 768 = heads * 64 = out_dim (SO400M: 1152 = heads * 72) */
+  int32_t layers;       /* 12 (SO400M: 27) */
+  int32_t heads;        /* 12 (SO400M: 16) */
+  int32_t mlp_dim;      /* 3072 (blocks and head MLP; SO400M: 4304) */
   float ln_eps;         /* 1e-6 */
 } NovicSiglipCfg;
 typedef struct NovicSiglipWeights {

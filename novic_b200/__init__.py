@@ -10,6 +10,7 @@ Public surface (mirrors the reference's classes for this path):
   serve.GenerationPipeline                - double-buffered host -> device -> host inference loop
   ImageEncoder, VitDims                   - CLIP ViT-H/14 image encoder (open_clip `visual.*` parameters)
   SiglipImageEncoder, SiglipDims          - SigLIP ViT-B/16 image encoder, the reference's default embedder (`visual.trunk.*` parameters)
+  SIGLIP_SO400M                           - SiglipDims of SigLIP SO400M/14, the image encoder of the F = 1152 checkpoints
   EncoderDecoder                          - either encoder feeding the decoder on the device (greedy and beam search)
   optim.FusedAdamW, dist.train_step       - training step: fused clip + AdamW, overlapped gradient all-reduce
 """
@@ -17,11 +18,11 @@ from .decoder import EmbeddingDecoder, ParamCount, PrefixedIterDecoder
 from .noise import (AngleNoise, EmbeddingNoise, GaussAngleNoise, GaussElemNoise, GaussElemUniformAngleNoise, GaussVecNoise,
                     UniformAngleNoise)
 from .factory import DEFAULT_DECODER_KWARGS, default_decoder, register
-from .encoder import EncoderDecoder, ImageEncoder, SiglipDims, SiglipImageEncoder, VitDims
+from .encoder import SIGLIP_SO400M, EncoderDecoder, ImageEncoder, SiglipDims, SiglipImageEncoder, VitDims
 from . import cache, stats, synth, targets
 
 __all__ = [
     "EmbeddingDecoder", "ParamCount", "PrefixedIterDecoder", "EmbeddingNoise", "AngleNoise", "GaussAngleNoise", "GaussElemNoise",
     "GaussElemUniformAngleNoise", "GaussVecNoise", "UniformAngleNoise", "DEFAULT_DECODER_KWARGS", "default_decoder", "register", "synth", "cache", "stats", "targets", "ImageEncoder", "EncoderDecoder", "VitDims",
-    "SiglipImageEncoder", "SiglipDims",
+    "SiglipImageEncoder", "SiglipDims", "SIGLIP_SO400M",
 ]

@@ -15,6 +15,13 @@
 // the 196 keys), y = proj(o), y += fc2(GELU(fc1(norm(y)))); the output is y (768), no projection after it.  Parameter names follow
 // open_clip (`visual.trunk.*`); parity is pinned only on tests/siglip_oracle.py:encode_image_siglip.
 //
+// open_clip `ViT-SO400M-14-SigLIP` (the image embedder of the F = 1152 checkpoints) is assumed to be the same architecture at other
+// dimensions (TimmModel around timm `vit_so400m_patch14_siglip_224`, timm_pool 'map', timm_proj 'none', equally un-vendored): a 14 x 14
+// patch convolution with bias on 224 x 224 images (16 x 16 = 256 tokens, no class token), 27 blocks of width 1152 with 16 heads of 72
+// (scale 1/sqrt(72)), MLP 1152 -> 4304 -> 1152 with the exact erf GELU in the blocks and in the MAP head, LayerNorm eps 1e-6, the final
+// norm on all tokens, the MAP head, output 1152 wide, the same `visual.trunk.*` names.  The GEMMs read K in 64-channel k-blocks, so the
+// 4304-wide MLP runs padded to 4352 (zero fc1 rows and bias, zero fc2 columns: GELU(0) = 0 keeps the padded hidden columns exact zeros).
+//
 // The dense contractions (patch embedding, QKV, out-proj, both MLP layers: 99 % of the FLOPs outside attention) run on the persistent
 // tcgen05 / TMEM / TMA GEMM of gemm.cuh through the epilogues below; attention (730 keys x 80 channels per head) runs on
 // mma.sync.m16n8k16 tiles with an online softmax (flash-style: scores never leave the registers).
@@ -27,6 +34,7 @@ namespace novic {
 
 constexpr int kVitHeadDim = 80;       // open_clip ViT-H/14 heads (the legacy mma.sync attention is built for this one)
 constexpr int kSiglipHeadDim = 64;    // SigLIP ViT-B/16 heads
+constexpr int kSo400mHeadDim = 72;    // SigLIP SO400M/14 heads
 
 // activation of EpiVitBias
 constexpr int kVitActNone = 0, kVitActQuickGelu = 1, kVitActGelu = 2;
@@ -503,13 +511,18 @@ __global__ void __launch_bounds__(kVaWarps * 32, 2) vit_attention_kernel(const V
 // scheduler: with one, every dependent instruction of the exponential chain waits out its own latency - 473 us against ... for this kernel).
 // ---------------------------------------------------------------------------------------------------------
 //
-// The kernel is a template on the head dimension D: D = 80 (ViT-H) as above; D = 64 (SigLIP) takes Q and K as one 64-channel k-block each,
-// S in four k-slices, Vᵀ tiles of 64 rows, O with N = 64, and the four 16-column O chunks split 2 / 2 between the two softmax halves.
+// The kernel is a template on the head dimension D: D = 80 (ViT-H) as above; D = 64 (SigLIP B/16) takes Q and K as one 64-channel k-block
+// each, S in four k-slices, Vᵀ tiles of 64 rows, O with N = 64, and the four 16-column O chunks split 2 / 2 between the two softmax halves.
+// D = 72 (SigLIP SO400M) stores 72 channels per head but computes at the MMA width 80 (N = 72 is not a UMMA shape for M = 128): Q K^T
+// reads one 64-channel k-block and one 16-channel slice whose channels 72..79 belong to the next head (or, for the last head's Q, to K) -
+// they are zeroed in the Q tile once per item, so they add exact zeros; Vᵀ tiles have 80 rows (rows 72..79: the next head's channels or
+// TMA zero-fill), and O columns 72..79 are computed but never stored.
+__host__ __device__ constexpr int ta_mma_width(int d) { return (d + 15) / 16 * 16; }
 constexpr int kTaQ = 128, kTaK = 128;
 constexpr int kTaStages = 3;                              // K / V^T ring: a tile's load (~2 k cycles) overlaps two tiles of work
-template <int D> constexpr int kTaQBytes = ((D + 63) / 64) * kABytes;   // Q: 128 rows x 128 B per 64-channel k-block (D = 80: two)
+template <int D> constexpr int kTaQBytes = ((D + 63) / 64) * kABytes;   // Q: 128 rows x 128 B per 64-channel k-block (D = 80, 72: two)
 template <int D> constexpr int kTaKBytes = kTaQBytes<D>;                // K tile: the same
-template <int D> constexpr int kTaVBytes = 2 * D * 128;                 // V^T tile: two k-blocks (64 keys each) of D rows x 128 B
+template <int D> constexpr int kTaVBytes = 2 * ta_mma_width(D) * 128;   // V^T tile: two k-blocks (64 keys each) of MMA-width rows x 128 B
 constexpr int kTaPBytes = 2 * kABytes;                    // P: 128 rows x 128 keys bf16
 template <int D>
 constexpr int kTaSmemBytes = kTaQBytes<D> + kTaStages * (kTaKBytes<D> + kTaVBytes<D>) + kTaPBytes + 1024 /*align*/ + 256 /*barriers*/ + 3 * 2 * 128 * 4 /*row exchange*/;   // D = 80: 224.3 KB
@@ -549,6 +562,7 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;
   constexpr int kQBytes = kTaQBytes<D>, kKBytes = kTaKBytes<D>, kVBytes = kTaVBytes<D>;
+  constexpr int DM = ta_mma_width(D);                      // MMA width: D = 72 computes as 80
   uint8_t* sK = sQ + kQBytes;                              // [kTaStages]
   uint8_t* sV = sK + kTaStages * kKBytes;                  // [kTaStages]
   uint8_t* sP = sV + kTaStages * kVBytes;
@@ -610,14 +624,14 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
           tma_load_3d_at(k, &tm_qkv, &kv_full[st], W + head * D, t * kTaK, img, kEvictLast);
           if (D > 64) tma_load_3d_at(k + kABytes, &tm_qkv, &kv_full[st], W + head * D + 64, t * kTaK, img, kEvictLast);
           tma_load_3d_at(v, &tm_vt, &kv_full[st], t * kTaK, head * D, img, kEvictLast);
-          tma_load_3d_at(v + D * 128, &tm_vt, &kv_full[st], t * kTaK + 64, head * D, img, kEvictLast);
+          tma_load_3d_at(v + DM * 128, &tm_vt, &kv_full[st], t * kTaK + 64, head * D, img, kEvictLast);
         }
       }
     }
   } else if (warp == 1) {
     if (elect_one()) {
       constexpr uint32_t kIdescS = umma_idesc_bf16_f32(kTaQ, kTaK);
-      constexpr uint32_t kIdescO = umma_idesc_bf16_f32(kTaQ, D);
+      constexpr uint32_t kIdescO = umma_idesc_bf16_f32(kTaQ, DM);
       // Q K^T of global tile gq (scores buffer gq & 1)
       auto issue_qk = [&](int gq) {
         const int st = gq % kTaStages, sb = gq & 1;
@@ -627,7 +641,7 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
         const uint32_t a = smem_u32(sQ), b = smem_u32(sK + st * kKBytes);
         const uint32_t d = tmem_base + kColS + sb * kTaK;
 #pragma unroll
-        for (int k = 0; k < D / kUmmaK; ++k) {                      // 4 slices of k-block 0 (D = 80: and 1 of k-block 1)
+        for (int k = 0; k < DM / kUmmaK; ++k) {                     // 4 slices of k-block 0 (D = 80, 72: and 1 of k-block 1)
           const uint32_t off = (k >> 2) * kABytes + (k & 3) * (kUmmaK * 2);
           umma_bf16_ss(d, umma_desc_sw128_kmajor(a + off), umma_desc_sw128_kmajor(b + off), kIdescS, k != 0 ? 1u : 0u);
         }
@@ -636,6 +650,15 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       int g = 0, it = 0;
       for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++it) {
         mbar_wait(q_full, it & 1, 4);
+        if constexpr (DM != D) {
+          // Q channels D..DM-1 (16-byte chunk 1 of k-block 1 in each 128-byte swizzled row) are another head's: zero them, so that
+          // they multiply K's foreign channels (finite values of the qkv rows, or TMA zero-fill) into exact zeros
+          static_assert(DM - D == 8 && D - 64 == 8, "one foreign 16-byte chunk per row");
+          uint8_t* q1 = sQ + kABytes;
+#pragma unroll 8
+          for (int r = 0; r < kTaQ; ++r) *reinterpret_cast<uint4*>(q1 + r * 128 + ((1 ^ (r & 7)) << 4)) = make_uint4(0u, 0u, 0u, 0u);
+          fence_proxy_async_smem();                                 // generic-proxy writes -> visible to the tensor core's reads
+        }
         issue_qk(g);
         for (int t = 0; t < ntiles; ++t, ++g) {
           const int st = g % kTaStages;
@@ -647,7 +670,7 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
 #pragma unroll
           for (int k = 0; k < kTaK / kUmmaK; ++k) {
             const uint32_t offa = (k >> 2) * kABytes + (k & 3) * (kUmmaK * 2);
-            const uint32_t offb = (k >> 2) * (D * 128) + (k & 3) * (kUmmaK * 2);
+            const uint32_t offb = (k >> 2) * (DM * 128) + (k & 3) * (kUmmaK * 2);
             umma_bf16_ss(tmem_base + kColO, umma_desc_sw128_kmajor(a + offa), umma_desc_sw128_kmajor(b + offb), kIdescO, (t | k) != 0 ? 1u : 0u);
           }
           umma_commit(&kv_empty[st]);
@@ -662,8 +685,8 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
     const int r = quad * 32 + lane;                                 // query row inside the tile
     const uint32_t tlane = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
     const float c = p.scale_log2e;
-    constexpr int kOSplit = (D / 16 + 1) / 2;                       // D = 80: chunks 0-2 | 3-4; D = 64: 0-1 | 2-3
-    const int oc0 = half == 0 ? 0 : kOSplit, oc1 = half == 0 ? kOSplit : D / 16;   // 16-column chunks of O this warp rescales / stores
+    constexpr int kOSplit = (DM / 16 + 1) / 2;                      // D = 80, 72: chunks 0-2 | 3-4; D = 64: 0-1 | 2-3
+    const int oc0 = half == 0 ? 0 : kOSplit, oc1 = half == 0 ? kOSplit : DM / 16;  // 16-column chunks of O this warp rescales / stages
     int g = 0, it = 0;
     for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++it) {
       const int qt = item % qtiles, head = (item / qtiles) % p.heads, img = item / (qtiles * p.heads);
@@ -748,7 +771,7 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
       tc_fence_after_sync();
       asm volatile("bar.sync 2, 256;\n" ::: "memory");
       const float inv = 1.0f / (l_run + xl[(half ^ 1) * 128 + r]);
-      __nv_bfloat16* so = reinterpret_cast<__nv_bfloat16*>(sP) + r * (D + 8);
+      __nv_bfloat16* so = reinterpret_cast<__nv_bfloat16*>(sP) + r * (DM + 8);
 #pragma unroll 1
       for (int ch = oc0; ch < oc1; ++ch) {
         float ov[16];
@@ -759,15 +782,15 @@ vit_attention_tc_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid
                                                                  pack_bf16x2(ov[12] * inv, ov[13] * inv), pack_bf16x2(ov[14] * inv, ov[15] * inv));
       }
       asm volatile("bar.sync 1, 256;\n" ::: "memory");                 // both halves of every row are staged
-      // each warp copies 16 rows: 16 rows x D / 8 chunks of 16 B
+      // each warp copies 16 rows: 16 rows x D / 8 chunks of 16 B (the staged columns D..DM-1 are not stored)
       constexpr int kChunks = D / 8;
       __nv_bfloat16* dst = p.out + static_cast<size_t>(img) * T * W + head * D;
       const int row0 = quad * 32 + half * 16;
-      const __nv_bfloat16* sw = reinterpret_cast<const __nv_bfloat16*>(sP) + row0 * (D + 8);
+      const __nv_bfloat16* sw = reinterpret_cast<const __nv_bfloat16*>(sP) + row0 * (DM + 8);
       for (int i = lane; i < 16 * kChunks; i += 32) {
         const int rr = i / kChunks, cc = i - rr * kChunks;
         const int row = q0 + row0 + rr;
-        if (row < T) *reinterpret_cast<uint4*>(dst + static_cast<size_t>(row) * W + cc * 8) = *reinterpret_cast<const uint4*>(sw + rr * (D + 8) + cc * 8);
+        if (row < T) *reinterpret_cast<uint4*>(dst + static_cast<size_t>(row) * W + cc * 8) = *reinterpret_cast<const uint4*>(sw + rr * (DM + 8) + cc * 8);
       }
       // the staging rows overlap the P rows of other warps: nobody writes the next item's P before everyone has copied
       asm volatile("bar.sync 1, 256;\n" ::: "memory");
@@ -793,35 +816,46 @@ __global__ void __launch_bounds__(256) siglip_latent_q_kernel(const float* __res
   if (lane == 0) q[n] = s + __ldg(bq + n);
 }
 
-// out[img, h * 64 + c] = softmax_t(q_h . k_t / 8) v_t[c] over the T tokens of one image (bf16 out, fp32 throughout).
-// kv: bf16 [images * T, 2 W] (k | v, head h at columns h * 64).  One warp per (image, head): lanes in four groups of eight, each group
-// one key (or value) row per step = 128 contiguous bytes, each lane 8 channels; scores go through the warp's T floats of shared memory.
+// out[img, h * D + c] = softmax_t(q_h . k_t / sqrt(D)) v_t[c] over the T tokens of one image (bf16 out, fp32 throughout).
+// kv: bf16 [images * T, 2 W] (k | v, head h at columns h * D).  One warp per (image, head): lanes in four groups of eight, each group
+// one key (or value) row per step, each lane the 16-byte chunks c, c + 8, ... of the row's D / 8 (D = 64: one 128-byte row, one chunk
+// per lane; D = 72: 144 bytes, the ninth chunk on the group's first lane); scores go through the warp's T floats of shared memory.
 constexpr int kMapWarps = 4;
 constexpr int kMapMaxTokens = 3072;       // the scores of kMapWarps warps stay within the 48 KB of default dynamic shared memory
+template <int D>
 __global__ void __launch_bounds__(kMapWarps * 32) siglip_map_attention_kernel(const __nv_bfloat16* __restrict__ kv, const float* __restrict__ q,
                                                                               __nv_bfloat16* __restrict__ out, int T, int W, int heads, int items, float scale_log2e) {
+  static_assert(D % 8 == 0 && D >= 64 && D < 128, "one to two 16-byte chunks per lane");
+  constexpr int kChunks = D / 8, kPer = (kChunks + 7) / 8;
   extern __shared__ float sm_map[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int item = blockIdx.x * kMapWarps + warp;
   if (item >= items) return;
   const int img = item / heads, head = item - img * heads;
   const int grp = lane >> 3, c0 = (lane & 7) * 8;
+  const bool has2 = kPer > 1 && (lane & 7) + 8 < kChunks;      // lane's second chunk (D = 72: the group's first lane)
   float* sc = sm_map + warp * T;
-  const __nv_bfloat16* krow = kv + static_cast<size_t>(img) * T * 2 * W + head * kSiglipHeadDim + c0;
+  const __nv_bfloat16* krow = kv + static_cast<size_t>(img) * T * 2 * W + head * D + c0;
   const __nv_bfloat16* vrow = krow + W;
-  float qv[8];
+  float qv[kPer][8];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) qv[j] = __ldg(q + head * kSiglipHeadDim + c0 + j) * scale_log2e;   // scores in log2 units
+  for (int i = 0; i < kPer; ++i)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) qv[i][j] = i == 0 || has2 ? __ldg(q + head * D + c0 + i * 64 + j) * scale_log2e : 0.f;   // scores in log2 units
   for (int t0 = 0; t0 < T; t0 += 4) {
     const int t = t0 + grp;
     float s = 0.f;
     if (t < T) {
-      const uint4 u = __ldg(reinterpret_cast<const uint4*>(krow + static_cast<size_t>(t) * 2 * W));
-      const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&u);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = __bfloat1622float2(h2[j]);
-        s = fmaf(qv[2 * j], f.x, fmaf(qv[2 * j + 1], f.y, s));
+      for (int i = 0; i < kPer; ++i) {
+        if (i > 0 && !has2) break;
+        const uint4 u = __ldg(reinterpret_cast<const uint4*>(krow + static_cast<size_t>(t) * 2 * W + i * 64));
+        const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float2 f = __bfloat1622float2(h2[j]);
+          s = fmaf(qv[i][2 * j], f.x, fmaf(qv[i][2 * j + 1], f.y, s));
+        }
       }
     }
     s += __shfl_xor_sync(0xffffffffu, s, 1);
@@ -842,28 +876,42 @@ __global__ void __launch_bounds__(kMapWarps * 32) siglip_map_attention_kernel(co
   }
   l = warp_sum(l);
   __syncwarp();
-  float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  float acc[kPer][8];
+#pragma unroll
+  for (int i = 0; i < kPer; ++i)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
   for (int t = grp; t < T; t += 4) {
     const float pt = sc[t];
-    const uint4 u = __ldg(reinterpret_cast<const uint4*>(vrow + static_cast<size_t>(t) * 2 * W));
-    const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&u);
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float2 f = __bfloat1622float2(h2[j]);
-      acc[2 * j] = fmaf(pt, f.x, acc[2 * j]);
-      acc[2 * j + 1] = fmaf(pt, f.y, acc[2 * j + 1]);
+    for (int i = 0; i < kPer; ++i) {
+      if (i > 0 && !has2) break;
+      const uint4 u = __ldg(reinterpret_cast<const uint4*>(vrow + static_cast<size_t>(t) * 2 * W + i * 64));
+      const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float2 f = __bfloat1622float2(h2[j]);
+        acc[i][2 * j] = fmaf(pt, f.x, acc[i][2 * j]);
+        acc[i][2 * j + 1] = fmaf(pt, f.y, acc[i][2 * j + 1]);
+      }
     }
   }
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], 8);
-    acc[j] += __shfl_xor_sync(0xffffffffu, acc[j], 16);
-  }
+  for (int i = 0; i < kPer; ++i)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      acc[i][j] += __shfl_xor_sync(0xffffffffu, acc[i][j], 8);
+      acc[i][j] += __shfl_xor_sync(0xffffffffu, acc[i][j], 16);
+    }
   if (grp == 0) {
     const float inv = 1.0f / l;
-    *reinterpret_cast<uint4*>(out + static_cast<size_t>(img) * W + head * kSiglipHeadDim + c0) =
-        make_uint4(pack_bf16x2(acc[0] * inv, acc[1] * inv), pack_bf16x2(acc[2] * inv, acc[3] * inv), pack_bf16x2(acc[4] * inv, acc[5] * inv),
-                   pack_bf16x2(acc[6] * inv, acc[7] * inv));
+#pragma unroll
+    for (int i = 0; i < kPer; ++i) {
+      if (i > 0 && !has2) break;
+      *reinterpret_cast<uint4*>(out + static_cast<size_t>(img) * W + head * D + c0 + i * 64) =
+          make_uint4(pack_bf16x2(acc[i][0] * inv, acc[i][1] * inv), pack_bf16x2(acc[i][2] * inv, acc[i][3] * inv),
+                     pack_bf16x2(acc[i][4] * inv, acc[i][5] * inv), pack_bf16x2(acc[i][6] * inv, acc[i][7] * inv));
+    }
   }
 }
 

@@ -10,7 +10,9 @@ DESIGN.md and parity is pinned only on the independent restatement oracle/vit_or
 `SiglipImageEncoder` does the same for the reference's default embedder, open_clip `ViT-B-16-SigLIP` (config/train.yaml:126; timm
 `vit_base_patch16_siglip_224` with its MAP attention-pool head, parameters `visual.trunk.*`; 768-dim embeddings for the F = 768
 decoder), on the same kernels (novic_siglip_create / novic_siglip_set_weights + novic_vit_encode); its architecture is equally an
-assumption (DESIGN.md §5d, tests/siglip_oracle.py:encode_image_siglip).
+assumption (DESIGN.md §5d, tests/siglip_oracle.py:encode_image_siglip).  With `SIGLIP_SO400M` it is open_clip `ViT-SO400M-14-SigLIP`
+(timm `vit_so400m_patch14_siglip_224`: heads of 72, MLP 4304; 1152-dim embeddings for the F = 1152 checkpoints), assumed to be the same
+architecture at those dimensions.
 """
 from __future__ import annotations
 
@@ -60,6 +62,15 @@ class SiglipDims:
     @property
     def out_dim(self) -> int:
         return self.width
+
+    @property
+    def head_dim(self) -> int:
+        return self.width // self.heads
+
+
+# open_clip `ViT-SO400M-14-SigLIP` (timm `vit_so400m_patch14_siglip_224`), the image embedder of the F = 1152 checkpoints, as assumed in
+# DESIGN.md §5d
+SIGLIP_SO400M = SiglipDims(image_size=224, patch_size=14, width=1152, layers=27, heads=16, mlp_dim=4304)
 
 
 # ---- parameter holders: they exist so that state_dict() has open_clip's key names; none has a forward() ----
@@ -281,20 +292,22 @@ class _SigVisual(nn.Module):
 
 class SiglipImageEncoder(_NativeEncoder):
     """open_clip `ViT-B-16-SigLIP` image tower (`visual.trunk.*` parameters) on libnovic_b200: encode_image(images, normalize) on
-    preprocessed 224 x 224 images (resize and mean / std 0.5 stay with the caller) -> [B, width] fp32."""
+    preprocessed 224 x 224 images (resize and mean / std 0.5 stay with the caller) -> [B, width] fp32.  `SiglipImageEncoder(SIGLIP_SO400M)`
+    is the `ViT-SO400M-14-SigLIP` tower.  Supported: heads of 64 or 72 channels, width 640, 768, 1024, 1152 or 1280, an MLP width that
+    is a multiple of 16."""
 
     def __init__(self, dims: SiglipDims = SiglipDims(), images_per_chunk: int = 64):
         super().__init__()
-        if dims.heads < 1 or dims.width != dims.heads * 64:
-            raise ValueError("SiglipImageEncoder (novic_b200) supports heads of 64 channels only (width = heads * 64)")
-        if dims.width not in (640, 768, 1024, 1280):
-            raise ValueError(f"SiglipImageEncoder: width {dims.width} has no LayerNorm kernel (640, 768, 1024, 1280)")
+        if dims.heads < 1 or dims.width % dims.heads or dims.head_dim not in (64, 72):
+            raise ValueError("SiglipImageEncoder (novic_b200) supports heads of 64 or 72 channels only (width = heads * 64 or heads * 72)")
+        if dims.width not in (640, 768, 1024, 1152, 1280):
+            raise ValueError(f"SiglipImageEncoder: width {dims.width} has no LayerNorm kernel (640, 768, 1024, 1152, 1280)")
         if not 1 <= dims.layers <= _abi.NOVIC_VIT_MAX_LAYERS:
             raise ValueError(f"SiglipImageEncoder: between 1 and {_abi.NOVIC_VIT_MAX_LAYERS} blocks")
         if dims.patch_size < 1 or dims.image_size % dims.patch_size:
             raise ValueError("SiglipImageEncoder: image_size must be a multiple of patch_size")
-        if dims.mlp_dim < 128 or dims.mlp_dim % 128:
-            raise ValueError("SiglipImageEncoder: mlp_dim must be a multiple of 128")
+        if dims.mlp_dim < 16 or dims.mlp_dim % 16:
+            raise ValueError("SiglipImageEncoder: mlp_dim must be a multiple of 16")
         self.dims = dims
         self.images_per_chunk = int(images_per_chunk)
         self.visual = _SigVisual(dims)

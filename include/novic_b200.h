@@ -324,6 +324,28 @@ int novic_debug_wgrad(const void* a_t, int32_t Mo, const void* b_t, int32_t No, 
 int novic_debug_wgrad_mn(const void* a, int32_t Mo, int32_t ld_a, const void* b, int32_t No, int32_t ld_b, int64_t K, float* dw, void* stream);
 int32_t novic_debug_wgrad_splits(int64_t tiles, int64_t kblocks, int32_t sms);
 
+/* Building blocks of the image encoders, exported for the test-suite: the encoder's own launch helpers on caller-owned device buffers.
+ *   novic_debug_vit_gemm: acc[M, N] = a[M, K] (bf16) * w[N, K]^T (bf16), K % 128 == 0, N % 32 == 0, through epilogue
+ *     epi 0 (EpiVitBias):     dst bf16 [M, ld] = act(acc + bias) (act 0 none, 1 QuickGELU, 2 erf GELU; direct: 256-bit stores from the
+ *                             registers, else through the staging tile);
+ *     epi 1 (EpiVitResid):    dst fp32 [*, ld]: residual mode (table NULL) dst[r] += acc + bias; patch mode dst[img * (patches + tok0) + tok0 + p]
+ *                             = acc + table[(tok0 + p) * ld] + bias for GEMM row r = img * patches + p;
+ *     epi 2 (EpiVitStoreF32): dst fp32 [M, N] = acc (+ bias), ld == N.
+ *     bias may be NULL.  path 128 / 256 / 512 forces 128 x 128, 128 x 256 or CTA-pair 256 x 256 tiles; the persistent grid is divided by
+ *     grid_div (>= 1), so that few CTAs walk many tiles.
+ *   novic_debug_vit_attention: ao [nimg * T, W] bf16 = softmax(q k^T / sqrt(D)) v per (image, head) from qkv [nimg * T, 3 W] bf16, D = W / heads;
+ *     kernel 0 = the tcgen05 kernel (D = 64, 72 or 80) on at most max_ctas persistent CTAs (0: the encoder's grid), 1 = the mma.sync kernel (D = 80).
+ *   novic_debug_siglip_map_attention: out [nimg, W] bf16 = the MAP head's attention of the fp32 query q [W] over kv [nimg * T, 2 W] bf16 (k | v).
+ *   novic_debug_vit_layernorm: the encoder's LayerNorm kernel with every field of its parameters (W = 640, 768, 1024, 1152 or 1280): row r reads
+ *     x + r * in_stride (first set to cls + pos0 when cls != NULL and r % cls_period == 0), y = LN(x; w1, b1) written back when store_x,
+ *     out_bf [rows, W] = y, or LN(y; w2, b2) when w2 != NULL (out_bf may be NULL). */
+int novic_debug_vit_gemm(const void* a, const void* w, int32_t M, int32_t N, int32_t K, int32_t epi, int32_t act, int32_t direct, const float* bias,
+                         void* dst, int32_t ld, const float* table, int32_t patches, int32_t tok0, int32_t path, int32_t grid_div, void* stream);
+int novic_debug_vit_attention(const void* qkv, int32_t nimg, int32_t T, int32_t W, int32_t heads, int32_t kernel, int32_t max_ctas, void* out, void* stream);
+int novic_debug_siglip_map_attention(const void* kv, const float* q, int32_t nimg, int32_t T, int32_t W, int32_t heads, void* out, void* stream);
+int novic_debug_vit_layernorm(float* x, int64_t in_stride, const float* w1, const float* b1, const float* w2, const float* b2, int32_t store_x, void* out_bf,
+                              int32_t rows, int32_t W, float eps, const float* cls, const float* pos0, int32_t cls_period, void* stream);
+
 /* Per-kernel-class device timing for roofline reports.  novic_kernel_timing(1) makes every subsequent direct
  * (non-graph) launch record a CUDA-event pair on its stream; novic_kernel_times() synchronises and returns the
  * accumulated milliseconds and launch counts per class, then clears.  Classes, in order: embed-prep, prefix GEMM,

@@ -131,6 +131,12 @@ SIGNATURES = {
     "novic_debug_wgrad": (C.c_int, [_FP, C.c_int32, _FP, C.c_int32, C.c_int64, C.c_int32, _FP, C.c_void_p]),
     "novic_debug_wgrad_mn": (C.c_int, [_FP, C.c_int32, C.c_int32, _FP, C.c_int32, C.c_int32, C.c_int64, _FP, C.c_void_p]),
     "novic_debug_wgrad_splits": (C.c_int32, [C.c_int64, C.c_int64, C.c_int32]),
+    "novic_debug_vit_gemm": (C.c_int, [_FP, _FP, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _FP, _FP, C.c_int32, _FP,
+                                       C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "novic_debug_vit_attention": (C.c_int, [_FP, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _FP, C.c_void_p]),
+    "novic_debug_siglip_map_attention": (C.c_int, [_FP, _FP, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _FP, C.c_void_p]),
+    "novic_debug_vit_layernorm": (C.c_int, [_FP, C.c_int64, _FP, _FP, _FP, _FP, C.c_int32, _FP, C.c_int32, C.c_int32, C.c_float, _FP, _FP, C.c_int32,
+                                            C.c_void_p]),
     "novic_kernel_timing": (C.c_int, [C.c_int32]),
     "novic_kernel_times": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int32]),
     "novic_launch_count": (C.c_int64, []),

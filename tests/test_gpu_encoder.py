@@ -6,6 +6,9 @@ CUDA path computes that architecture: bf16 operands / fp32 accumulation and resi
 Tolerance (stated per test): ||got - ref|| / ||ref|| of the un-normalised features <= 2 % after two blocks, <= 3 % after all 32 (every
 block rounds its GEMM and attention operands to bf16, ~0.4 % each), no element off by more than six times that, cosine >= 0.999; and
 <= 0.8 % against the same restatement with its matrix-product operands rounded to bf16 (what separates a wrong kernel from rounding).
+The `vith_11_images` tests run a production-sized chunk (every trunk GEMM on CTA pairs, tests/encoder_chunks.py): sampled images within
+those bounds, the same bits as chunks of two and under NOVIC_VIT_BN=256 / 128 and NOVIC_VIT_DIRECT=0, and the mma.sync attention
+(NOVIC_VIT_ATTN=mma) within the bounds.  Each kernel alone against fp64: tests/test_gpu_vit_kernels.py.
 """
 import dataclasses
 
@@ -15,6 +18,7 @@ import torch
 from novic_b200 import default_decoder, synth
 from novic_b200.encoder import EncoderDecoder, ImageEncoder, VitDims, synth_images, synth_vit_state_dict
 from oracle import vit_oracle as vo
+from tests.encoder_chunks import check_bounds, production_chunk, same_under_switches
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -75,6 +79,44 @@ def test_full_depth_encoder_feeds_the_decoder():
     assert tok.shape[0] == 2 and tok.shape[1] == 1
     assert torch.equal(tok[:, 0], t2) and torch.equal(pad[:, 0], p2)
     assert (score[:, 0] - s2).abs().max().item() < 1e-3
+
+
+TWO = VitDims(layers=2)
+
+
+@pytest.fixture(scope="module")
+def vith_chunk():
+    """11 images in one chunk after two blocks: 8 030 token rows and 8 019 patch rows, 63 row tiles each (odd: the last pair's second CTA
+    has no rows), so every trunk GEMM runs on CTA pairs.  The final projection has one row per image and stays on 128 x 128 tiles."""
+    sd = synth_vit_state_dict(TWO, seed=19)
+
+    def make(n):
+        enc = ImageEncoder(TWO, images_per_chunk=n)
+        enc.load_state_dict(sd, strict=True)
+        return enc.to(DEV).eval()
+    restate = lambda x, bf16: vo.encode_image(_cfg(TWO), sd, x, bf16_operands=bf16)
+    return production_chunk(make, synth_images(11, TWO, seed=29), restate, 0.02, 0.008, {"EpiVitBias", "EpiVitResid"}), make
+
+
+def test_vith_11_images_in_one_chunk_run_on_cta_pairs(vith_chunk):
+    """gemm2_kernel ran the bias and residual epilogues (patch mode included); sampled images within the two-block bounds; chunks of two
+    give the same bits."""
+    run, _ = vith_chunk
+    assert run.got.shape == (11, 1024)
+
+
+def test_vith_11_images_bit_identical_under_tile_and_store_switches(vith_chunk, monkeypatch):
+    run, make = vith_chunk
+    same_under_switches(run, make, monkeypatch)
+
+
+def test_vith_11_images_mma_attention_within_bounds(vith_chunk, monkeypatch):
+    """NOVIC_VIT_ATTN=mma: the mma.sync attention kernel accumulates in another order, so it is held to the restatement bounds."""
+    run, make = vith_chunk
+    monkeypatch.setenv("NOVIC_VIT_ATTN", "mma")
+    with torch.inference_mode():
+        got = make(11).encode_image(run.img.to(DEV)).cpu()
+    check_bounds(got[run.sample], run.ref, run.ref16, 0.02, 0.008, "NOVIC_VIT_ATTN=mma, 11 images in one chunk")
 
 
 def test_encoder_state_dict_keys_follow_open_clip():

@@ -5,7 +5,9 @@ PARITY UNPINNED: open_clip_torch and timm are un-vendored dependencies of the re
 memory (DESIGN.md §5d) and cannot be checked against the reference here.  What the GPU tests establish is that the CUDA path computes
 that architecture: bf16 operands / fp32 accumulation and residual stream against fp32 on the CPU, with the tolerances of
 tests/test_gpu_encoder.py - ||got - ref|| / ||ref|| <= 2 % after two blocks, <= 3 % after all twelve, no element off by more than six
-times that, cosine >= 0.999, and <= 0.8 % against the restatement whose matrix-product operands are rounded to bf16.
+times that, cosine >= 0.999, and <= 0.8 % against the restatement whose matrix-product operands are rounded to bf16.  The `b16_67_images`
+tests run a production-sized chunk (every trunk GEMM on CTA pairs, tests/encoder_chunks.py): sampled images within the two-block bounds,
+the same bits as chunks of two, under NOVIC_VIT_BN=256 / 128 and NOVIC_VIT_DIRECT=0, and on a workspace poisoned with 0xFF.
 """
 import ctypes as C
 import dataclasses
@@ -18,6 +20,7 @@ import torch
 from novic_b200 import _abi, default_decoder, synth
 from novic_b200.encoder import EncoderDecoder, SiglipDims, SiglipImageEncoder, synth_images, synth_siglip_state_dict
 from tests import siglip_oracle as vo
+from tests.encoder_chunks import poisoned_workspace, production_chunk, same_under_switches
 
 DEV = "cuda:0"
 HEADER = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "novic_b200.h")
@@ -167,6 +170,44 @@ def test_full_depth_encoder_feeds_the_f768_decoder():
     assert bt.shape[:2] == (4, 10)
     assert torch.equal(bt, bt2) and torch.equal(bp, bp2)
     assert (bs - bs2).abs().max().item() < 1e-3
+
+
+B16_TWO = SiglipDims(layers=2)
+
+
+@pytest.fixture(scope="module")
+def b16_chunk():
+    """67 images in one chunk after two blocks: 13 132 token rows = 103 row tiles (odd: the last pair's second CTA has no rows), so every
+    trunk GEMM runs on CTA pairs (>= 2 x 148 tiles of 128 x 256).  The MAP head's GEMMs have one row per image and stay on 128 x 128 tiles
+    (tests/test_gpu_vit_kernels.py covers their epilogue on pairs)."""
+    sd = synth_siglip_state_dict(B16_TWO, seed=21)
+
+    def make(n):
+        enc = SiglipImageEncoder(B16_TWO, images_per_chunk=n)
+        enc.load_state_dict(sd, strict=True)
+        return enc.to(DEV).eval()
+    restate = lambda x, bf16: vo.encode_image_siglip(_cfg(B16_TWO), sd, x, bf16_operands=bf16)
+    return production_chunk(make, synth_images(67, B16_TWO, seed=25), restate, 0.02, 0.008, {"EpiVitBias", "EpiVitResid"}), make
+
+
+@pytest.mark.gpu
+def test_b16_67_images_in_one_chunk_run_on_cta_pairs(b16_chunk):
+    """gemm2_kernel ran the bias and residual epilogues; the first, middle and last images are within the two-block bounds; every image
+    equals its features from chunks of two, bit for bit."""
+    run, _ = b16_chunk
+    assert run.got.shape == (67, 768)
+
+
+@pytest.mark.gpu
+def test_b16_67_images_bit_identical_under_tile_and_store_switches(b16_chunk, monkeypatch):
+    run, make = b16_chunk
+    same_under_switches(run, make, monkeypatch)
+
+
+@pytest.mark.gpu
+def test_b16_67_images_poisoned_workspace(b16_chunk):
+    """T = 196 < Tpad = 256: the V^T columns past T and the zero-filled key rows of the ragged tile are read on every item."""
+    poisoned_workspace(b16_chunk[0])
 
 
 def test_mismatched_embed_width_is_rejected():

@@ -7,7 +7,10 @@ for SO400M: timm `vit_so400m_patch14_siglip_224` is B/16's architecture with 14 
 dimension as width / heads, so the same restatement serves at these dimensions (`SiglipCfg(**asdict(dims))`).  The GPU tests
 establish that the CUDA path computes that architecture at these dimensions - attention at 72 stored / 80 computed channels per head,
 the MAP head's 144-byte rows, the LayerNorm at width 1152 and the MLP padded from 4304 to 4352 hidden channels - with B/16's bounds
-after two blocks (<= 2 % against fp32, <= 0.8 % against the bf16-operand restatement, cosine >= 0.999) and <= 4 % after all 27.
+after two blocks (<= 2 % against fp32, <= 0.8 % against the bf16-operand restatement, cosine >= 0.999) and <= 4 % after all 27.  The
+`so400m_31_images` tests run a production-sized chunk (every trunk GEMM on CTA pairs, with N = 1152 and 3456 ending inside a pair tile's
+B half): sampled images within the two-block bounds, the same bits as chunks of two and under NOVIC_VIT_BN=256 / 128 and
+NOVIC_VIT_DIRECT=0.
 """
 import dataclasses
 
@@ -16,7 +19,9 @@ import torch
 
 from novic_b200 import SIGLIP_SO400M, _abi, default_decoder, synth
 from novic_b200.encoder import EncoderDecoder, SiglipDims, SiglipImageEncoder, synth_images, synth_siglip_state_dict
-from tests.test_siglip_encoder import _compare, expected_shapes
+from tests import siglip_oracle as vo
+from tests.encoder_chunks import production_chunk, same_under_switches
+from tests.test_siglip_encoder import _cfg, _compare, expected_shapes
 
 DEV = "cuda:0"
 TWO = dataclasses.replace(SIGLIP_SO400M, layers=2)
@@ -140,3 +145,30 @@ def test_poisoned_workspace_gives_the_same_features(full_depth):
         b = enc.encode_image(x)
     assert torch.isfinite(a).all() and torch.isfinite(b).all()
     assert torch.equal(a, b)
+
+
+@pytest.fixture(scope="module")
+def so400m_chunk():
+    """31 images in one chunk after two blocks: 7 936 token rows = 62 row tiles; N = 1152 (out-proj, fc2, patch embedding) ends in the B
+    half of the last pair tile, N = 3456 (QKV) likewise."""
+    sd = synth_siglip_state_dict(TWO, seed=23)
+
+    def make(n):
+        enc = SiglipImageEncoder(TWO, images_per_chunk=n)
+        enc.load_state_dict(sd, strict=True)
+        return enc.to(DEV).eval()
+    restate = lambda x, bf16: vo.encode_image_siglip(_cfg(TWO), sd, x, bf16_operands=bf16)
+    return production_chunk(make, synth_images(31, TWO, seed=27), restate, 0.02, 0.008, {"EpiVitBias", "EpiVitResid"}), make
+
+
+@pytest.mark.gpu
+def test_so400m_31_images_in_one_chunk_run_on_cta_pairs(so400m_chunk):
+    """gemm2_kernel ran the bias and residual epilogues; sampled images within the two-block bounds; chunks of two give the same bits."""
+    run, _ = so400m_chunk
+    assert run.got.shape == (31, 1152)
+
+
+@pytest.mark.gpu
+def test_so400m_31_images_bit_identical_under_tile_and_store_switches(so400m_chunk, monkeypatch):
+    run, make = so400m_chunk
+    same_under_switches(run, make, monkeypatch)

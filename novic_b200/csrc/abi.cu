@@ -163,36 +163,15 @@ int make_tmap_3d(CUtensorMap* map, const void* base, const cuuint64_t (&dims)[3]
 // GEMM launch
 // ---------------------------------------------------------------------------------------------------------
 constexpr int kStagesQKV = 5, kStagesGelu = 5, kStagesRow = 4, kStagesLogits = 5;
-bool g_fuse_block = true;                      // NOVIC_FUSE_BLOCK=0: out-proj + LN2 and the feed-forward block as two row kernels
 int g_block_rows64_min = 148 * 32 + 1;         // NOVIC_BLOCK_ROWS64_MIN: passes of at least this many rows run the row-owner block kernel on 64 rows per CTA (block_rows64_kernel); 0 = never
-int g_attn_split_max = 0;                      // NOVIC_ATTN_SPLIT_MAX: largest decode batch (sequences) of the split-key attention kernel; 0 = two waves of CTAs (8 x #SMs = 1184: measured 0.75 against 0.84 ms at 1024 sequences, 1.37 against 0.94 ms at 2048)
-int g_qkv_ws_div = 24;                         // NOVIC_QKV_WS_DIV: the weight-stationary QKV kernel from 24 / div row blocks per pass on (24 = every pass - with three activation stages and 256-bit stores it beats the generic persistent kernel at every size measured: QKV class 0.52 -> 0.42 ms at 128 rows, 0.55 -> 0.45 at 512, 0.58 -> 0.47 at 1024, 0.82 -> 0.69 at 2048; 1 = the round-2 rule, at least two row blocks per CTA)
-int g_qkv_ws_stages = 3;                       // NOVIC_QKV_WS_STAGES: 3 = three 32 KB activation stages in the weight-stationary QKV kernel, q / K / V stored from registers with 256-bit stores (default: QKV class 1.10 -> 0.99 ms per decode); 2 = two stages + the epilogue's 32 KB staging tile
 int g_vit_direct = 1;                          // NOVIC_VIT_DIRECT=0: the image encoder's bias / QuickGELU epilogues store their bf16 rows through the staging tile instead of with 256-bit stores from the registers (measured: 848 -> 855 images/s)
-bool g_attn_prefix = true;                     // NOVIC_ATTN_PREFIX=0: the prefix pass on attention_bulk_kernel instead of attention_prefix_kernel
-bool g_attn_split = true;                      // NOVIC_ATTN_SPLIT=0: the stream attention kernel (one warp per sequence) for small batches too
-bool g_fuse_attn = false;                      // NOVIC_FUSE_ATTN=1: the decode-step attention runs inside the row-owner block kernel (block_rows_kernel<true>; bit-identical, one launch and the ao round trip less per layer; measured 5.05 vs 5.09 ms per decode - kept as a switch so that the attention stays a launch of its own with its own HBM roofline record)
-bool g_ffn1_ksplit = true;                     // NOVIC_FFN1_KSPLIT=0: the 128-row block kernel gathers the whole LN2 row in every CTA (outproj_ffn_kernel) instead of reduce-scattering partial FFN1 sums
-int g_block64_pad = 16384;                     // NOVIC_BLOCK64_PAD=0: no extra shared memory per CTA of the 64-row block kernel -> two CTAs per SM (measured slower, DESIGN.md section 5)
-int g_block_rows = 0;                          // NOVIC_BLOCK_ROWS: 0 / 32 = the row-owner block kernel (blockrows.cuh, one CTA per 32 rows); 64 / 128 = the cluster kernels on 64- / 128-row tiles; -1 = the round-2 policy (64-row tiles up to kBlock64MaxRows rows, 128-row tiles above)
-constexpr int kBlock64MaxRows = 1536;
-int g_qkv_ws = 1;                              // NOVIC_QKV_WS=0: the QKV projection on the generic persistent kernel (else weight-stationary when every CTA gets >= 2 row blocks)
+int g_block_rows = 0;                          // NOVIC_BLOCK_ROWS=128: the block kernel on the 4-CTA cluster kernel with 128-row tiles (outproj_ffn_kernel, the tests' reference) instead of the row-owner kernel (blockrows.cuh)
+int g_qkv_ws = 1;                              // NOVIC_QKV_WS=0: the decode path's QKV projection on the generic persistent kernel (the tests' reference) instead of the weight-stationary one
 bool g_wgrad_mn = true;                        // NOVIC_WGRAD_MN=0: the training step's weight-gradient GEMMs on transposed bf16 copies of their operands (K-major descriptors)
-int g_qkv_per_tile = 0;                        // NOVIC_QKV_PER_TILE: cap on the CTAs per column tile of the weight-stationary QKV kernel (tuning)
-int g_qkv_mc = 0;                              // NOVIC_QKV_MC=0: the weight-stationary QKV kernel without the cluster multicast of its activation stages
-int g_qkv_bn = 128;                            // NOVIC_QKV_BN=256: 128 x 256 tiles in the QKV GEMM when they fill a wave
-bool g_fuse_qkv = false;                       // NOVIC_FUSE_QKV=1: layer l + 1's QKV projection in the tail of layer l's block kernel (bit-identical; measured 0.2-0.3 ms per decode slower than its own launch)
-bool g_attn_tf = true;                         // NOVIC_ATTN_TF=0: teacher-forced passes use the key-by-key bulk kernel instead of attention_tf_kernel
-int g_attn_hint = 1;                           // NOVIC_ATTN_HINT bit 0: evict-first L2 policy on the streamed K/V rows; bit 1: evict-last on new K/V rows
-int g_row_stages = 4;                          // NOVIC_ROW_STAGES=2|3: shallower row-kernel pipelines (tuning: co-residency with the next kernel)
-bool g_split_ffn = true;                       // NOVIC_SPLIT_FFN=0: every CTA of a cluster recomputes the whole hidden tile
-bool g_early_b = true;                         // NOVIC_EARLY_B=0: no weight-tile requests before griddepcontrol.wait
-bool g_wide_gemm = true;                       // NOVIC_WIDE_GEMM=0: the 16 KB-request pipeline (5 stages of one k-block)
 constexpr int kWideKbs = 2, kWideStages = 3;   // decode-path QKV / logits GEMMs: 3 stages of 2 k-blocks, 32 KB TMA requests
 int g_num_sms = 148;
-int g_logits_ew = 16;                          // NOVIC_LOGITS_EW=8: eight epilogue warps in the 128 x 256 logits kernel (else 16)
-int g_logits_bn = 256;                         // NOVIC_LOGITS_BN=128: the logits GEMM on 128 x 128 tiles everywhere
-int g_grid_div = 1;   // persistent grids are divided by the number of concurrent chains so that chains co-run on disjoint SMs
+int g_logits_bn = 256;                         // NOVIC_LOGITS_BN=128: the logits GEMM on 128 x 128 tiles everywhere (the tests' reference)
+int g_grid_div = 1;   // persistent grids are divided by this (the encoder's debug hooks run kernels on a fraction of the SMs)
 constexpr int kLogitBN = kTileN;
 
 // All decode-loop kernels are launched with programmatic stream serialization (PDL): the next kernel's CTAs may start
@@ -254,56 +233,18 @@ int launch_gemm_mn(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tb,
 }
 
 // Weight-stationary GEMM (gemm_ws_kernel): K = 512, ta / tb 3-D maps with 128-row boxes and 2 k-blocks per request.
-template <class Epi, int WS_STAGES>
+static_assert(kE == kWsKb * kBlockK, "the weight-stationary kernel holds the whole K = 512 weight tile");
+template <class Epi>
 int set_gemm_ws_attr() {
-  static_assert(gemm_ws_smem_bytes(WS_STAGES) <= 227 * 1024, "weight-stationary GEMM does not fit in shared memory");
-  CUDA_TRY(cudaFuncSetAttribute(gemm_ws_kernel<Epi, WS_STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_ws_smem_bytes(WS_STAGES)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_wsmc_kernel<Epi, WS_STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_ws_smem_bytes(WS_STAGES)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_wsmc2_kernel<Epi, WS_STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_ws_smem_bytes(WS_STAGES)));
-  return 0;
-}
-template <class Epi, int WS_STAGES>
-int launch_gemm_ws(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tb, int M, int N, const typename Epi::Params& ep, bool b_is_static,
-                   const CUtensorMap* ta2 = nullptr) {   // ta2: 2-D map of the activations (one k-block per request) for the multicast variant
-  const int n_tiles = static_cast<int>(ceil_div(N, kTileN));
-  int per_tile = std::max(1, std::min<int>(g_num_sms / g_grid_div / n_tiles, static_cast<int>(ceil_div(M, kBlockM))));
-  if (g_qkv_per_tile > 0) per_tile = std::min(per_tile, g_qkv_per_tile);
-  if (getenv("NOVIC_DEBUG_CLUSTERS")) {
-    static bool once = false;
-    if (!once) {
-      once = true;
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(144); cfg.blockDim = dim3(kGemmThreads); cfg.dynamicSmemBytes = gemm_ws_smem_bytes(WS_STAGES);
-      int n4 = -1, n2 = -1;
-      cudaOccupancyMaxActiveClusters(&n4, gemm_wsmc_kernel<Epi, WS_STAGES>, &cfg);
-      cudaOccupancyMaxActiveClusters(&n2, gemm_wsmc2_kernel<Epi, WS_STAGES>, &cfg);
-      fprintf(stderr, "max active clusters: of 4 CTAs %d, of 2 CTAs %d\n", n4, n2);
-    }
-  }
-  if (g_qkv_mc == 2 && ta2 != nullptr && n_tiles % 2 == 0)
-    CUDA_TRY(launch_k(gemm_wsmc2_kernel<Epi, WS_STAGES>, dim3(static_cast<unsigned>(n_tiles * per_tile)), dim3(kGemmThreads), gemm_ws_smem_bytes(WS_STAGES), s, *ta2, tb, M, n_tiles, b_is_static ? 1 : 0, ep));
-  else if (g_qkv_mc == 4 && ta2 != nullptr && n_tiles % 4 == 0)
-    CUDA_TRY(launch_k(gemm_wsmc_kernel<Epi, WS_STAGES>, dim3(static_cast<unsigned>(n_tiles * per_tile)), dim3(kGemmThreads), gemm_ws_smem_bytes(WS_STAGES), s, *ta2, tb, M, n_tiles, b_is_static ? 1 : 0, ep));
-  else
-    CUDA_TRY(launch_k(gemm_ws_kernel<Epi, WS_STAGES>, dim3(static_cast<unsigned>(n_tiles * per_tile)), dim3(kGemmThreads), gemm_ws_smem_bytes(WS_STAGES), s, ta, tb, M, n_tiles, b_is_static ? 1 : 0, ep));
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
-// Weight-stationary GEMM on CTA pairs (gemm_ws2_kernel): K = 512; ta 3-D map with 128-row boxes, tb 3-D map with 64-row boxes (2 k-blocks per request).
-template <class Epi>
-int set_gemm_ws2_attr() {
-  static_assert(gemm_ws2_smem_bytes() <= 227 * 1024, "pair weight-stationary GEMM does not fit in shared memory");
-  CUDA_TRY(cudaFuncSetAttribute(gemm_ws2_kernel<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_ws2_smem_bytes()));
+  static_assert(gemm_ws_smem_bytes() <= 227 * 1024, "weight-stationary GEMM does not fit in shared memory");
+  CUDA_TRY(cudaFuncSetAttribute(gemm_ws_kernel<Epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_ws_smem_bytes()));
   return 0;
 }
 template <class Epi>
-int launch_gemm_ws2(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tbh, int M, int N, const typename Epi::Params& ep, bool b_is_static) {
+int launch_gemm_ws(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tb, int M, int N, const typename Epi::Params& ep, bool b_is_static) {
   const int n_tiles = static_cast<int>(ceil_div(N, kTileN));
-  int per_tile = std::max(1, std::min<int>(g_num_sms / g_grid_div / 2 / n_tiles, static_cast<int>(ceil_div(M, 2 * kBlockM))));
-  if (g_qkv_per_tile > 0) per_tile = std::min(per_tile, g_qkv_per_tile);
-  CUDA_TRY(launch_k(gemm_ws2_kernel<Epi>, dim3(static_cast<unsigned>(2 * n_tiles * per_tile)), dim3(kGemmThreads), gemm_ws2_smem_bytes(), s, ta, tbh, M, n_tiles, b_is_static ? 1 : 0, ep));
+  const int per_tile = std::max(1, std::min<int>(g_num_sms / g_grid_div / n_tiles, static_cast<int>(ceil_div(M, kBlockM))));
+  CUDA_TRY(launch_k(gemm_ws_kernel<Epi>, dim3(static_cast<unsigned>(n_tiles * per_tile)), dim3(kGemmThreads), gemm_ws_smem_bytes(), s, ta, tb, M, n_tiles, b_is_static ? 1 : 0, ep));
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -330,20 +271,10 @@ int launch_gemm2(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tb, i
 
 int set_rowln_attr() {
   CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<kStagesRow, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(kStagesRow, false)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<kStagesRow, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(kStagesRow, true)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<kStagesRow, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(kStagesRow, true)));
-  CUDA_TRY(cudaFuncSetAttribute(outproj_ffn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, outproj_ffn_smem_bytes()));
-  CUDA_TRY(cudaFuncSetAttribute(outproj_ffn_ks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, outproj_ffn_smem_bytes()));
-  CUDA_TRY(cudaFuncSetAttribute(outproj_ffn64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, outproj_ffn64_smem_bytes() + 16384));
-  CUDA_TRY(cudaFuncSetAttribute(outproj_ffn64_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));   // two CTAs per SM need all of it
-  CUDA_TRY(cudaFuncSetAttribute(block_rows_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, block_rows_smem_bytes()));
-  CUDA_TRY(cudaFuncSetAttribute(block_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, block_rows_smem_bytes()));
-  CUDA_TRY(cudaFuncSetAttribute(block_rows64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, block_rows64_smem_bytes()));
   CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<kStagesRow, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(kStagesRow, false)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(2, false)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(2, true)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(3, false)));
-  CUDA_TRY(cudaFuncSetAttribute(gemm_rowln_kernel<3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, rowln_smem_bytes(3, true)));
+  CUDA_TRY(cudaFuncSetAttribute(outproj_ffn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, outproj_ffn_smem_bytes()));
+  CUDA_TRY(cudaFuncSetAttribute(block_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, block_rows_smem_bytes()));
+  CUDA_TRY(cudaFuncSetAttribute(block_rows64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, block_rows64_smem_bytes()));
   return 0;
 }
 
@@ -351,43 +282,18 @@ int set_rowln_attr() {
 int launch_rowln(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tb, int M, int N, int K, const RowParams& ep) {
   dim3 grid(static_cast<unsigned>(N / kRowBN), static_cast<unsigned>(ceil_div(M, kBlockM)));
   if (ep.drop.thresh != 0u) CUDA_TRY(launch_k(gemm_rowln_kernel<kStagesRow, 0, true>, grid, dim3(kRowThreads), rowln_smem_bytes(kStagesRow, false), s, ta, tb, tb, M, K / kBlockK, ep));
-  else if (g_row_stages == 2) CUDA_TRY(launch_k(gemm_rowln_kernel<2, false>, grid, dim3(kRowThreads), rowln_smem_bytes(2, false), s, ta, tb, tb, M, K / kBlockK, ep));
-  else if (g_row_stages == 3) CUDA_TRY(launch_k(gemm_rowln_kernel<3, false>, grid, dim3(kRowThreads), rowln_smem_bytes(3, false), s, ta, tb, tb, M, K / kBlockK, ep));
   else CUDA_TRY(launch_k(gemm_rowln_kernel<kStagesRow, false>, grid, dim3(kRowThreads), rowln_smem_bytes(kStagesRow, false), s, ta, tb, tb, M, K / kBlockK, ep));
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return 0;
 }
 
-// Whole feed-forward block: x += W2 * gelu(W1 * xn), then LayerNorm.  ta = LN2(x) rows, tw1 = linear1 [128, 512], tw2 = linear2 [512, 128].
-// split_h: tw1 has a 32-row box and every CTA of a cluster computes a quarter of the hidden tile (gemm_rowln_kernel<., 2>).
-int launch_ffn(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tw1, const CUtensorMap& tw2, int M, const RowParams& ep, bool split_h = false) {
-  dim3 grid(static_cast<unsigned>(kE / kRowBN), static_cast<unsigned>(ceil_div(M, kBlockM)));
-  if (split_h && g_row_stages == 2) CUDA_TRY(launch_k(gemm_rowln_kernel<2, 2>, grid, dim3(kRowThreads), rowln_smem_bytes(2, true), s, ta, tw2, tw1, M, kE / kBlockK, ep));
-  else if (split_h && g_row_stages == 3) CUDA_TRY(launch_k(gemm_rowln_kernel<3, 2>, grid, dim3(kRowThreads), rowln_smem_bytes(3, true), s, ta, tw2, tw1, M, kE / kBlockK, ep));
-  else if (split_h) CUDA_TRY(launch_k(gemm_rowln_kernel<kStagesRow, 2>, grid, dim3(kRowThreads), rowln_smem_bytes(kStagesRow, true), s, ta, tw2, tw1, M, kE / kBlockK, ep));
-  else CUDA_TRY(launch_k(gemm_rowln_kernel<kStagesRow, true>, grid, dim3(kRowThreads), rowln_smem_bytes(kStagesRow, true), s, ta, tw2, tw1, M, kE / kBlockK, ep));
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
-// Attention output -> next LayerNorm rows in one cluster kernel (out-proj + LN2 + feed-forward + LN), decode path.
-int launch_outproj_ffn(cudaStream_t s, const CUtensorMap& tao, const CUtensorMap& two, const CUtensorMap& tw1q, const CUtensorMap& tw2,
-                       const CUtensorMap& twqkv, int M, const FusedBlockParams& ep) {
+// Attention output -> next LayerNorm rows in one cluster kernel (out-proj + LN2 + feed-forward + LN) on 128-row tiles.
+int launch_outproj_ffn(cudaStream_t s, const CUtensorMap& tao, const CUtensorMap& two, const CUtensorMap& tw1q, const CUtensorMap& tw2, int M,
+                       const FusedBlockParams& ep) {
   static_assert(outproj_ffn_smem_bytes() <= 227 * 1024, "fused block kernel does not fit in shared memory");
   dim3 grid(static_cast<unsigned>(kRowCluster), static_cast<unsigned>(ceil_div(M, kBlockM)));
-  CUDA_TRY(launch_k(outproj_ffn_kernel, grid, dim3(kRowThreads), outproj_ffn_smem_bytes(), s, tao, two, tw1q, tw2, twqkv, M, ep));
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
-// The block kernel with FFN1 split over K (outproj_ffn_ks_kernel); tw1 = linear1 with a 128-row box.
-int launch_outproj_ffn_ks(cudaStream_t s, const CUtensorMap& tao, const CUtensorMap& two, const CUtensorMap& tw1, const CUtensorMap& tw2, int M,
-                          const FusedBlockParams& ep) {
-  dim3 grid(static_cast<unsigned>(kRowCluster), static_cast<unsigned>(ceil_div(M, kBlockM)));
-  CUDA_TRY(launch_k(outproj_ffn_ks_kernel, grid, dim3(kRowThreads), outproj_ffn_smem_bytes(), s, tao, two, tw1, tw2, M, ep));
+  CUDA_TRY(launch_k(outproj_ffn_kernel, grid, dim3(kRowThreads), outproj_ffn_smem_bytes(), s, tao, two, tw1q, tw2, M, ep));
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -395,28 +301,13 @@ int launch_outproj_ffn_ks(cudaStream_t s, const CUtensorMap& tao, const CUtensor
 
 // The same block with one CTA per 32 rows and the weights streamed as the M operand (block_rows_kernel, blockrows.cuh); tao: 3-D, 32 rows x 8
 // k-blocks; two / tw2: 4-D row-permuted maps (make_tmap4_perm); tw1: 3-D, 128 rows x 4 k-blocks.
-// pa != nullptr: the decode-step attention of the same rows runs inside the kernel (block_rows_kernel<true>: no attention launch, no ao round trip).
+// ta64 != nullptr: 64 rows per CTA (block_rows64_kernel), ta64 = the attention rows as 64 rows x 8 k-blocks.
 int launch_block_rows(cudaStream_t s, const CUtensorMap& tao, const CUtensorMap& two, const CUtensorMap& tw1, const CUtensorMap& tw2, const CUtensorMap& tx,
-                      int M, const FusedBlockParams& ep, const AttnParams* pa, const CUtensorMap* ta64 = nullptr) {
-  const dim3 grid(static_cast<unsigned>(ceil_div(M, kBrRows)));
-  if (pa == nullptr && ta64 != nullptr) {
+                      int M, const FusedBlockParams& ep, const CUtensorMap* ta64) {
+  if (ta64 != nullptr)
     CUDA_TRY(launch_k(block_rows64_kernel, dim3(static_cast<unsigned>(ceil_div(M, kB64Rows))), dim3(kBrThreads), block_rows64_smem_bytes(), s, *ta64, two, tw1, tw2, tx, M, ep));
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
-    return 0;
-  }
-  if (pa != nullptr) CUDA_TRY(launch_k(block_rows_kernel<true>, grid, dim3(kBrThreads), block_rows_smem_bytes(), s, tao, two, tw1, tw2, tx, M, ep, *pa));
-  else CUDA_TRY(launch_k(block_rows_kernel<false>, grid, dim3(kBrThreads), block_rows_smem_bytes(), s, tao, two, tw1, tw2, tx, M, ep, AttnParams{}));
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
-// The same block on 64-row tiles, two CTAs per SM (outproj_ffn64_kernel); all four maps are 3-D (tao: 64 rows x 2 k-blocks).
-int launch_outproj_ffn64(cudaStream_t s, const CUtensorMap& tao, const CUtensorMap& two, const CUtensorMap& tw1q, const CUtensorMap& tw2, int M,
-                         const FusedBlockParams& ep) {
-  dim3 grid(static_cast<unsigned>(kRowCluster), static_cast<unsigned>(ceil_div(M, kHbRows)));
-  CUDA_TRY(launch_k(outproj_ffn64_kernel, grid, dim3(kHbThreads), outproj_ffn64_smem_bytes() + g_block64_pad, s, tao, two, tw1q, tw2, M, ep));
+  else
+    CUDA_TRY(launch_k(block_rows_kernel, dim3(static_cast<unsigned>(ceil_div(M, kBrRows))), dim3(kBrThreads), block_rows_smem_bytes(), s, tao, two, tw1, tw2, tx, M, ep));
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -516,16 +407,11 @@ struct WeightPtrs {
   const __nv_bfloat16 *embed_mlp, *tok;
   const __nv_bfloat16 *in_proj[NOVIC_MAX_LAYERS], *out_proj[NOVIC_MAX_LAYERS], *linear1[NOVIC_MAX_LAYERS], *linear2[NOVIC_MAX_LAYERS];
   const float *tok_f32, *pos, *final_norm, *norm1[NOVIC_MAX_LAYERS], *norm2[NOVIC_MAX_LAYERS];
-  CUtensorMap tm_linear1_q[NOVIC_MAX_LAYERS];            // linear1 with a 32-row box (split-hidden feed-forward kernel)
-  // 3-D maps of the 64-row block kernel: out_proj (128 rows x 2 k-blocks = 32 KB per request), linear1 (32 rows x 8 k-blocks: the CTA's whole
-  // slice in one request), linear2 (128 rows x 2 k-blocks: the CTA's whole slice in one request)
-  CUtensorMap tm_out_proj3[NOVIC_MAX_LAYERS], tm_linear1_q3[NOVIC_MAX_LAYERS], tm_linear2_3[NOVIC_MAX_LAYERS];
+  CUtensorMap tm_linear1_q[NOVIC_MAX_LAYERS];            // linear1 with a 32-row box (the cluster block kernel's hidden-column split)
   // maps of the row-owner block kernel: out_proj / linear2 with rows split as 4 i + t (64 KB requests), linear1 as 128 rows x 4 k-blocks
   CUtensorMap tm_out_proj4[NOVIC_MAX_LAYERS], tm_linear1_r3[NOVIC_MAX_LAYERS], tm_linear2_4[NOVIC_MAX_LAYERS];
   CUtensorMap tm_tok3, tm_in_proj3[NOVIC_MAX_LAYERS];   // 3-D maps (kWideKbs k-blocks per request) for the wide-stage decode GEMMs
   CUtensorMap tm_tok3w;                                   // the tied matrix with 256-row boxes (128 x 256 logits tiles)
-  CUtensorMap tm_in_proj3w[NOVIC_MAX_LAYERS];             // in_proj with 256-row boxes (NOVIC_QKV_BN=256)
-  CUtensorMap tm_in_proj3h[NOVIC_MAX_LAYERS];             // in_proj with 64-row boxes (CTA pairs on 256 x 128 tiles: each CTA loads half of the tile's weight rows)
   CUtensorMap tm_embed_mlp, tm_tok, tm_in_proj[NOVIC_MAX_LAYERS], tm_out_proj[NOVIC_MAX_LAYERS], tm_linear1[NOVIC_MAX_LAYERS],
       tm_linear2[NOVIC_MAX_LAYERS];
   // transposed bf16 copies (B operands of the backward dgrad GEMMs: dX = dY * W needs W^T in K-major form)
@@ -536,7 +422,7 @@ struct WeightPtrs {
 struct Workspace {
   // sizes
   int64_t B = 0, nseq = 0, rows = 0, logit_rows = 0;
-  int H = 1, rps = 0, ntiles = 0, hcap = 0, chains = 1;
+  int H = 1, rps = 0, ntiles = 0, hcap = 0;
   // device pointers
   float* ein; __nv_bfloat16* ebf; float* x; __nv_bfloat16 *xn, *xfin, *q, *ao, *hb; __nv_bfloat16* kv;
   LogitPartial* part; float* topv; int* topi;
@@ -565,16 +451,8 @@ struct NovicHandle {
   int device = 0;
   bool weights_set = false;
   bool use_graphs = true;
-  bool attn_v1 = false;
   int attn_early = 1;
-  int attn_cfg = 0;                   // stream-attention shape (tuning): 0 = 16 warps x 3 slots x 4 keys
-  bool attn_stream = true;            // decode steps use attention_stream_kernel (NOVIC_ATTN_STREAM=0: the bulk-ring kernel)
-  bool fuse_ffn = true;
-  bool split_sms = true;
   int num_sms = 148;
-  int max_chains = 1;                 // concurrent sub-batch chains per decode (NOVIC_CHAINS); measured: no gain for greedy on B200
-  cudaStream_t chain_streams[8] = {};
-  cudaEvent_t fork_ev = nullptr, join_ev[8] = {};
   int attn_smem_budget = 200 * 1024;
   DropCfg drop_in{nullptr, 0u, 1.f}, drop_layer{nullptr, 0u, 1.f};   // training dropout (novic_set_dropout); thresh 0 = off
   uint32_t* d_drop_seed = nullptr;    // device word both DropCfg point at (rewritten before every training step)
@@ -688,7 +566,7 @@ AttnParams attention_params(NovicHandle* h, const Workspace& ws, const PassCfg& 
   pa.slot_mul = pc.slot_mul;
   pa.early_loads = h->attn_early;
   pa.scale_log2e = 1.4426950408889634f / sqrtf(static_cast<float>(kHeadDim));
-  pa.stream_hint = g_attn_hint;
+  pa.stream_hint = 1;
   return pa;
 }
 
@@ -697,38 +575,26 @@ int launch_attention(NovicHandle* h, const Workspace& ws, const PassCfg& pc, int
   const AttnParams pa = attention_params(h, ws, pc, l);
   KSpan t(kKAttn, s);
   const int nkeys_step = (pa.prefix_bidir && pc.q0 < pa.P) ? pa.P : pc.q0 + 1;
-  if (h->attn_stream && g_attn_split && pc.nq == 1 && pc.keypad == nullptr && nkeys_step <= kSpMaxKeys &&
-      pc.nseq <= (g_attn_split_max > 0 ? g_attn_split_max : 2 * kSpSeqs * std::max(1, h->num_sms / g_grid_div))) {
-    // small batches: four warps per sequence, one HBM round trip (attention_split_kernel)
+  const int grid_max = std::max(1, h->num_sms / g_grid_div);
+  if (pc.nq == 1 && pc.keypad == nullptr && nkeys_step <= kSpMaxKeys && pc.nseq <= 2 * kSpSeqs * grid_max) {
+    // small batches (up to two waves of CTAs: measured 0.75 against 0.84 ms at 1024 sequences, 1.37 against 0.94 ms at 2048): four warps
+    // per sequence, one HBM round trip (attention_split_kernel)
     CUDA_TRY(launch_k(attention_split_kernel, dim3(static_cast<unsigned>(ceil_div(pc.nseq, kSpSeqs))), dim3(kSpWarps * 32), kSpSmemBytes, s, pa));
-  } else if (h->attn_stream && pc.nq == 1 && pc.keypad == nullptr) {
-    auto go = [&](auto kernel, int warps, int slots, int chunk) {
-      const int grid = static_cast<int>(std::min<int64_t>(std::max(1, h->num_sms / g_grid_div), ceil_div(pc.nseq, warps)));
-      return launch_k(kernel, dim3(grid), dim3(warps * 32), as_smem_bytes(warps, slots, chunk), s, pa);
-    };
-    switch (h->attn_cfg) {
-      case 1: CUDA_TRY(go(attention_stream_kernel_t<12, 2, 8>, 12, 2, 8)); break;
-      case 2: CUDA_TRY(go(attention_stream_kernel_t<16, 2, 6>, 16, 2, 6)); break;
-      case 3: CUDA_TRY(go(attention_stream_kernel_t<8, 3, 8>, 8, 3, 8)); break;
-      case 4: CUDA_TRY(go(attention_stream_kernel_t<24, 2, 4>, 24, 2, 4)); break;
-      case 5: CUDA_TRY(go(attention_stream_kernel_t<14, 3, 4>, 14, 3, 4)); break;   // 28 sequences per CTA = 2 per warp exactly
-      case 6: CUDA_TRY(go(attention_stream_kernel_t<14, 4, 4>, 14, 4, 4)); break;
-      case 7: CUDA_TRY(go(attention_stream_kernel_t<28, 2, 4>, 28, 2, 4)); break;   // one sequence per warp
-      case 8: CUDA_TRY(go(attention_stream_kernel_t<16, 2, 4>, 16, 2, 4)); break;   // 128 KB: can share an SM with a 2-stage row kernel
-      default: CUDA_TRY(go(attention_stream_kernel_t<16, 3, 4>, 16, 3, 4)); break;
-    }
-  } else if (g_attn_prefix && pc.q0 == 0 && pc.nq == c.prefix_len && pc.nq <= kApMaxP && pc.keypad == nullptr && pc.anc == nullptr) {
+  } else if (pc.nq == 1 && pc.keypad == nullptr) {
+    // decode steps: one warp per sequence, 16 warps x 3 slots x 4 keys (attention_stream_kernel_t)
+    const int grid = static_cast<int>(std::min<int64_t>(grid_max, ceil_div(pc.nseq, 16)));
+    CUDA_TRY(launch_k(attention_stream_kernel_t<16, 3, 4>, dim3(grid), dim3(16 * 32), as_smem_bytes(16, 3, 4), s, pa));
+  } else if (pc.q0 == 0 && pc.nq == c.prefix_len && pc.nq <= kApMaxP && pc.keypad == nullptr && pc.anc == nullptr) {
     // prefix pass: a warp per sequence, all P queries against the P prefix keys (attention_prefix_kernel)
-    const int grid = static_cast<int>(std::min<int64_t>(std::max(1, h->num_sms / g_grid_div), ceil_div(pc.nseq, kApWarps)));
+    const int grid = static_cast<int>(std::min<int64_t>(grid_max, ceil_div(pc.nseq, kApWarps)));
     CUDA_TRY(launch_k(attention_prefix_kernel, dim3(grid), dim3(kApWarps * 32), kApSmemBytes, s, pa));
-  } else if (g_attn_tf && pc.q0 == 0 && pc.nq > c.prefix_len && pc.nq <= kAttnBwdMaxS && pc.beams == 1 && pc.slot_mul == 1 && pc.anc == nullptr) {
+  } else if (pc.q0 == 0 && pc.nq > c.prefix_len && pc.nq <= kAttnBwdMaxS && pc.beams == 1 && pc.slot_mul == 1 && pc.anc == nullptr) {
     // teacher-forced passes (forward, score_targets): all positions of a sequence at once on tensor-core tiles
     const unsigned grid = static_cast<unsigned>(ceil_div(static_cast<int64_t>(pc.nseq) * kHeads, kAttnTfWarps));
     attention_tf_kernel<false><<<grid, kAttnTfWarps * 32, kAttnTfSmemBytes, s>>>(pa);
     CUDA_TRY(cudaGetLastError());
-  } else if (h->attn_v1) {
-    attention_kernel<<<static_cast<unsigned>(ceil_div(static_cast<int64_t>(pc.nseq) * pc.nq, kWarpsPerBlock)), kWarpsPerBlock * 32, 0, s>>>(pa);
   } else {
+    // everything else (a prefix longer than kApMaxP, teacher forcing of beams / repeated slots): K / V rows streamed through a bulk-copy ring
     const int nk_max = std::max(c.strictly_causal ? 1 : c.prefix_len, pc.q0 + pc.nq);
     const int stage_bytes = nk_max * 2048;
     const int budget = h->attn_smem_budget;
@@ -736,7 +602,7 @@ int launch_attention(NovicHandle* h, const Workspace& ws, const PassCfg& pc, int
     const int ncons = std::min(kAttnConsumers, nstages);
     nstages = nstages / ncons * ncons;
     const int smem = nstages * stage_bytes + 2 * kAttnMaxStages * 8;
-    const int grid = static_cast<int>(std::min<int64_t>(std::max(1, h->num_sms / g_grid_div), ceil_div(pc.nseq, 2)));
+    const int grid = static_cast<int>(std::min<int64_t>(grid_max, ceil_div(pc.nseq, 2)));
     CUDA_TRY(launch_k(attention_bulk_kernel, dim3(grid), dim3(kAttnThreads), smem, s, pa, nstages, stage_bytes, ncons));
   }
   ++g_launches;
@@ -746,107 +612,42 @@ int launch_attention(NovicHandle* h, const Workspace& ws, const PassCfg& pc, int
 int run_layers(NovicHandle* h, const Workspace& ws, const PassCfg& pc, cudaStream_t s) {
   const NovicCfg& c = h->cfg;
   const int L = c.num_layers, S = h->S(), M = pc.M;
-  CUtensorMap tm_xn, tm_ao, tm_hb;
-  if (make_tmap(&tm_xn, ws.xn, M, kE, kBlockM)) return 1;
+  CUtensorMap tm_ao, tm_xn3, tm_ao32, tm_ao64r, tm_x_st;
   if (make_tmap(&tm_ao, ws.ao, M, kE, kBlockM)) return 1;
-  if (make_tmap(&tm_hb, ws.hb, M, c.ffn_dim, kBlockM)) return 1;
-  CUtensorMap tm_xn3, tm_ao64;
   if (make_tmap3(&tm_xn3, ws.xn, M, kE, kBlockM, kWideKbs)) return 1;
-  if (make_tmap3(&tm_ao64, ws.ao, M, kE, kHbRows, 2)) return 1;
-  CUtensorMap tm_ao32;
   if (make_tmap3(&tm_ao32, ws.ao, M, kE, kBrRows, kE / kBlockK)) return 1;
-  CUtensorMap tm_ao64r;
   if (make_tmap3(&tm_ao64r, ws.ao, M, kE, kB64Rows, kE / kBlockK)) return 1;
+  if (make_tmap_xblk(&tm_x_st, ws.x, static_cast<int64_t>(ceil_div(M, 32)) * 32)) return 1;
   // 64 rows per CTA once 32-row CTAs need more than one wave (g_block_rows64_min, NOVIC_BLOCK_ROWS64_MIN; 0 = never)
   const bool rows64 = g_block_rows64_min > 0 && M >= g_block_rows64_min;
-  CUtensorMap tm_x_st;
-  if (make_tmap_xblk(&tm_x_st, ws.x, static_cast<int64_t>(ceil_div(M, 32)) * 32)) return 1;
   const size_t kv_layer = static_cast<size_t>(ws.nseq) * S * kE;
-  const bool block_fused = g_fuse_block && h->fuse_ffn && c.ffn_dim == kFfnDim;
-  const bool qkv_tail = block_fused && g_fuse_qkv && g_wide_gemm;     // layer l + 1's QKV projection in the tail of layer l's block kernel
-  auto qkv_params = [&](int l) {
-    __nv_bfloat16* kc = ws.kv + (static_cast<size_t>(l) * 2 + 0) * kv_layer;
-    __nv_bfloat16* vc = ws.kv + (static_cast<size_t>(l) * 2 + 1) * kv_layer;
-    return EpiQKV::Params{ws.q, kc, vc, pc.nq, pc.q0, pc.slot_mul, S, (g_attn_hint & 2) ? 1 : 0};
-  };
   for (int l = 0; l < L; ++l) {
-    if (l == 0 || !qkv_tail) {
-      const EpiQKV::Params pq = qkv_params(l);
-      if (g_wide_gemm) {
-        KSpan t(kKQkv, s);
-        if (g_qkv_ws && kE == kWsKb * kBlockK && ceil_div(M, kBlockM) * g_qkv_ws_div >= 2 * (g_num_sms / g_grid_div / (3 * kE / kTileN))) {   // weight-stationary: >= 2 (NOVIC_QKV_WS_DIV: 2 / div) row blocks per CTA
-          if (g_qkv_ws == 2) {
-            if (launch_gemm_ws2<EpiQKV>(s, tm_xn3, h->w.tm_in_proj3h[l], M, 3 * kE, pq, g_early_b)) return 1;
-          } else if (g_qkv_ws_stages == 3) {
-            if (launch_gemm_ws<EpiQKV, 3>(s, tm_xn3, h->w.tm_in_proj3[l], M, 3 * kE, pq, g_early_b, &tm_xn)) return 1;
-          } else if (launch_gemm_ws<EpiQKV, 2>(s, tm_xn3, h->w.tm_in_proj3[l], M, 3 * kE, pq, g_early_b, &tm_xn)) return 1;
-        } else if (g_qkv_bn == 512 && ceil_div(M, kBlockM) * (3 * kE / 256) >= g_num_sms) {            // CTA pairs, 256 x 256 tiles
-          if (launch_gemm2<EpiQKV, 3>(s, tm_xn3, h->w.tm_in_proj3[l], M, 3 * kE, kE, pq, g_early_b)) return 1;
-        } else if (g_qkv_bn == 384 && ceil_div(M, 2 * kBlockM) * (3 * kE / 128) >= g_num_sms / 2) {   // CTA pairs, 256 x 128 tiles
-          if (launch_gemm2<EpiQKV, 4, 128>(s, tm_xn3, h->w.tm_in_proj3h[l], M, 3 * kE, kE, pq, g_early_b)) return 1;
-        } else if (g_qkv_bn == 256 && ceil_div(M, kBlockM) * (3 * kE / 256) >= g_num_sms) {
-          if (launch_gemm<EpiQKV, 2, kWideKbs, 256>(s, tm_xn3, h->w.tm_in_proj3w[l], M, 3 * kE, kE, pq, 1, g_early_b)) return 1;
-        } else if (launch_gemm<EpiQKV, kWideStages, kWideKbs>(s, tm_xn3, h->w.tm_in_proj3[l], M, 3 * kE, kE, pq, 1, g_early_b)) return 1;
-      } else {
-        KSpan t(kKQkv, s);
-        if (launch_gemm<EpiQKV, kStagesQKV>(s, tm_xn, h->w.tm_in_proj[l], M, 3 * kE, kE, pq, 1, g_early_b)) return 1;
-      }
+    {
+      __nv_bfloat16* kc = ws.kv + (static_cast<size_t>(l) * 2 + 0) * kv_layer;
+      __nv_bfloat16* vc = ws.kv + (static_cast<size_t>(l) * 2 + 1) * kv_layer;
+      const EpiQKV::Params pq{ws.q, kc, vc, pc.nq, pc.q0, pc.slot_mul, S, 0};
+      KSpan t(kKQkv, s);
+      // weight-stationary: each CTA keeps one 128-column tile of in_proj resident and walks the row blocks; it beats the generic persistent
+      // kernel at every size measured (QKV class 0.52 -> 0.42 ms at 128 rows, 0.55 -> 0.45 at 512, 0.58 -> 0.47 at 1024, 0.82 -> 0.69 at 2048)
+      if (g_qkv_ws) {
+        if (launch_gemm_ws<EpiQKV>(s, tm_xn3, h->w.tm_in_proj3[l], M, 3 * kE, pq, true)) return 1;
+      } else if (launch_gemm<EpiQKV, kWideStages, kWideKbs>(s, tm_xn3, h->w.tm_in_proj3[l], M, 3 * kE, kE, pq, 1, true)) return 1;
     }
-    // decode steps (one query per sequence, no key padding) with the row-owner block kernel: the attention runs inside it
-    const bool attn_in_block = block_fused && !qkv_tail && (g_block_rows == 32 || g_block_rows == 0) && g_fuse_attn && h->attn_stream && pc.nq == 1 &&
-                               pc.keypad == nullptr;
-    if (!attn_in_block && launch_attention(h, ws, pc, l, s)) return 1;
-    if (block_fused) {
-      FusedBlockParams fb{};
-      fb.x = ws.x; fb.gain_mid = h->w.norm2[l]; fb.eps = c.ln_eps;
-      if (l + 1 < L) {
-        fb.xn = ws.xn; fb.gain_out = h->w.norm1[l + 1];
-        if (qkv_tail) { fb.qkv_tail = 1; fb.qkv = qkv_params(l + 1); }
-      } else {
-        fb.gain_out = h->w.final_norm;
-        fb.xn = pc.remap_in > 0 ? ws.xfin : ws.xn;
-        fb.remap_rows_in = pc.remap_in; fb.remap_skip = pc.remap_skip; fb.remap_rows_out = pc.remap_out;
-      }
-      KSpan t(kKFfn2, s);
-      if ((g_block_rows == 32 || g_block_rows == 0) && !fb.qkv_tail) {
-        const AttnParams pa = attention_params(h, ws, pc, l);
-        if (launch_block_rows(s, tm_ao32, h->w.tm_out_proj4[l], h->w.tm_linear1_r3[l], h->w.tm_linear2_4[l], tm_x_st, M, fb, attn_in_block ? &pa : nullptr,
-                              (rows64 && !attn_in_block) ? &tm_ao64r : nullptr)) return 1;
-        continue;
-      }
-      if ((g_block_rows == 64 || (g_block_rows <= 0 && M <= kBlock64MaxRows)) && !fb.qkv_tail) {
-        if (launch_outproj_ffn64(s, tm_ao64, h->w.tm_out_proj3[l], h->w.tm_linear1_q3[l], h->w.tm_linear2_3[l], M, fb)) return 1;
-        continue;
-      }
-      if (g_ffn1_ksplit && !fb.qkv_tail) {
-        if (launch_outproj_ffn_ks(s, tm_ao, h->w.tm_out_proj[l], h->w.tm_linear1[l], h->w.tm_linear2[l], M, fb)) return 1;
-        continue;
-      }
-      if (launch_outproj_ffn(s, tm_ao, h->w.tm_out_proj[l], h->w.tm_linear1_q[l], h->w.tm_linear2[l], h->w.tm_in_proj3[l + 1 < L ? l + 1 : l], M, fb)) return 1;
-      continue;
-    }
-    RowParams po{};
-    po.x = ws.x; po.xn = ws.xn; po.gain = h->w.norm2[l]; po.pos = nullptr; po.eps = c.ln_eps;
-    { KSpan t(kKOutProj, s); if (launch_rowln(s, tm_ao, h->w.tm_out_proj[l], M, kE, kE, po)) return 1; }
-    RowParams pf{};
-    pf.x = ws.x; pf.pos = nullptr; pf.eps = c.ln_eps;
+    if (launch_attention(h, ws, pc, l, s)) return 1;
+    FusedBlockParams fb{};
+    fb.x = ws.x; fb.gain_mid = h->w.norm2[l]; fb.eps = c.ln_eps;
     if (l + 1 < L) {
-      pf.xn = ws.xn; pf.gain = h->w.norm1[l + 1];
+      fb.xn = ws.xn; fb.gain_out = h->w.norm1[l + 1];
     } else {
-      pf.gain = h->w.final_norm;
-      pf.xn = pc.remap_in > 0 ? ws.xfin : ws.xn;
-      pf.remap_rows_in = pc.remap_in; pf.remap_skip = pc.remap_skip; pf.remap_rows_out = pc.remap_out;
+      fb.gain_out = h->w.final_norm;
+      fb.xn = pc.remap_in > 0 ? ws.xfin : ws.xn;
+      fb.remap_rows_in = pc.remap_in; fb.remap_skip = pc.remap_skip; fb.remap_rows_out = pc.remap_out;
     }
-    if (h->fuse_ffn) {
-      // note: the fused kernel reads LN2(x) rows from ws.xn and (unless remapped) writes the next LayerNorm's rows to ws.xn:
-      // every CTA of a cluster reads its whole 128-row A tile before any of them writes (the writes come after two
-      // cluster barriers that follow the last MMA), and different clusters own different rows.
-      KSpan t(kKFfn2, s);
-      if (launch_ffn(s, tm_xn, g_split_ffn ? h->w.tm_linear1_q[l] : h->w.tm_linear1[l], h->w.tm_linear2[l], M, pf, g_split_ffn)) return 1;
-    } else {
-      EpiGelu::Params pg{ws.hb, c.ffn_dim};
-      { KSpan t(kKFfn1, s); if (launch_gemm<EpiGelu, kStagesGelu>(s, tm_xn, h->w.tm_linear1[l], M, c.ffn_dim, kE, pg)) return 1; }
-      { KSpan t(kKFfn2, s); if (launch_rowln(s, tm_hb, h->w.tm_linear2[l], M, kE, c.ffn_dim, pf)) return 1; }
+    KSpan t(kKFfn2, s);
+    if (g_block_rows == 128) {
+      if (launch_outproj_ffn(s, tm_ao, h->w.tm_out_proj[l], h->w.tm_linear1_q[l], h->w.tm_linear2[l], M, fb)) return 1;
+    } else if (launch_block_rows(s, tm_ao32, h->w.tm_out_proj4[l], h->w.tm_linear1_r3[l], h->w.tm_linear2_4[l], tm_x_st, M, fb, rows64 ? &tm_ao64r : nullptr)) {
+      return 1;
     }
   }
   CUDA_TRY(cudaGetLastError());
@@ -885,7 +686,7 @@ int launch_logits(NovicHandle* h, const Workspace& ws, const __nv_bfloat16* a, i
                   const long long* target, float inv_tau, int ban_eos, bool mask_lse, int allow_mod, cudaStream_t s,
                   const float* bias = nullptr) {
   CUtensorMap tm_a;
-  if (g_wide_gemm ? make_tmap3(&tm_a, a, M, kE, kBlockM, kWideKbs) : make_tmap(&tm_a, a, M, kE, kBlockM)) return 1;
+  if (make_tmap3(&tm_a, a, M, kE, kBlockM, kWideKbs)) return 1;
   typename EpiLogits<HCAP, MASKED, BIAS>::Params pl;
   pl.edge0 = ws.allow_edge0; pl.bias = bias; pl.tau = 1.0f / inv_tau;
   pl.logits = logits; pl.ld_logits = ld_logits; pl.part = ws.part; pl.topv = ws.topv; pl.topi = ws.topi; pl.target = target;
@@ -893,26 +694,16 @@ int launch_logits(NovicHandle* h, const Workspace& ws, const __nv_bfloat16* a, i
   pl.want_sumx = h->cfg.label_smoothing != 0.f ? 1 : 0;
   pl.allow = MASKED ? ws.allow : nullptr; pl.allow_ld = ws.allow_words; pl.allow_mod = allow_mod; pl.mask_lse = mask_lse ? 1 : 0;
   KSpan t(kKLogits, s);
-  if constexpr ((HCAP == 4 || HCAP == 12) && !BIAS) {
-    // beam search with up to 3 / up to 11 beams (HCAP = 4 / 12 candidates per 64-column slice), guided or not: the same 128 x 256 tiles with 16
-    // epilogue warps as the greedy GEMM - the top-k epilogue on two warps per scheduler ran at 0.27 of the tensor roof (7.1 of the 29.8 ms
-    // of BASELINE config #3)
+  if constexpr ((HCAP == 0 && !MASKED && !BIAS) || ((HCAP == 4 || HCAP == 12) && !BIAS)) {
+    // 128 x 256 tiles with 16 epilogue warps (0.75 of the operand bytes per FLOP): the plain arg-max / log-sum-exp epilogue of greedy decoding
+    // and teacher forcing, and beam search with up to 3 / up to 11 beams (HCAP = 4 / 12 candidates per 64-column slice), guided or not - the
+    // top-k epilogue on two warps per scheduler ran at 0.27 of the tensor roof (7.1 of the 29.8 ms of BASELINE config #3).  Needs the same
+    // number of 64-column slices per row as the 128-column tiling the workspace was planned for, and at least a wave of tiles.
     const int V = h->cfg.vocab_size;
-    if (g_wide_gemm && g_logits_bn >= 256 && g_logits_ew == 16 && 4 * ceil_div(V, 256) == ws.ntiles && ceil_div(M, kBlockM) * ceil_div(V, 256) >= g_num_sms)
-      return launch_gemm<EpiLogits<HCAP, MASKED, false>, 2, kWideKbs, 256, 16>(s, tm_a, h->w.tm_tok3w, M, V, kE, pl, 1, g_early_b);
+    if (g_logits_bn >= 256 && 4 * ceil_div(V, 256) == ws.ntiles && ceil_div(M, kBlockM) * ceil_div(V, 256) >= g_num_sms)
+      return launch_gemm<EpiLogits<HCAP, MASKED, false>, 2, kWideKbs, 256, 16>(s, tm_a, h->w.tm_tok3w, M, V, kE, pl, 1, true);
   }
-  if constexpr (HCAP == 0 && !MASKED && !BIAS) {
-    // 128 x 256 tiles (0.75 of the operand bytes per FLOP): the plain arg-max / log-sum-exp epilogue of greedy decoding and teacher forcing.
-    // Needs the same number of 64-column slices per row as the 128-column tiling the workspace was planned for, and at least a wave of tiles.
-    const int V = h->cfg.vocab_size;
-    if (g_wide_gemm && g_logits_bn == 512 && 4 * ceil_div(V, 256) == ws.ntiles && ceil_div(M, kBlockM) * ceil_div(V, 256) >= g_num_sms)
-      return launch_gemm2<EpiLogits<0, false, false>, 3>(s, tm_a, h->w.tm_tok3, M, V, kE, pl, g_early_b);      // CTA pairs, 256 x 256 tiles
-    if (g_wide_gemm && g_logits_bn >= 256 && 4 * ceil_div(V, 256) == ws.ntiles && ceil_div(M, kBlockM) * ceil_div(V, 256) >= g_num_sms)
-      return g_logits_ew == 16 ? launch_gemm<EpiLogits<0, false, false>, 2, kWideKbs, 256, 16>(s, tm_a, h->w.tm_tok3w, M, V, kE, pl, 1, g_early_b)
-                               : launch_gemm<EpiLogits<0, false, false>, 2, kWideKbs, 256>(s, tm_a, h->w.tm_tok3w, M, V, kE, pl, 1, g_early_b);
-  }
-  if (g_wide_gemm) return launch_gemm<EpiLogits<HCAP, MASKED, BIAS>, kWideStages, kWideKbs>(s, tm_a, h->w.tm_tok3, M, h->cfg.vocab_size, kE, pl, 1, g_early_b);
-  return launch_gemm<EpiLogits<HCAP, MASKED, BIAS>, kStagesLogits>(s, tm_a, h->w.tm_tok, M, h->cfg.vocab_size, kE, pl, 1, g_early_b);
+  return launch_gemm<EpiLogits<HCAP, MASKED, BIAS>, kWideStages, kWideKbs>(s, tm_a, h->w.tm_tok3, M, h->cfg.vocab_size, kE, pl, 1, true);
 }
 
 int run_logits(NovicHandle* h, const Workspace& ws, const __nv_bfloat16* a, int M, float* logits, long long ld_logits,
@@ -949,7 +740,7 @@ int launch_guide_mask(const Workspace& ws, const GuideCfg& g, const int* node, i
 
 int enqueue_greedy(NovicHandle* h, const Workspace& ws, float tau, float alpha, float* logits, const GuideCfg& guide, cudaStream_t s) {
   const NovicCfg& c = h->cfg;
-  g_grid_div = h->split_sms ? ws.chains : 1;
+  g_grid_div = 1;
   const int B = static_cast<int>(ws.B), P = c.prefix_len, G = h->G(), V = c.vocab_size;
   const float inv_tau = 1.0f / tau;
   CUDA_TRY(cudaMemsetAsync(ws.g_done, 0, B, s));
@@ -1000,7 +791,7 @@ void launch_select_beam(const Workspace& ws, NovicHandle* h, int step, float inv
 
 int enqueue_beam(NovicHandle* h, const Workspace& ws, float tau, float alpha, const GuideCfg& guide, cudaStream_t s) {
   const NovicCfg& c = h->cfg;
-  g_grid_div = h->split_sms ? ws.chains : 1;
+  g_grid_div = 1;
   const int B = static_cast<int>(ws.B), H = ws.H, P = c.prefix_len, G = h->G();
   const int A = B * H;
   const float inv_tau = 1.0f / tau;
@@ -1035,51 +826,11 @@ int enqueue_beam(NovicHandle* h, const Workspace& ws, float tau, float alpha, co
 
 #include "train_host.inc"
 
-// A decode is latency-bound per kernel (~500 dependent launches of 5-20 us); independent sub-batches ("chains") are
-// enqueued on parallel streams / graph branches so that one chain's launch gaps, pipeline fill and epilogues overlap
-// another chain's work.  Sequences are independent, so results do not depend on the split.
-int choose_chains(const NovicHandle* h, int64_t B, int seqs_per_embed) {
-  const int64_t nseq = B * seqs_per_embed;
-  int n = 1;
-  while (n < h->max_chains && nseq / (n * 2) >= 512 && B / (n * 2) >= 1) n *= 2;
-  return n;
-}
-
-struct ChainPlan {
-  int n = 1;
-  int64_t b0[8], nb[8];
-  Workspace ws[8];
-  size_t bytes = 0;
-};
-
-void plan_chains(const NovicHandle* h, int64_t B, int H, int rps, char* base, ChainPlan* cp) {
-  cp->n = rps > 0 ? 1 : choose_chains(h, B, H);
-  size_t off = 0;
-  for (int i = 0; i < cp->n; ++i) {
-    cp->b0[i] = B * i / cp->n;
-    cp->nb[i] = B * (i + 1) / cp->n - cp->b0[i];
-    plan_workspace(h, cp->nb[i], H, rps, base + off, &cp->ws[i]);
-    cp->ws[i].chains = cp->n;
-    off += align_up(cp->ws[i].bytes, 1024);
-  }
-  cp->bytes = off;
-}
-
-// Fork `n` chains from stream `s` (chain 0 runs on s itself), run fn(i, stream_i), join back into s.
-template <class F>
-int run_chains(NovicHandle* h, cudaStream_t s, int n, F&& fn) {
-  if (n == 1) return fn(0, s);
-  CUDA_TRY(cudaEventRecord(h->fork_ev, s));
-  for (int i = 1; i < n; ++i) CUDA_TRY(cudaStreamWaitEvent(h->chain_streams[i], h->fork_ev, 0));
-  for (int i = 0; i < n; ++i) {
-    cudaStream_t cs = i == 0 ? s : h->chain_streams[i];
-    if (fn(i, cs)) return 1;
-    if (i > 0) {
-      CUDA_TRY(cudaEventRecord(h->join_ev[i], cs));
-      CUDA_TRY(cudaStreamWaitEvent(s, h->join_ev[i], 0));
-    }
-  }
-  return 0;
+// The decode workspace: plan_workspace's buffers, padded to a multiple of 1 KB.
+size_t decode_workspace_bytes(const NovicHandle* h, int64_t B, int H, int rps) {
+  Workspace ws;
+  plan_workspace(h, B, H, rps, nullptr, &ws);
+  return align_up(ws.bytes, 1024);
 }
 
 int check_ready(NovicHandle* h) {
@@ -1158,13 +909,10 @@ int novic_create(const NovicCfg* cfg, NovicHandle** out) {
   CUDA_TRY(cudaGetDeviceProperties(&prop, dev));
   if (prop.major != 10) return fail("device %d is sm_%d%d; novic_b200 kernels are sm_100a only", dev, prop.major, prop.minor);
   if (load_driver_entry()) return 1;
-  if (set_gemm_attr<EpiQKV, kStagesQKV>() || set_gemm_attr<EpiGelu, kStagesGelu>() || set_rowln_attr() ||
-      set_gemm_attr<EpiLogits<0>, kStagesLogits>() || set_gemm_attr<EpiLogits<4>, kStagesLogits>() ||
-      set_gemm_attr<EpiLogits<16>, kStagesLogits>() || set_gemm_attr<EpiLogits<0, true>, kStagesLogits>() ||
-      set_gemm_attr<EpiLogits<4, true>, kStagesLogits>() || set_gemm_attr<EpiLogits<16, true>, kStagesLogits>() ||
-      set_gemm_attr<EpiLogits<4, true, true>, kStagesLogits>() || set_gemm_attr<EpiLogits<16, true, true>, kStagesLogits>() ||
-      set_gemm_attr<EpiQKV, kWideStages, kWideKbs>() || set_gemm_attr<EpiQKV, 2, kWideKbs, 256>() || set_gemm2_attr<EpiQKV, 3>() || set_gemm2_attr<EpiQKV, 4, 128>() || set_gemm_ws_attr<EpiQKV, 2>() || set_gemm_ws_attr<EpiQKV, 3>() || set_gemm_ws2_attr<EpiQKV>() || set_gemm2_attr<EpiLogits<0>, 3>() || set_gemm_attr<EpiLogits<0>, 2, kWideKbs, 256>() || set_gemm_attr<EpiLogits<0>, 2, kWideKbs, 256, 16>() || set_gemm_attr<EpiLogits<4>, 2, kWideKbs, 256, 16>() || set_gemm_attr<EpiLogits<12>, 2, kWideKbs, 256, 16>() || set_gemm_attr<EpiLogits<4, true>, 2, kWideKbs, 256, 16>() || set_gemm_attr<EpiLogits<12, true>, 2, kWideKbs, 256, 16>() ||
-      set_gemm_attr<EpiLogits<12>, kStagesLogits>() || set_gemm_attr<EpiLogits<12, true>, kStagesLogits>() || set_gemm_attr<EpiLogits<12, true, true>, kStagesLogits>() ||
+  if (set_gemm_attr<EpiQKV, kStagesQKV>() || set_rowln_attr() || set_gemm_attr<EpiLogits<0>, kStagesLogits>() ||
+      set_gemm_attr<EpiQKV, kWideStages, kWideKbs>() || set_gemm_ws_attr<EpiQKV>() || set_gemm_attr<EpiLogits<0>, 2, kWideKbs, 256, 16>() ||
+      set_gemm_attr<EpiLogits<4>, 2, kWideKbs, 256, 16>() || set_gemm_attr<EpiLogits<12>, 2, kWideKbs, 256, 16>() ||
+      set_gemm_attr<EpiLogits<4, true>, 2, kWideKbs, 256, 16>() || set_gemm_attr<EpiLogits<12, true>, 2, kWideKbs, 256, 16>() ||
       set_gemm_attr<EpiLogits<12>, kWideStages, kWideKbs>() || set_gemm_attr<EpiLogits<12, true>, kWideStages, kWideKbs>() ||
       set_gemm_attr<EpiLogits<12, true, true>, kWideStages, kWideKbs>() ||
       set_gemm_attr<EpiLogits<0>, kWideStages, kWideKbs>() || set_gemm_attr<EpiLogits<4>, kWideStages, kWideKbs>() ||
@@ -1197,54 +945,15 @@ int novic_create(const NovicCfg* cfg, NovicHandle** out) {
   CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<16, 3, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(16, 3, 4)));
   CUDA_TRY(cudaFuncSetAttribute(attention_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSpSmemBytes));
   CUDA_TRY(cudaFuncSetAttribute(attention_prefix_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kApSmemBytes));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<12, 2, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(12, 2, 8)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<16, 2, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(16, 2, 6)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<8, 3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(8, 3, 8)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<24, 2, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(24, 2, 4)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<14, 3, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(14, 3, 4)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<14, 4, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(14, 4, 4)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<28, 2, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(28, 2, 4)));
-  CUDA_TRY(cudaFuncSetAttribute(attention_stream_kernel_t<16, 2, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, as_smem_bytes(16, 2, 4)));
-  if (const char* e12 = getenv("NOVIC_ATTN_CFG")) h->attn_cfg = atoi(e12);
-  if (const char* e14 = getenv("NOVIC_WIDE_GEMM")) g_wide_gemm = e14[0] != '0';
-  if (const char* e21 = getenv("NOVIC_LOGITS_BN")) g_logits_bn = atoi(e21);
-  if (const char* e28 = getenv("NOVIC_LOGITS_EW")) g_logits_ew = atoi(e28);
-  if (const char* e15 = getenv("NOVIC_EARLY_B")) g_early_b = e15[0] != '0';
-  if (const char* e16 = getenv("NOVIC_SPLIT_FFN")) g_split_ffn = e16[0] != '0';
-  if (const char* e17 = getenv("NOVIC_ROW_STAGES")) g_row_stages = atoi(e17);
-  if (const char* e18 = getenv("NOVIC_ATTN_HINT")) g_attn_hint = atoi(e18);
-  if (const char* e19 = getenv("NOVIC_ATTN_TF")) g_attn_tf = atoi(e19) != 0;
-  if (const char* e22 = getenv("NOVIC_FUSE_BLOCK")) g_fuse_block = e22[0] != '0';
-  if (const char* e23 = getenv("NOVIC_FUSE_QKV")) g_fuse_qkv = e23[0] != '0';
-  if (const char* e24 = getenv("NOVIC_QKV_BN")) g_qkv_bn = atoi(e24);
-  if (const char* e27 = getenv("NOVIC_QKV_WS")) g_qkv_ws = atoi(e27);
-  if (const char* e27b = getenv("NOVIC_QKV_MC")) g_qkv_mc = atoi(e27b);
-  if (const char* e27c = getenv("NOVIC_QKV_PER_TILE")) g_qkv_per_tile = atoi(e27c);
-  if (const char* e27d = getenv("NOVIC_WGRAD_MN")) g_wgrad_mn = atoi(e27d) != 0;
-  if (const char* e25 = getenv("NOVIC_BLOCK_ROWS")) g_block_rows = atoi(e25);
-  if (const char* e25b = getenv("NOVIC_FUSE_ATTN")) g_fuse_attn = e25b[0] != '0';
-  if (const char* e25d = getenv("NOVIC_ATTN_SPLIT")) g_attn_split = e25d[0] != '0';
-  if (const char* e25h = getenv("NOVIC_ATTN_PREFIX")) g_attn_prefix = e25h[0] != '0';
-  if (const char* e25j = getenv("NOVIC_VIT_DIRECT")) g_vit_direct = atoi(e25j) != 0 ? 1 : 0;
-  if (const char* e25i = getenv("NOVIC_QKV_WS_DIV")) g_qkv_ws_div = std::max(1, atoi(e25i));
-  if (const char* e25g = getenv("NOVIC_QKV_WS_STAGES")) g_qkv_ws_stages = atoi(e25g) == 2 ? 2 : 3;
-  if (const char* e25e = getenv("NOVIC_ATTN_SPLIT_MAX")) g_attn_split_max = atoi(e25e);
-  if (const char* e25c = getenv("NOVIC_BLOCK_ROWS64_MIN")) g_block_rows64_min = atoi(e25c);
-  if (const char* e26 = getenv("NOVIC_BLOCK64_PAD")) g_block64_pad = atoi(e26);
-  if (const char* e29 = getenv("NOVIC_FFN1_KSPLIT")) g_ffn1_ksplit = e29[0] != '0';
-  if (const char* e13 = getenv("NOVIC_SKIP_CLASSES")) g_skip_classes = static_cast<unsigned>(strtoul(e13, nullptr, 0));
-  if (const char* e1 = getenv("NOVIC_ATTN_V1")) h->attn_v1 = e1[0] == '1';
-  if (const char* e7 = getenv("NOVIC_ATTN_STREAM")) h->attn_stream = e7[0] != '0';
-  if (const char* e9 = getenv("NOVIC_ATTN_EARLY")) h->attn_early = atoi(e9);
-  if (const char* e6 = getenv("NOVIC_NO_PDL")) g_use_pdl = e6[0] != '1';
-  if (const char* e5 = getenv("NOVIC_NO_SM_SPLIT")) h->split_sms = e5[0] != '1';
-  if (const char* e4 = getenv("NOVIC_NO_FFN_FUSION")) h->fuse_ffn = e4[0] != '1';
-  if (const char* e3 = getenv("NOVIC_CHAINS")) h->max_chains = std::max(1, std::min(8, atoi(e3)));
-  for (int i = 0; i < 8; ++i) {
-    CUDA_TRY(cudaStreamCreateWithFlags(&h->chain_streams[i], cudaStreamNonBlocking));
-    CUDA_TRY(cudaEventCreateWithFlags(&h->join_ev[i], cudaEventDisableTiming));
-  }
-  CUDA_TRY(cudaEventCreateWithFlags(&h->fork_ev, cudaEventDisableTiming));
+  if (const char* e = getenv("NOVIC_LOGITS_BN")) g_logits_bn = atoi(e);
+  if (const char* e = getenv("NOVIC_QKV_WS")) g_qkv_ws = atoi(e) != 0 ? 1 : 0;
+  if (const char* e = getenv("NOVIC_WGRAD_MN")) g_wgrad_mn = atoi(e) != 0;
+  if (const char* e = getenv("NOVIC_BLOCK_ROWS")) g_block_rows = atoi(e);
+  if (const char* e = getenv("NOVIC_VIT_DIRECT")) g_vit_direct = atoi(e) != 0 ? 1 : 0;
+  if (const char* e = getenv("NOVIC_BLOCK_ROWS64_MIN")) g_block_rows64_min = atoi(e);
+  if (const char* e = getenv("NOVIC_SKIP_CLASSES")) g_skip_classes = static_cast<unsigned>(strtoul(e, nullptr, 0));
+  if (const char* e = getenv("NOVIC_ATTN_EARLY")) h->attn_early = atoi(e);
+  if (const char* e = getenv("NOVIC_NO_PDL")) g_use_pdl = e[0] != '1';
   const char* env = getenv("NOVIC_NO_GRAPHS");
   if (env != nullptr && env[0] == '1') h->use_graphs = false;
   *out = h;
@@ -1257,8 +966,6 @@ int novic_destroy(NovicHandle* h) {
   for (auto& kv : h->train_graph_cache) { cudaGraphExecDestroy(kv.second.first); if (kv.second.second) cudaGraphExecDestroy(kv.second.second); }
   if (h->d_drop_seed) cudaFree(h->d_drop_seed);
   if (h->capture_stream) cudaStreamDestroy(h->capture_stream);
-  for (int i = 0; i < 8; ++i) { if (h->chain_streams[i]) cudaStreamDestroy(h->chain_streams[i]); if (h->join_ev[i]) cudaEventDestroy(h->join_ev[i]); }
-  if (h->fork_ev) cudaEventDestroy(h->fork_ev);
   if (h->h_flags) cudaFreeHost(h->h_flags);
   delete h;
   return 0;
@@ -1393,16 +1100,11 @@ int novic_set_weights(NovicHandle* h, const NovicWeights* w, void* wbuf, size_t 
   for (size_t l = 0; l < L; ++l) {
     if (make_tmap(&o.tm_in_proj[l], o.in_proj[l], 3 * E, E, 128)) return 1;
     if (make_tmap3(&o.tm_in_proj3[l], o.in_proj[l], 3 * E, E, 128, kWideKbs)) return 1;
-    if (make_tmap3(&o.tm_in_proj3w[l], o.in_proj[l], 3 * E, E, 256, kWideKbs)) return 1;
-    if (make_tmap3(&o.tm_in_proj3h[l], o.in_proj[l], 3 * E, E, 64, kWideKbs)) return 1;
     if (make_tmap(&o.tm_out_proj[l], o.out_proj[l], E, E, kRowBN)) return 1;
     if (make_tmap(&o.tm_linear1[l], o.linear1[l], K, E, 128)) return 1;
     if (make_tmap(&o.tm_linear1_q[l], o.linear1[l], K, E, kFfnDim / kRowCluster)) return 1;
     if (make_tmap(&o.tm_linear2[l], o.linear2[l], E, K, kRowBN)) return 1;
     if (K == kFfnDim) {
-      if (make_tmap3(&o.tm_out_proj3[l], o.out_proj[l], E, E, kRowBN, 2)) return 1;
-      if (make_tmap3(&o.tm_linear1_q3[l], o.linear1[l], K, E, kFfnDim / kRowCluster, E / kBlockK)) return 1;
-      if (make_tmap3(&o.tm_linear2_3[l], o.linear2[l], E, K, kRowBN, K / kBlockK)) return 1;
       if (make_tmap4_perm(&o.tm_out_proj4[l], o.out_proj[l], E, E, 1, 4)) return 1;
       if (make_tmap3(&o.tm_linear1_r3[l], o.linear1[l], K, E, 128, 4)) return 1;
       if (make_tmap4_perm(&o.tm_linear2_4[l], o.linear2[l], E, K, 2, 2)) return 1;
@@ -1424,9 +1126,7 @@ int novic_set_weights(NovicHandle* h, const NovicWeights* w, void* wbuf, size_t 
 }
 
 size_t novic_workspace_bytes(const NovicHandle* h, int64_t num_embeds, int32_t seqs_per_embed, int32_t rows_per_seq) {
-  ChainPlan cp;
-  plan_chains(h, num_embeds, seqs_per_embed, rows_per_seq, nullptr, &cp);
-  return cp.bytes;
+  return decode_workspace_bytes(h, num_embeds, seqs_per_embed, rows_per_seq);
 }
 
 static int make_guide(const NovicGuide* guide, const NovicHandle* h, GuideCfg* out) {
@@ -1441,7 +1141,7 @@ static int make_guide(const NovicGuide* guide, const NovicHandle* h, GuideCfg* o
   return 0;
 }
 
-// T[0] = max over the chains of the first step whose "every row finished" flag is still set (else G): the number of columns
+// T[0] = max over the workspaces of the first step whose "every row finished" flag is still set (else G): the number of columns
 // the reference returns (embedding_decoder.py:817-820).  Device-side twin of the host loop in novic_generate_greedy.
 struct FlagPtrs { const int* f[8]; int n; };
 __global__ void early_exit_len_kernel(FlagPtrs fp, int G, int* T) {
@@ -1465,48 +1165,35 @@ static int greedy_impl(NovicHandle* h, const float* embed, int64_t B, float temp
   if (B < 1 || B > (1 << 24)) return fail("batch size out of range");
   if (!(temperature > 0.f)) return fail("temperature must be positive");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  ChainPlan cp;
-  plan_chains(h, B, 1, 0, static_cast<char*>(wsbuf), &cp);
-  if (ws_bytes < cp.bytes) return fail("workspace too small: %zu < %zu", ws_bytes, cp.bytes);
-  const int G = h->G(), F = h->cfg.embed_dim, V = h->cfg.vocab_size;
-  for (int i = 0; i < cp.n; ++i)
-    CUDA_TRY(cudaMemcpyAsync(cp.ws[i].ein, embed + cp.b0[i] * F, sizeof(float) * cp.nb[i] * F, cudaMemcpyDeviceToDevice, s));
-  GraphKey key{0, B, cp.n, temperature, length_alpha, wsbuf, gcfg.on ? static_cast<const void*>(gcfg.trie.child_off) : nullptr,
+  Workspace ws;
+  plan_workspace(h, B, 1, 0, static_cast<char*>(wsbuf), &ws);
+  const size_t need = decode_workspace_bytes(h, B, 1, 0);
+  if (ws_bytes < need) return fail("workspace too small: %zu < %zu", ws_bytes, need);
+  const int G = h->G(), F = h->cfg.embed_dim;
+  CUDA_TRY(cudaMemcpyAsync(ws.ein, embed, sizeof(float) * B * F, cudaMemcpyDeviceToDevice, s));
+  GraphKey key{0, B, 1, temperature, length_alpha, wsbuf, gcfg.on ? static_cast<const void*>(gcfg.trie.child_off) : nullptr,
                (gcfg.on ? 1 : 0) | (gcfg.renorm ? 2 : 0)};
   if (gcfg.on) { key.guide_tok = gcfg.trie.child_tok; key.guide_node = gcfg.trie.child_node; key.num_nodes = guide->num_nodes; key.num_edges = guide->num_edges; }
-  if (run_maybe_graph(h, key, logits == nullptr, s, [&](cudaStream_t cs) {
-        return run_chains(h, cs, cp.n, [&](int i, cudaStream_t st) {
-          float* lg = logits != nullptr ? logits + static_cast<size_t>(cp.b0[i]) * G * V : nullptr;
-          return enqueue_greedy(h, cp.ws[i], temperature, length_alpha, lg, gcfg, st);
-        });
-      }))
+  if (run_maybe_graph(h, key, logits == nullptr, s, [&](cudaStream_t cs) { return enqueue_greedy(h, ws, temperature, length_alpha, logits, gcfg, cs); }))
     return 1;
-  for (int i = 0; i < cp.n; ++i) {
-    const Workspace& ws = cp.ws[i];
-    const int64_t b0 = cp.b0[i], nb = cp.nb[i];
-    CUDA_TRY(cudaMemcpyAsync(tok + b0 * G, ws.g_tok, 8 * nb * G, cudaMemcpyDeviceToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(pad + b0 * G, ws.g_pad, nb * G, cudaMemcpyDeviceToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(score + b0, ws.g_score_out, 4 * nb, cudaMemcpyDeviceToDevice, s));
-    if (nll) CUDA_TRY(cudaMemcpyAsync(nll + b0, ws.g_nll, 4 * nb, cudaMemcpyDeviceToDevice, s));
-    if (len) CUDA_TRY(cudaMemcpyAsync(len + b0, ws.g_len, 4 * nb, cudaMemcpyDeviceToDevice, s));
-    if (T_dev == nullptr) CUDA_TRY(cudaMemcpyAsync(h->h_flags + i * (G + 2), ws.flags, sizeof(int) * (G + 2), cudaMemcpyDeviceToHost, s));
-  }
+  CUDA_TRY(cudaMemcpyAsync(tok, ws.g_tok, 8 * B * G, cudaMemcpyDeviceToDevice, s));
+  CUDA_TRY(cudaMemcpyAsync(pad, ws.g_pad, B * G, cudaMemcpyDeviceToDevice, s));
+  CUDA_TRY(cudaMemcpyAsync(score, ws.g_score_out, 4 * B, cudaMemcpyDeviceToDevice, s));
+  if (nll) CUDA_TRY(cudaMemcpyAsync(nll, ws.g_nll, 4 * B, cudaMemcpyDeviceToDevice, s));
+  if (len) CUDA_TRY(cudaMemcpyAsync(len, ws.g_len, 4 * B, cudaMemcpyDeviceToDevice, s));
   if (T_dev != nullptr) {   // asynchronous variant: the early-exit length stays on the device, no host synchronisation
     FlagPtrs fp{};
-    fp.n = cp.n;
-    for (int i = 0; i < cp.n; ++i) fp.f[i] = cp.ws[i].flags;
+    fp.n = 1;
+    fp.f[0] = ws.flags;
     early_exit_len_kernel<<<1, 32, 0, s>>>(fp, G, T_dev);
     ++g_launches;
     CUDA_TRY(cudaGetLastError());
     return 0;
   }
+  CUDA_TRY(cudaMemcpyAsync(h->h_flags, ws.flags, sizeof(int) * (G + 2), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
-  int T = 0;
-  for (int i = 0; i < cp.n; ++i) {
-    int Ti = G;
-    for (int c = 1; c <= G; ++c) if (h->h_flags[i * (G + 2) + c] != 0) { Ti = c; break; }
-    T = std::max(T, Ti);
-  }
+  int T = G;
+  for (int c = 1; c <= G; ++c) if (h->h_flags[c] != 0) { T = c; break; }
   if (T_out) *T_out = T;
   return 0;
 }
@@ -1535,35 +1222,25 @@ int novic_generate_beam(NovicHandle* h, const float* embed, int64_t B, int32_t H
   if (H >= h->cfg.vocab_size) return fail("beam width must be smaller than the vocabulary");
   if (!(temperature > 0.f)) return fail("temperature must be positive");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  ChainPlan cp;
-  plan_chains(h, B, H, 0, static_cast<char*>(wsbuf), &cp);
-  if (ws_bytes < cp.bytes) return fail("workspace too small: %zu < %zu", ws_bytes, cp.bytes);
+  Workspace ws;
+  plan_workspace(h, B, H, 0, static_cast<char*>(wsbuf), &ws);
+  const size_t need = decode_workspace_bytes(h, B, H, 0);
+  if (ws_bytes < need) return fail("workspace too small: %zu < %zu", ws_bytes, need);
   const int G = h->G(), F = h->cfg.embed_dim;
-  for (int i = 0; i < cp.n; ++i)
-    CUDA_TRY(cudaMemcpyAsync(cp.ws[i].ein, embed + cp.b0[i] * F, sizeof(float) * cp.nb[i] * F, cudaMemcpyDeviceToDevice, s));
-  GraphKey key{1, B, H * 16 + cp.n, temperature, length_alpha, wsbuf, gcfg.on ? static_cast<const void*>(gcfg.trie.child_off) : nullptr,
+  CUDA_TRY(cudaMemcpyAsync(ws.ein, embed, sizeof(float) * B * F, cudaMemcpyDeviceToDevice, s));
+  GraphKey key{1, B, H, temperature, length_alpha, wsbuf, gcfg.on ? static_cast<const void*>(gcfg.trie.child_off) : nullptr,
                (gcfg.on ? 1 : 0) | (gcfg.renorm ? 2 : 0), gcfg.bias};
   if (gcfg.on) { key.guide_tok = gcfg.trie.child_tok; key.guide_node = gcfg.trie.child_node; key.num_nodes = guide->num_nodes; key.num_edges = guide->num_edges; }
-  if (run_maybe_graph(h, key, true, s, [&](cudaStream_t cs) {
-        return run_chains(h, cs, cp.n, [&](int i, cudaStream_t st) { return enqueue_beam(h, cp.ws[i], temperature, length_alpha, gcfg, st); });
-      }))
+  if (run_maybe_graph(h, key, true, s, [&](cudaStream_t cs) { return enqueue_beam(h, ws, temperature, length_alpha, gcfg, cs); }))
     return 1;
   const int fin = G & 1;
-  for (int i = 0; i < cp.n; ++i) {
-    const Workspace& ws = cp.ws[i];
-    const int64_t a0 = cp.b0[i] * H;
-    CUDA_TRY(cudaMemcpyAsync(tok + a0 * G, ws.b_tok[fin], 8 * ws.nseq * G, cudaMemcpyDeviceToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(pad + a0 * G, ws.b_pad[fin], ws.nseq * G, cudaMemcpyDeviceToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(score + a0, length_alpha != 0.f ? ws.b_norm : ws.b_score[fin], 4 * ws.nseq, cudaMemcpyDeviceToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(h->h_flags + i * (G + 2), ws.flags, sizeof(int) * (G + 2), cudaMemcpyDeviceToHost, s));
-  }
+  CUDA_TRY(cudaMemcpyAsync(tok, ws.b_tok[fin], 8 * ws.nseq * G, cudaMemcpyDeviceToDevice, s));
+  CUDA_TRY(cudaMemcpyAsync(pad, ws.b_pad[fin], ws.nseq * G, cudaMemcpyDeviceToDevice, s));
+  CUDA_TRY(cudaMemcpyAsync(score, length_alpha != 0.f ? ws.b_norm : ws.b_score[fin], 4 * ws.nseq, cudaMemcpyDeviceToDevice, s));
+  CUDA_TRY(cudaMemcpyAsync(h->h_flags, ws.flags, sizeof(int) * (G + 2), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
-  int T = 0;
-  for (int i = 0; i < cp.n; ++i) {
-    int Ti = G;
-    for (int c = 1; c < G; ++c) if (h->h_flags[i * (G + 2) + c] != 0) { Ti = c; break; }
-    T = std::max(T, Ti);
-  }
+  int T = G;
+  for (int c = 1; c < G; ++c) if (h->h_flags[c] != 0) { T = c; break; }
   if (T_out) *T_out = T;
   return 0;
 }
@@ -1962,9 +1639,8 @@ int64_t novic_debug_zones(const NovicHandle* h, int32_t kind, int64_t num_embeds
   std::vector<std::pair<size_t, size_t>> zones;
   g_zone_log = &zones;
   if (kind == 0) {
-    ChainPlan cp;
-    plan_chains(h, num_embeds, seqs_per_embed, rows_or_cols, nullptr, &cp);
-    if (cp.n != 1) { g_zone_log = nullptr; fail("guard-band listing supports one chain"); return -1; }
+    Workspace ws;
+    plan_workspace(h, num_embeds, seqs_per_embed, rows_or_cols, nullptr, &ws);
   } else if (kind == 1) {
     TrainPlan t;
     plan_train(h, num_embeds, seqs_per_embed, rows_or_cols, nullptr, &t);
@@ -1998,7 +1674,7 @@ int novic_debug_gemm(const void* a_bf16, const void* w_bf16, float* out, int32_t
     q.n_valid = N; q.nparts = np; q.inv_tau = 1.0f; q.ban_eos = 0; q.want_sumx = 0;
     q.allow = nullptr; q.allow_ld = 0; q.allow_mod = 0; q.mask_lse = 0;
     int rc2;
-    if (block_n == 256) rc2 = set_gemm_attr<EpiLogits<0>, 2, kWideKbs, 256>() || set_gemm_attr<EpiLogits<0>, 2, kWideKbs, 256, 16>() || launch_gemm<EpiLogits<0>, 2, kWideKbs, 256>(s, ta3, tb3, M, N, K, q);
+    if (block_n == 256) rc2 = set_gemm_attr<EpiLogits<0>, 2, kWideKbs, 256, 16>() || launch_gemm<EpiLogits<0>, 2, kWideKbs, 256, 16>(s, ta3, tb3, M, N, K, q);
     else rc2 = set_gemm2_attr<EpiLogits<0>, 3>() || launch_gemm2<EpiLogits<0>, 3>(s, ta3, tb3, M, N, K, q);
     CUDA_TRY(cudaFreeAsync(pt, s));
     return rc2;

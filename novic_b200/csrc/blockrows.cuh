@@ -30,9 +30,7 @@ constexpr int kBrEpiWarps = 16;
 constexpr int kBrThreads = 64 + 32 * kBrEpiWarps;   // 576
 constexpr int kBrRequests = 12;                     // 8 x Wo, 2 x W1, 2 x W2
 constexpr int kBrStatsBytes = kBrRows * 4 * 8;      // [row][quadrant] (sum, sum of squares)
-constexpr int kBrBarBytes = 512;                    // pipeline barriers (first 256 B) + the attention phase's [16 warps][2 slots] (second 256 B)
-constexpr int kBrAttnSlots = 2;                     // attention phase: 4 KB K / V chunks in flight per warp (16 warps x 2 x 4 KB = ring slots 0 and 1)
-constexpr int kBrAttnChunk = 4;                     // keys per chunk
+constexpr int kBrBarBytes = 512;                    // pipeline barriers (the first 256 B are used)
 __host__ __device__ constexpr int block_rows_smem_bytes() {
   return 1024 /*align*/ + kBrSlots * kBrSlotBytes + kBrActBytes + kBrBarBytes /*barriers*/ + kBrStatsBytes;
 }
@@ -115,167 +113,10 @@ __device__ __forceinline__ float br_warp_reduce16(float (&val)[16], int lane) {
 }
 
 
-// ---------------------------------------------------------------------------------------------------------
-// Attention phase of the fused kernel: attention_stream_kernel_t<16, 2, 4> (kernels.cuh) for the CTA's own 32 sequences, executed by the 16
-// epilogue warps before they become the epilogue: warp ew streams the K / V rows of sequences m0 + ew and m0 + ew + 16 through two 4 KB
-// slots of its own (ring slots 0 and 1 of the weight ring, idle until the out-proj weights are needed), four keys per chunk scored as
-// independent chains, online softmax in fp32.  The attention row never leaves the SM: it is written as bf16 straight into the K-major
-// 128B-swizzled resident operand of the out-proj MMAs (lane = 16 channels = two 16-byte chunks of k-block lane / 4).
-// ---------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void br_attention_phase(const AttnParams& p, int m0, int ew, int lane, uint8_t* ring, uint64_t* attn_bar, uint8_t* act) {
-  constexpr int kSlots = kBrAttnSlots, kChunk = kBrAttnChunk, kSlotBytes = kBrAttnChunk * 1024;
-  uint8_t* slots = ring + static_cast<size_t>(ew) * (kSlots * kSlotBytes);
-  uint64_t* full_bar = attn_bar + ew * kSlots;
-  const int qpos = p.q0;
-  const int nkeys = (p.prefix_bidir && qpos < p.P) ? p.P : qpos + 1;
-  const int nchunks = (nkeys + kChunk - 1) / kChunk;
-  const int per_item = 2 * nchunks;                                  // K chunk, V chunk, K chunk, ...
-  const int nitems = (m0 + ew < p.nseq ? 1 : 0) + (m0 + ew + kBrEpiWarps < p.nseq ? 1 : 0);
-  const int nloads = nitems * per_item;
-  const bool contiguous = p.beams == 1;
-  if (lane == 0) {
-#pragma unroll
-    for (int s = 0; s < kSlots; ++s) mbar_init(&full_bar[s], 1);
-    fence_mbar_init();
-  }
-  __syncwarp();
-  auto issue = [&](int n) {
-    const int i = n / per_item, r = n - i * per_item;
-    const int c = r >> 1, kv = r & 1;
-    const int a = m0 + ew + i * kBrEpiWarps;
-    const int j0 = c * nkeys / nchunks, rows = (c + 1) * nkeys / nchunks - j0;
-    const __nv_bfloat16* base = kv ? p.vcache : p.kcache;
-    const int sl = n % kSlots;
-    uint8_t* dst = slots + sl * kSlotBytes;
-    const int own_slot = a * p.slot_mul;
-    if (lane == 0) mbar_arrive_expect_tx(&full_bar[sl], static_cast<uint32_t>(rows) * 1024u);
-    if (contiguous) {
-      if (lane == 0) {
-        const void* src = base + (static_cast<size_t>(own_slot) * p.smax + j0) * kE;
-        if (p.stream_hint) bulk_load_1d_hint(dst, src, static_cast<uint32_t>(rows) * 1024u, &full_bar[sl], kEvictFirst);
-        else bulk_load_1d(dst, src, static_cast<uint32_t>(rows) * 1024u, &full_bar[sl]);
-      }
-    } else {
-      __syncwarp();
-      if (lane < rows) {
-        const int j = j0 + lane;
-        const int group0 = (own_slot / p.beams) * p.beams;
-        int slot;
-        if (j < p.P) slot = group0;
-        else if (p.anc != nullptr && j < qpos) slot = group0 + p.anc[static_cast<size_t>(a) * p.anc_ld + (j - p.P)];
-        else slot = own_slot;
-        bulk_load_1d(dst + lane * 1024, base + (static_cast<size_t>(slot) * p.smax + j) * kE, 1024u, &full_bar[sl]);
-      }
-    }
-  };
-  // chunks other than an item's last hold only rows written by earlier decode steps: safe to request before the wait (see
-  // attention_stream_kernel_t: select_greedy_kernel releases its dependents only after its own wait)
-  int issued = 0;
-  if (p.early_loads == 1 && contiguous && nchunks >= 2) {
-    const int early = min(min(nloads, kSlots), 2);
-    for (; issued < early; ++issued) issue(issued);
-  }
-  pdl_wait();
-  for (; issued < min(nloads, kSlots); ++issued) issue(issued);
-
-  float qf[16], acc[16], pj[kChunk];
-  float m = -INFINITY, l = 0.f, corr = 0.f;
-  uint4 qa = make_uint4(0, 0, 0, 0), qb = qa;
-  if (nitems > 0) {
-    const uint4* q4 = reinterpret_cast<const uint4*>(p.q + static_cast<size_t>(m0 + ew) * kE) + lane * 2;
-    qa = __ldg(q4); qb = __ldg(q4 + 1);
-  }
-  int i = 0, r = 0;
-  for (int n = 0; n < nloads; ++n) {
-    const int c = r >> 1;
-    const int j0 = c * nkeys / nchunks, rows = (c + 1) * nkeys / nchunks - j0;
-    if (r == 0) {
-      bf16x8_to_f32(qa, qf);
-      bf16x8_to_f32(qb, qf + 8);
-#pragma unroll
-      for (int k = 0; k < 16; ++k) { qf[k] *= p.scale_log2e; acc[k] = 0.f; }
-      m = -INFINITY; l = 0.f;
-      if (i + 1 < nitems) {   // next item's query: in flight while this item streams
-        const uint4* q4 = reinterpret_cast<const uint4*>(p.q + static_cast<size_t>(m0 + ew + kBrEpiWarps) * kE) + lane * 2;
-        qa = __ldg(q4); qb = __ldg(q4 + 1);
-      }
-    }
-    const int sl = n % kSlots;
-    const uint8_t* src = slots + sl * kSlotBytes + lane * 32;
-    mbar_wait(&full_bar[sl], static_cast<uint32_t>(n / kSlots) & 1u, 5);
-    if ((r & 1) == 0) {
-      float s[kChunk];
-#pragma unroll
-      for (int u = 0; u < kChunk; ++u) {
-        s[u] = -INFINITY;
-        if (u < rows) {
-          const uint4* k4 = reinterpret_cast<const uint4*>(src + u * 1024);
-          float kf[16];
-          bf16x8_to_f32(k4[0], kf);
-          bf16x8_to_f32(k4[1], kf + 8);
-          float d0 = 0.f, d1 = 0.f;
-#pragma unroll
-          for (int k = 0; k < 8; ++k) { d0 = fmaf(qf[k], kf[k], d0); d1 = fmaf(qf[8 + k], kf[8 + k], d1); }
-          s[u] = d0 + d1;
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < kChunk; ++u) {
-        if (u < rows) {
-          s[u] += __shfl_xor_sync(0xffffffffu, s[u], 1);
-          s[u] += __shfl_xor_sync(0xffffffffu, s[u], 2);
-        }
-      }
-      float m_new = m;
-#pragma unroll
-      for (int u = 0; u < kChunk; ++u) m_new = fmaxf(m_new, s[u]);
-      corr = exp2f(m - m_new);
-      float psum = 0.f;
-#pragma unroll
-      for (int u = 0; u < kChunk; ++u) { pj[u] = exp2f(s[u] - m_new); psum += pj[u]; }
-      l = l * corr + psum;
-      m = m_new;
-    } else {
-#pragma unroll
-      for (int k = 0; k < 16; ++k) acc[k] *= corr;
-#pragma unroll
-      for (int u = 0; u < kChunk; ++u) {
-        if (u < rows) {
-          const uint4* v4 = reinterpret_cast<const uint4*>(src + u * 1024);
-          float vf[16];
-          bf16x8_to_f32(v4[0], vf);
-          bf16x8_to_f32(v4[1], vf + 8);
-#pragma unroll
-          for (int k = 0; k < 16; ++k) acc[k] = fmaf(pj[u], vf[k], acc[k]);
-        }
-      }
-    }
-    __syncwarp();                       // every lane has consumed the slot: refill it
-    if (issued < nloads) { issue(issued); ++issued; }
-    if (++r == per_item) {
-      const float inv = 1.0f / l;
-      uint32_t o[8];
-#pragma unroll
-      for (int k = 0; k < 8; ++k) o[k] = pack_bf16x2(acc[2 * k] * inv, acc[2 * k + 1] * inv);
-      const int row = ew + i * kBrEpiWarps;                       // local row of the sequence
-      uint8_t* d = act + (lane >> 2) * kBrKbBytes + row * 128;
-      const int c0 = (lane & 3) * 2;
-      *reinterpret_cast<uint4*>(d + (((c0) ^ (row & 7)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
-      *reinterpret_cast<uint4*>(d + (((c0 + 1) ^ (row & 7)) << 4)) = make_uint4(o[4], o[5], o[6], o[7]);
-      r = 0;
-      ++i;
-    }
-  }
-}
-
-template <bool ATTN>
 __global__ void __launch_bounds__(kBrThreads, 1)
 block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_constant__ CUtensorMap tmap_wo, const __grid_constant__ CUtensorMap tmap_w1,
                   const __grid_constant__ CUtensorMap tmap_w2, const __grid_constant__ CUtensorMap tmap_x, int M,
-                  FusedBlockParams ep, AttnParams pa) {
-  // ATTN: the decode-step attention of the CTA's 32 sequences runs first, on the epilogue warps (br_attention_phase): pa is valid, tmap_ao is
-  // not used.  The weight ring is rotated by two slots so that request 0 (prefetched at launch) lands in slot 2 while slots 0 and 1 stage K / V.
-  constexpr int kSlotOff = ATTN ? 2 : 0;
+                  FusedBlockParams ep) {
   constexpr uint32_t kIdesc = umma_idesc_bf16_f32(128, kBrRows);
   constexpr uint32_t kColHidden = 128, kColFfn2 = 160;
   extern __shared__ uint8_t smem_raw[];
@@ -292,8 +133,6 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
   uint64_t* acc2_full = h_ready + 1;                                    // [4]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc2_full + 4);
   static_assert((2 * kBrSlots + 1 + 4 + 3 + 4) * 8 + 4 <= 256, "barrier area");
-  uint64_t* attn_bar = full_bar + 32;                                   // [16 warps][2 slots], second half of the barrier area
-  static_assert(256 + kBrEpiWarps * kBrAttnSlots * 8 <= kBrBarBytes && kBrEpiWarps * kBrAttnSlots * kBrAttnChunk * 1024 <= 2 * kBrSlotBytes, "attention staging");
   float2* s_stats = reinterpret_cast<float2*>(act + kBrActBytes + kBrBarBytes);  // [32 rows][4 quadrants]
 
   const int warp = threadIdx.x >> 5;
@@ -305,7 +144,7 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
 
   // request i of the weight stream: 0..7 = Wo tile i / 2, k-blocks 4 (i & 1) .. + 3;  8, 9 = W1 k-blocks 0..3 / 4..7;  10, 11 = W2 tiles 0, 1 / 2, 3
   auto issue = [&](int i) {
-    const int slot = (i + kSlotOff) % kBrSlots;
+    const int slot = i % kBrSlots;
     mbar_arrive_expect_tx(&full_bar[slot], kBrSlotBytes);
     uint8_t* dst = ring + slot * kBrSlotBytes;
     if (i < 8) tma_load_4d(dst, &tmap_wo, &full_bar[slot], 0, 0, i >> 1, (i & 1) * 4, kEvictLast);
@@ -315,22 +154,18 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
 
   if (warp == 0) {
     if (elect_one()) {
-      if (!ATTN) tma_prefetch_desc(&tmap_ao);
+      tma_prefetch_desc(&tmap_ao);
       tma_prefetch_desc(&tmap_wo); tma_prefetch_desc(&tmap_w1); tma_prefetch_desc(&tmap_w2);
       tma_prefetch_desc(&tmap_x);
       for (int st = 0; st < kBrSlots; ++st) { mbar_init(&full_bar[st], 1); mbar_init(&empty_bar[st], 1); }
-      mbar_init(act_full, ATTN ? kBrEpiWarps : 1);
+      mbar_init(act_full, 1);
       for (int t = 0; t < 4; ++t) { mbar_init(&acc0_full[t], 1); mbar_init(&acc2_full[t], 1); }
       mbar_init(ln2_ready, kBrEpiWarps); mbar_init(acc1_full, 1); mbar_init(h_ready, kBrEpiWarps);
       fence_mbar_init();
-      if (ATTN) {
-        issue(0);                                           // slot 2; slots 0 and 1 belong to the attention phase
-      } else {
-        for (int i = 0; i < kBrSlots; ++i) issue(i);        // the weights do not depend on the previous kernel
-        pdl_wait();
-        mbar_arrive_expect_tx(act_full, kBrActBytes);
-        tma_load_3d(act, &tmap_ao, act_full, m0, 0, kEvictFirst);
-      }
+      for (int i = 0; i < kBrSlots; ++i) issue(i);          // the weights do not depend on the previous kernel
+      pdl_wait();
+      mbar_arrive_expect_tx(act_full, kBrActBytes);
+      tma_load_3d(act, &tmap_ao, act_full, m0, 0, kEvictFirst);
     }
   } else if (warp == 1) {
     tmem_alloc<512>(tmem_slot);
@@ -345,12 +180,8 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
 
   if (warp == 0) {
     if (elect_one()) {
-      if (ATTN) {
-        mbar_wait(act_full, 0, 1);                          // all 16 warps have finished their sequences: the K / V staging slots are free
-        issue(1); issue(2);
-      }
       for (int i = kBrSlots; i < kBrRequests; ++i) {
-        mbar_wait(&empty_bar[(i + kSlotOff) % kBrSlots], ((i / kBrSlots) - 1) & 1, 1);
+        mbar_wait(&empty_bar[i % kBrSlots], ((i / kBrSlots) - 1) & 1, 1);
         issue(i);
       }
     }
@@ -364,7 +195,7 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
       tp(22);
       // ---- out-proj: tile t (features 4 i + t) = requests 2 t, 2 t + 1
       for (int i = 0; i < 8; ++i) {
-        const int slot = (i + kSlotOff) % kBrSlots;
+        const int slot = i % kBrSlots;
         mbar_wait(&full_bar[slot], (i / kBrSlots) & 1, 3);
         tp(10 + i);
         tc_fence_after_sync();
@@ -387,7 +218,7 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
       tp(23);
       tc_fence_after_sync();
       for (int i = 8; i < 10; ++i) {
-        const int slot = (i + kSlotOff) % kBrSlots;
+        const int slot = i % kBrSlots;
         mbar_wait(&full_bar[slot], (i / kBrSlots) & 1, 5);
         tp(10 + i);
         tc_fence_after_sync();
@@ -410,7 +241,7 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
       tp(24);
       tc_fence_after_sync();
       for (int i = 10; i < 12; ++i) {
-        const int slot = (i + kSlotOff) % kBrSlots;
+        const int slot = i % kBrSlots;
         mbar_wait(&full_bar[slot], (i / kBrSlots) & 1, 7);
         tp(10 + i);
         tc_fence_after_sync();
@@ -438,14 +269,7 @@ block_rows_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_cons
     const float4 g_mid = __ldg(reinterpret_cast<const float4*>(ep.gain_mid) + fi);
     const float4 g_out = __ldg(reinterpret_cast<const float4*>(ep.gain_out) + fi);
     float r[8][4];
-    if (ATTN) {
-      br_attention_phase(pa, m0, ew, lane, ring, attn_bar, act);      // includes griddepcontrol.wait
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(act_full);
-    } else {
-      pdl_wait();
-    }
+    pdl_wait();
     tp(1);
 #pragma unroll
     for (int p = 0; p < 4; ++p) {

@@ -182,31 +182,6 @@ __device__ __forceinline__ float gelu_fast(float x) {
   return 0.5f * x * (1.0f + copysignf(erf_abs, x));
 }
 
-// FFN first linear + GELU -> bf16 h[M, 128] (only used when the fused feed-forward kernel is disabled)
-struct EpiGelu {
-  struct Params {
-    __nv_bfloat16* h;
-    int ldh;
-  };
-  template <class Release>
-  __device__ static __forceinline__ void run(const Params& p, const EpiCtx& c, Release release) {
-    const int lane = lane_id();
-#pragma unroll
-    for (int ch = 0; ch < kEpiCols / 32; ++ch) {
-      float v[32];
-      tmem_ld_32x32(c.tmem_row + ch * 32, v);
-      if (ch == kEpiCols / 32 - 1) release();
-#pragma unroll
-      for (int j = 0; j < 32; ++j) v[j] = gelu_fast(v[j]);
-      stage_put32(c.stage, lane, ch * 32, v);
-    }
-    stage_copy_out(c.stage, lane, [&](int r) -> __nv_bfloat16* {
-      const int row = c.warp_row0 + r;
-      return row < c.M ? p.h + static_cast<size_t>(row) * p.ldh + c.n0 : nullptr;
-    });
-  }
-};
-
 // Per (row, 64-column vocabulary slice) statistics written by the logits epilogue and merged by the selection kernels.
 struct __align__(32) LogitPartial {
   float max_all;     // max over the slice's valid columns (natural units)
@@ -702,42 +677,30 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
 // SMs pull, against 2.1 k cycles of MMA - and half of those bytes are the same 128 KB weight tile every time.  Here CTA b owns ONE column
 // tile (b % n_tiles) for the whole launch: its weight tile (8 k-blocks, 128 KB) is loaded once - before griddepcontrol.wait, i.e. under the
 // previous kernel's tail, since weights do not depend on it - and stays in shared memory; the CTA then walks the row blocks
-// b / n_tiles, + gridDim.x / n_tiles, ... streaming only the activation tiles through two or three 32 KB stages.  Grid = n_tiles x floor(#SMs / n_tiles).
+// b / n_tiles, + gridDim.x / n_tiles, ... streaming only the activation tiles through three 32 KB stages.  Grid = n_tiles x floor(#SMs / n_tiles).
 // Same accumulation order as gemm_kernel: results are bit-identical.
 // ---------------------------------------------------------------------------------------------------------
 constexpr int kWsKb = 8;                                   // k-blocks of the stationary weight tile (K = 512)
 constexpr int kWsABytes = 2 * kABytes;                     // activation stage: two k-blocks (32 KB)
-// WS_STAGES = 2: with the epilogue's 32 KB staging tile.  WS_STAGES = 3 (default): a third activation stage instead; q / K / V then leave
-// straight from the registers as 256-bit stores (st.global.v8.b32: a thread's 64 columns are four full 32-byte sectors of its row).  With
-// 16-byte stores - half-sector writes - the third stage cost more than it gained (5.5 k instead of 4.5 k cycles per tile); with full
-// sectors the QKV class drops from 1.10 to 0.99 ms per decode (bit-identical: same accumulation order, same rounding).
-__host__ __device__ constexpr int gemm_ws_smem_bytes(int stages) { return kWsKb * kBBytes + stages * kWsABytes + (stages == 2 ? kEpiWarps * kEpiStageBytes : 0) + 1024 + 256; }
+constexpr int kWsStages = 3;                               // activation stages
+// Three activation stages and no epilogue staging tile: q / K / V leave straight from the registers as 256-bit stores (st.global.v8.b32: a
+// thread's 64 columns are four full 32-byte sectors of its row).  With 16-byte stores - half-sector writes - the third stage cost more than
+// it gained (5.5 k instead of 4.5 k cycles per tile); with full sectors the QKV class dropped from 1.10 to 0.99 ms per decode against two
+// stages plus the staging tile.
+__host__ __device__ constexpr int gemm_ws_smem_bytes() { return kWsKb * kBBytes + kWsStages * kWsABytes + 1024 + 256; }
 
-// MC (gemm_wsmc_kernel): the four CTAs of a cluster own four neighbouring column tiles and walk the SAME row blocks, so every activation
-// stage is requested once per cluster and multicast - stage-load n by the CTA of rank n % 4, which first waits until all four CTAs'
-// MMAs have released the stage (their commits arrive on every peer's `a_empty`, count 4).  A quarter of the L2 -> SM activation
-// traffic and of the TMA requests per SM (the limiter of the non-multicast kernel: two 32 KB requests in flight per SM, ~1.7 k cycles
-// each when 144 SMs pull at once).  Same operands, same accumulation order: bit-identical.
-// MC runs WS_STAGES * 2 stages of ONE k-block (16 KB, 2-D map tmap_a2): the same 64 KB of ring, but four requests in flight per cluster,
-// one per SM's TMA unit (with two 32 KB stages the cross-CTA release -> request -> multicast round trip was the cadence: measured
-// 6.2 instead of 5.3 ms per decode).
-template <class Epi, int WS_STAGES, int CL>     // CL = cluster size: 1 (no multicast), 2 or 4
-__device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CUtensorMap& tmap_a2, const CUtensorMap& tmap_b, int M, int n_tiles, int b_is_static,
-                                             const typename Epi::Params& ep) {
-  constexpr bool MC = CL > 1;
-  constexpr int kWsCluster = CL;
-  constexpr int KBS = MC ? 1 : 2;                           // k-blocks per activation stage
-  constexpr int NST = WS_STAGES * 2 / KBS;                  // activation stages
-  constexpr int kStBytes = KBS * kABytes;
+template <class Epi>
+__global__ void __launch_bounds__(kGemmThreads, 1)
+gemm_ws_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, int M, int n_tiles, int b_is_static,
+               typename Epi::Params ep) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* b_smem = smem;                                   // [8 k-blocks][128 rows x 128 B]
   uint8_t* a_ring = b_smem + kWsKb * kBBytes;
-  uint8_t* epi_stage = a_ring + WS_STAGES * kWsABytes;
-  uint64_t* b_full = reinterpret_cast<uint64_t*>(epi_stage + (WS_STAGES == 2 ? kEpiWarps * kEpiStageBytes : 0));   // [4] one per pair of k-blocks
+  uint64_t* b_full = reinterpret_cast<uint64_t*>(a_ring + kWsStages * kWsABytes);   // [4] one per pair of k-blocks
   uint64_t* a_full = b_full + kWsKb / 2;
-  uint64_t* a_empty = a_full + NST;
-  uint64_t* tmem_full_bar = a_empty + NST;
+  uint64_t* a_empty = a_full + kWsStages;
+  uint64_t* tmem_full_bar = a_empty + kWsStages;
   uint64_t* tmem_empty_bar = tmem_full_bar + kAccStages;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty_bar + kAccStages);
   __shared__ int s_trace;
@@ -754,7 +717,7 @@ __device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CU
       tma_prefetch_desc(&tmap_a);
       tma_prefetch_desc(&tmap_b);
       for (int j = 0; j < kWsKb / 2; ++j) mbar_init(&b_full[j], 1);
-      for (int s = 0; s < NST; ++s) { mbar_init(&a_full[s], 1); mbar_init(&a_empty[s], MC ? kWsCluster : 1); }
+      for (int s = 0; s < kWsStages; ++s) { mbar_init(&a_full[s], 1); mbar_init(&a_empty[s], 1); }
       for (int a = 0; a < kAccStages; ++a) { mbar_init(&tmem_full_bar[a], 1); mbar_init(&tmem_empty_bar[a], kEpiWarps); }
       fence_mbar_init();
       if (b_is_static && g0 < m_blocks) {
@@ -769,12 +732,9 @@ __device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CU
   }
   tc_fence_before_sync();
   __syncthreads();
-  if (MC) cluster_sync_all();     // every CTA's barriers exist before a peer's multicast load or commit can reach them
   tc_fence_after_sync();
   const uint32_t tmem_base = *tmem_slot;
   const bool tr = s_trace != 0;
-  const uint32_t crank = MC ? cluster_ctarank() : 0u;
-  constexpr uint16_t kMcMask = (1u << kWsCluster) - 1u;
   pdl_wait();
   if (threadIdx.x == 0) trace_point(tr, 1);
 
@@ -787,14 +747,12 @@ __device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CU
         }
       }
       int stage = 0; uint32_t phase = 0;
-      uint32_t nload = 0;
       for (int mb = g0; mb < m_blocks; mb += gstep) {
-        for (int j = 0; j < kWsKb / KBS; ++j, ++nload) {
+        for (int j = 0; j < kWsKb / 2; ++j) {
           mbar_wait(&a_empty[stage], phase ^ 1, 1);
-          mbar_arrive_expect_tx(&a_full[stage], kStBytes);
-          if (!MC) tma_load_3d(a_ring + stage * kStBytes, &tmap_a, &a_full[stage], mb * kBlockM, 2 * j, kEvictNormal);
-          else if ((nload % kWsCluster) == crank) tma_load_2d_mc(a_ring + stage * kStBytes, &tmap_a2, &a_full[stage], j * kBlockK, mb * kBlockM, kMcMask, kEvictNormal);
-          if (++stage == NST) { stage = 0; phase ^= 1; }
+          mbar_arrive_expect_tx(&a_full[stage], kWsABytes);
+          tma_load_3d(a_ring + stage * kWsABytes, &tmap_a, &a_full[stage], mb * kBlockM, 2 * j, kEvictNormal);
+          if (++stage == kWsStages) { stage = 0; phase ^= 1; }
         }
       }
       trace_point(tr, 3);
@@ -809,21 +767,21 @@ __device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CU
         mbar_wait(&tmem_empty_bar[as], ((i >> 1) & 1) ^ 1, 9);
         tc_fence_after_sync();
         const uint32_t acc = tmem_base + as * kTileN;
-        for (int j = 0; j < kWsKb / KBS; ++j) {
-          if (i == 0 && (j * KBS) % 2 == 0) mbar_wait(&b_full[j * KBS / 2], 0, 4);
+        for (int j = 0; j < kWsKb / 2; ++j) {
+          if (i == 0) mbar_wait(&b_full[j], 0, 4);
           mbar_wait(&a_full[stage], phase, 2);
           if (i == 0 && j == 0) trace_point(tr, 4);
           tc_fence_after_sync();
-          const uint32_t sa = smem_u32(a_ring + stage * kStBytes);
-          const uint32_t sb = smem_u32(b_smem + j * KBS * kBBytes);
+          const uint32_t sa = smem_u32(a_ring + stage * kWsABytes);
+          const uint32_t sb = smem_u32(b_smem + j * 2 * kBBytes);
 #pragma unroll
-          for (int jj = 0; jj < KBS; ++jj)
+          for (int jj = 0; jj < 2; ++jj)
 #pragma unroll
             for (int k = 0; k < kBlockK / kUmmaK; ++k)
               umma_bf16_ss(acc, umma_desc_sw128_kmajor(sa + jj * kABytes + k * (kUmmaK * 2)),
                            umma_desc_sw128_kmajor(sb + jj * kBBytes + k * (kUmmaK * 2)), kIdesc, (j | jj | k) != 0 ? 1u : 0u);
-          if (MC) umma_commit_mc(&a_empty[stage], kMcMask); else umma_commit(&a_empty[stage]);
-          if (++stage == NST) { stage = 0; phase ^= 1; }
+          umma_commit(&a_empty[stage]);
+          if (++stage == kWsStages) { stage = 0; phase ^= 1; }
         }
         umma_commit(&tmem_full_bar[as]);
         if (i == 0) trace_point(tr, 5);
@@ -848,7 +806,7 @@ __device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CU
       c.ncols = kTileN / 2;
       c.M = M;
       c.part = nt * 2 + half;
-      c.stage = WS_STAGES == 2 ? epi_stage + ew * kEpiStageBytes : nullptr;
+      c.stage = nullptr;
       uint64_t* rel = &tmem_empty_bar[as];
       Epi::run(ep, c, [rel, lane]() {
         tc_fence_before_sync();
@@ -861,28 +819,8 @@ __device__ __forceinline__ void gemm_ws_body(const CUtensorMap& tmap_a, const CU
 
   tc_fence_before_sync();
   __syncthreads();
-  if (MC) cluster_sync_relaxed();   // a peer's last commits still arrive on this CTA's barriers: shared memory must outlive them
   if (threadIdx.x == 0) trace_point(tr, 10);
   if (warp == 1) tmem_dealloc<kAccStages * kTileN>(tmem_base);
-}
-
-template <class Epi, int WS_STAGES>
-__global__ void __launch_bounds__(kGemmThreads, 1)
-gemm_ws_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, int M, int n_tiles, int b_is_static,
-               typename Epi::Params ep) {
-  gemm_ws_body<Epi, WS_STAGES, 1>(tmap_a, tmap_a, tmap_b, M, n_tiles, b_is_static, ep);
-}
-template <class Epi, int WS_STAGES>
-__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(kGemmThreads, 1)
-gemm_wsmc_kernel(const __grid_constant__ CUtensorMap tmap_a2, const __grid_constant__ CUtensorMap tmap_b, int M, int n_tiles, int b_is_static,
-                 typename Epi::Params ep) {
-  gemm_ws_body<Epi, WS_STAGES, 4>(tmap_a2, tmap_a2, tmap_b, M, n_tiles, b_is_static, ep);
-}
-template <class Epi, int WS_STAGES>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGemmThreads, 1)
-gemm_wsmc2_kernel(const __grid_constant__ CUtensorMap tmap_a2, const __grid_constant__ CUtensorMap tmap_b, int M, int n_tiles, int b_is_static,
-                  typename Epi::Params ep) {
-  gemm_ws_body<Epi, WS_STAGES, 2>(tmap_a2, tmap_a2, tmap_b, M, n_tiles, b_is_static, ep);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1258,13 +1196,11 @@ struct FusedBlockParams {
   const float* gain_out;    // weight of the LayerNorm that follows the block
   int remap_rows_in, remap_skip, remap_rows_out;   // xn row remap of the last layer (0 = identity)
   float eps;
-  int qkv_tail;             // != 0: the NEXT layer's QKV projection runs in the kernel's tail (tmap_wqkv / qkv are valid; xn is not written)
-  EpiQKV::Params qkv;       // q buffer and the next layer's K / V cache pages
 };
 
 __global__ void __cluster_dims__(kRowCluster, 1, 1) __launch_bounds__(kRowThreads, 1)
 outproj_ffn_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_constant__ CUtensorMap tmap_wo, const __grid_constant__ CUtensorMap tmap_w1q,
-                   const __grid_constant__ CUtensorMap tmap_w2, const __grid_constant__ CUtensorMap tmap_wqkv, int M, FusedBlockParams ep) {
+                   const __grid_constant__ CUtensorMap tmap_w2, int M, FusedBlockParams ep) {
   constexpr int BN = kRowBN;
   constexpr int kHSplit = kFfnDim / kRowCluster;              // 32 hidden columns per CTA
   constexpr int kW1kb = kHSplit * kBlockK * 2;                // bytes of one k-block of the W1 slice: 4 KB
@@ -1288,13 +1224,8 @@ outproj_ffn_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_con
   uint64_t* affn_full = tmem_full0 + 5;                       // the three peers' LN2 slices have landed in this CTA's FFN1 operand
   uint64_t* hx_full = tmem_full0 + 6;                         // the three peers' hidden-column slices have landed in the h region
   uint64_t* hop_ready = tmem_full0 + 7;                       // the epilogue warps have assembled the FFN2 A operand
-  // QKV tail (the next layer's projection; ep.qkv_tail)
-  uint64_t* aq_full = tmem_full0 + 8;                         // the three peers' LayerNorm slices have landed in this CTA's QKV A operand
-  uint64_t* bq_full = tmem_full0 + 9;                         // [2] in_proj weight stages (two k-blocks of one 128-row tile each)
-  uint64_t* bq_empty = tmem_full0 + 11;                       // [2]
-  uint64_t* tmem_full_q = tmem_full0 + 13;                    // [3] one per 128-column output tile of this CTA
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full0 + 16);
-  static_assert((2 * kFbStages + 16) * 8 + 4 <= 256, "barrier area");
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full0 + 8);
+  static_assert((2 * kFbStages + 8) * 8 + 4 <= 256, "barrier area");
   constexpr int kHSlice = kBlockM * kHSplit * 2;              // one CTA's hidden columns: 128 rows x 64 B = 8 KB
   float* s_gain_mid = reinterpret_cast<float*>(after + 256);
   float* s_gain_out = s_gain_mid + BN;
@@ -1318,16 +1249,12 @@ outproj_ffn_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_con
   if (warp == 0) {
     if (elect_one()) {
       tma_prefetch_desc(&tmap_ao); tma_prefetch_desc(&tmap_wo); tma_prefetch_desc(&tmap_w1q); tma_prefetch_desc(&tmap_w2);
-      if (ep.qkv_tail) tma_prefetch_desc(&tmap_wqkv);
       for (int st = 0; st < kFbStages; ++st) { mbar_init(&full_bar[st], 1); mbar_init(&empty_bar[st], 1); }
       mbar_init(tmem_full0, 1); mbar_init(w1_full, 1); mbar_init(w2_full, 1); mbar_init(tmem_full1, 1); mbar_init(tmem_full2, 1);
       mbar_init(affn_full, 1); mbar_init(hx_full, 1); mbar_init(hop_ready, kRowEpiWarps);
-      mbar_init(aq_full, 1); mbar_init(&bq_full[0], 1); mbar_init(&bq_full[1], 1); mbar_init(&bq_empty[0], 1); mbar_init(&bq_empty[1], 1);
-      mbar_init(&tmem_full_q[0], 1); mbar_init(&tmem_full_q[1], 1); mbar_init(&tmem_full_q[2], 1);
       fence_mbar_init();
       mbar_arrive_expect_tx(affn_full, (kRowCluster - 1) * 2 * kABytes);   // the peers' copies can only start after cluster barrier #1
       mbar_arrive_expect_tx(hx_full, (kRowCluster - 1) * kHSlice);
-      if (ep.qkv_tail) mbar_arrive_expect_tx(aq_full, (kRowCluster - 1) * 2 * kABytes);   // ... and these after barrier #4
       // all weights first (they do not depend on the previous kernel), then wait, then the activation tiles
       for (int kb = 0; kb < kFbStages; ++kb) {
         mbar_arrive_expect_tx(&full_bar[kb], kStageBytes);
@@ -1558,480 +1485,6 @@ outproj_ffn_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_con
   __syncwarp();
   cluster_sync_all();       // #4
   if (threadIdx.x == 64) trace_point(tr, 12);
-  if (!ep.qkv_tail) {
-    if (is_epi) {
-      float mean = 0.f, rstd = 0.f;
-      s_stats = reinterpret_cast<float2*>(w2_smem);
-      if (row < M) gather_stats(mean, rstd);
-      uint8_t* stage = ring + ew * (32 * kRowStagePitch);      // the FFN1 operand is dead: every CTA's phase-B MMAs completed before #3
-      {
-        uint4* d = reinterpret_cast<uint4*>(stage + lane * kRowStagePitch);
-#pragma unroll
-        for (int q = 0; q < kRowCols / 8; ++q) {
-          float y[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) y[i] = (r[q * 8 + i] - mean) * rstd * s_gain_out[half * kRowCols + q * 8 + i];
-          d[q] = make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
-        }
-      }
-      if (row < M) {
-#pragma unroll
-        for (int q = 0; q < kRowCols / 4; ++q)
-          *reinterpret_cast<float4*>(ep.x + xblk_off(row, (c0 >> 2) + q)) = make_float4(r[q * 4], r[q * 4 + 1], r[q * 4 + 2], r[q * 4 + 3]);
-      }
-      __syncwarp();
-      const int warp_row0 = m0 + quad * 32;
-      const int sub = lane >> 3, chunk = lane & 7;
-#pragma unroll 4
-      for (int i = 0; i < 8; ++i) {
-        const int rr = i * 4 + sub;
-        const int grow = warp_row0 + rr;
-        if (grow < M) {
-          int nrow = grow;
-          bool keep = true;
-          if (ep.remap_rows_in > 0) {
-            const int seq = grow / ep.remap_rows_in;
-            const int k = grow - seq * ep.remap_rows_in;
-            keep = k >= ep.remap_skip;
-            nrow = seq * ep.remap_rows_out + (k - ep.remap_skip);
-          }
-          if (keep)
-            *reinterpret_cast<uint4*>(ep.xn + static_cast<size_t>(nrow) * kE + c0 + chunk * 8) =
-                *reinterpret_cast<const uint4*>(stage + rr * kRowStagePitch + chunk * 16);
-        }
-      }
-    }
-    if (threadIdx.x == 64) trace_point(tr, 13);
-  } else {
-    // ---- QKV tail: the next layer's LayerNorm rows become the A operand of its in_proj GEMM without leaving the cluster.
-    // Same hand-over as for LN2 above: every thread writes its 128-byte row of k-block (2 * rank + half) into the local operand buffer (the
-    // ring, dead since phase B), one thread pushes the CTA's two k-block tiles to the peers.  The CTA then computes output columns
-    // [384 * rank, +384) of q | k | v: three 128-column tiles, accumulators in TMEM columns 0 / 128 / 256 (all consumed by now), weight tiles
-    // streamed as 32 KB requests (two k-blocks) through two stages that live in the dead W1 and h regions; the dead W2 region is the
-    // epilogue's staging memory.  The products are accumulated in the same order as gemm_kernel<EpiQKV> does: results are bit-identical.
-    uint8_t* bstage[2] = {w1_smem, h_smem};
-    if (is_epi) {
-      float mean = 0.f, rstd = 0.f;
-      s_stats = reinterpret_cast<float2*>(w2_smem);
-      if (row < M) gather_stats(mean, rstd);
-      const int kb = static_cast<int>(crank) * 2 + half;
-      uint8_t* arow = ring + kb * kABytes + row_in_tile * 128;
-#pragma unroll
-      for (int q = 0; q < kRowCols / 8; ++q) {
-        float y[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) y[i] = (r[q * 8 + i] - mean) * rstd * s_gain_out[half * kRowCols + q * 8 + i];
-        *reinterpret_cast<uint4*>(arow + ((q ^ (row_in_tile & 7)) << 4)) =
-            make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
-      }
-      fence_proxy_async_smem();
-      if (row < M) {
-#pragma unroll
-        for (int q = 0; q < kRowCols / 4; ++q)
-          *reinterpret_cast<float4*>(ep.x + xblk_off(row, (c0 >> 2) + q)) = make_float4(r[q * 4], r[q * 4 + 1], r[q * 4 + 2], r[q * 4 + 3]);
-      }
-    }
-    __syncthreads();
-    if (threadIdx.x == 64) trace_point(tr, 13);
-    constexpr int kQTiles = 3 * kE / (kRowCluster * kTileN);    // 3 output tiles per CTA
-    constexpr int kQLoads = kQTiles * (kNkb / 2);               // 12 weight requests of two k-blocks
-    if (warp == 0) {
-      if (elect_one()) {
-        const uint8_t* src = ring + static_cast<int>(crank) * 2 * kABytes;
-#pragma unroll
-        for (uint32_t d = 1; d < kRowCluster; ++d) {
-          const uint32_t pr = (crank + d) % kRowCluster;
-          dsmem_bulk_copy(dsmem_addr(src, pr), src, 2 * kABytes, dsmem_addr(aq_full, pr));
-        }
-        for (int i = 0; i < kQLoads; ++i) {
-          const int st = i & 1;
-          mbar_wait(&bq_empty[st], ((i >> 1) & 1) ^ 1, 1);
-          mbar_arrive_expect_tx(&bq_full[st], 2 * kBBytes);
-          tma_load_3d(bstage[st], &tmap_wqkv, &bq_full[st], static_cast<int>(crank) * (kQTiles * kTileN) + (i / (kNkb / 2)) * kTileN, (i % (kNkb / 2)) * 2, kEvictLast);
-        }
-      }
-    } else if (warp == 1) {
-      if (elect_one()) {
-        mbar_wait(aq_full, 0, 5);
-        tc_fence_after_sync();
-        const uint32_t sa = smem_u32(ring);
-        for (int nt = 0; nt < kQTiles; ++nt) {
-          for (int kp = 0; kp < kNkb / 2; ++kp) {
-            const int i = nt * (kNkb / 2) + kp, st = i & 1;
-            mbar_wait(&bq_full[st], (i >> 1) & 1, 2);
-            tc_fence_after_sync();
-            const uint32_t sb = smem_u32(bstage[st]);
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-#pragma unroll
-              for (int k = 0; k < kBlockK / kUmmaK; ++k)
-                umma_bf16_ss(tmem_base + nt * kTileN, umma_desc_sw128_kmajor(sa + (kp * 2 + j) * kABytes + k * (kUmmaK * 2)),
-                             umma_desc_sw128_kmajor(sb + j * kBBytes + k * (kUmmaK * 2)), kIdesc, (kp | j | k) != 0 ? 1u : 0u);
-            umma_commit(&bq_empty[st]);
-          }
-          umma_commit(&tmem_full_q[nt]);
-        }
-      }
-    }
-    __syncwarp();
-    if (is_epi) {
-      for (int nt = 0; nt < kQTiles; ++nt) {
-        mbar_wait(&tmem_full_q[nt], 0, 9);
-        tc_fence_after_sync();
-        EpiCtx c;
-        c.tmem_row = tmem_lane + nt * kTileN + half * kEpiCols;
-        c.warp_row0 = m0 + quad * 32;
-        c.row = c.warp_row0 + lane;
-        c.n0 = static_cast<int>(crank) * (kQTiles * kTileN) + nt * kTileN + half * kEpiCols;
-        c.ncols = kEpiCols;
-        c.M = M;
-        c.part = 0;
-        c.stage = w2_smem + ew * kEpiStageBytes;
-        EpiQKV::run(ep.qkv, c, []() {});
-      }
-    }
-    if (threadIdx.x == 64) trace_point(tr, 15);
-  }
-  tc_fence_before_sync();
-  __syncwarp();
-  cluster_sync_relaxed();   // peers may still be reading this CTA's statistics / operand tiles
-  if (threadIdx.x == 0) trace_point(tr, 14);
-  if (warp == 1) tmem_dealloc<512>(tmem_base);
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// The block kernel with the first feed-forward GEMM split over K instead of over the hidden columns (default; NOVIC_FFN1_KSPLIT=0 restores
-// outproj_ffn_kernel).  The phase trace of outproj_ffn_kernel shows its largest single wait - 5.6 k of 29 k cycles - between the local LN2
-// rows and FFN1: every CTA needs the whole 512-wide LN2 row, i.e. 96 KB from its three peers at the ~17 B/clk a CTA receives over DSMEM.
-// Here a CTA multiplies only ITS OWN 128 LN2 columns (resident, nothing to wait for) with W1[:, own 128 columns]: a partial 128 x 128 hidden
-// tile in fp32.  The partial sums are then reduce-scattered - each CTA receives the three 128 x 32 fp32 blocks for the hidden columns it owns,
-// 48 KB instead of 96 KB - added in the order of the source rank, passed through GELU, and from there the kernel continues as before
-// (hidden-column exchange, FFN2, LayerNorm).  The hidden pre-activations are sums of four K = 128 partial products instead of one K = 512
-// accumulation: equal to fp32 rounding, not bit-identical to the other variants (tests compare with a tolerance of 1e-5 relative).
-// Shared memory after the out-proj phase: ring slot 0-1 = own LN2 tiles, 2-4 = outgoing blocks, 5-7 = incoming blocks (16 KB each).
-// ---------------------------------------------------------------------------------------------------------
-__global__ void __cluster_dims__(kRowCluster, 1, 1) __launch_bounds__(kRowThreads, 1)
-outproj_ffn_ks_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_constant__ CUtensorMap tmap_wo, const __grid_constant__ CUtensorMap tmap_w1,
-                      const __grid_constant__ CUtensorMap tmap_w2, int M, FusedBlockParams ep) {
-  constexpr int BN = kRowBN;
-  constexpr int kHSplit = kFfnDim / kRowCluster;              // 32 hidden columns per CTA
-  constexpr int kW1kb = kHSplit * kBlockK * 2;                // bytes of one k-block of the W1 slice: 4 KB
-  constexpr uint32_t kIdesc = umma_idesc_bf16_f32(kBlockM, BN);
-  constexpr int kNkb = kE / kBlockK;                          // 8
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* ring = smem;                                       // phase A pipeline; afterwards the 8 k-block tiles of LN2(x_mid)
-  uint8_t* w1_smem = ring + kFbRing * kStageBytes;
-  uint8_t* w2_smem = w1_smem + kNkb * kW1kb;
-  uint8_t* h_smem = w2_smem + 2 * kBBytes;
-  uint8_t* after = h_smem + 2 * kABytes;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(after);
-  uint64_t* empty_bar = full_bar + kFbStages;
-  uint64_t* tmem_full0 = empty_bar + kFbStages;
-  uint64_t* w1_full = tmem_full0 + 1;
-  uint64_t* w2_full = tmem_full0 + 2;
-  uint64_t* tmem_full1 = tmem_full0 + 3;
-  uint64_t* tmem_full2 = tmem_full0 + 4;
-  uint64_t* pq_full = tmem_full0 + 5;                         // the three peers' partial FFN1 sums for this CTA's hidden columns have landed
-  uint64_t* hx_full = tmem_full0 + 6;                         // the three peers' hidden-column slices have landed in the h region
-  uint64_t* hop_ready = tmem_full0 + 7;                       // the epilogue warps have assembled the FFN2 A operand
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full0 + 8);
-  static_assert((2 * kFbStages + 8) * 8 + 4 <= 256, "barrier area");
-  constexpr int kPartBytes = kBlockM * kHSplit * 4;           // one peer's block of partial sums: 128 rows x 32 floats = 16 KB
-  constexpr int kHSlice = kBlockM * kHSplit * 2;              // one CTA's hidden columns: 128 rows x 64 B = 8 KB
-  float* s_gain_mid = reinterpret_cast<float*>(after + 256);
-  float* s_gain_out = s_gain_mid + BN;
-  // LayerNorm partials [2 halves][128 rows]: the first exchange uses the start of the h region (no hidden slice exists yet), the second
-  // the start of the W2 region (FFN2 has read it; the h region may still be the source of this CTA's outgoing slice copies)
-  float2* s_stats = reinterpret_cast<float2*>(h_smem);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = static_cast<int>(lane_id());
-  const int m0 = blockIdx.y * kBlockM;
-  const uint32_t crank = cluster_ctarank();
-  const int coff = static_cast<int>(crank) * BN;
-  const int n0 = coff;
-  __shared__ int s_trace;
-  pdl_trigger();
-  if (threadIdx.x == 0) { s_trace = trace_begin() ? 1 : 0; trace_point(s_trace != 0, 0); }
-
-  GemmSmemView sv;
-  sv.stages = ring; sv.full_bar = full_bar; sv.empty_bar = empty_bar; sv.tmem_full_bar = tmem_full0; sv.tmem_slot = tmem_slot; sv.scratch = nullptr;
-
-  if (warp == 0) {
-    if (elect_one()) {
-      tma_prefetch_desc(&tmap_ao); tma_prefetch_desc(&tmap_wo); tma_prefetch_desc(&tmap_w1); tma_prefetch_desc(&tmap_w2);
-      for (int st = 0; st < kFbStages; ++st) { mbar_init(&full_bar[st], 1); mbar_init(&empty_bar[st], 1); }
-      mbar_init(tmem_full0, 1); mbar_init(w1_full, 1); mbar_init(w2_full, 1); mbar_init(tmem_full1, 1); mbar_init(tmem_full2, 1);
-      mbar_init(pq_full, 1); mbar_init(hx_full, 1); mbar_init(hop_ready, kRowEpiWarps);
-      fence_mbar_init();
-      mbar_arrive_expect_tx(pq_full, (kRowCluster - 1) * kPartBytes);     // the peers' copies can only start after cluster barrier #1
-      mbar_arrive_expect_tx(hx_full, (kRowCluster - 1) * kHSlice);
-      // all weights first (they do not depend on the previous kernel), then wait, then the activation tiles
-      for (int kb = 0; kb < kFbStages; ++kb) {
-        mbar_arrive_expect_tx(&full_bar[kb], kStageBytes);
-        tma_load_2d(ring + kb * kStageBytes + kABytes, &tmap_wo, &full_bar[kb], kb * kBlockK, n0, kEvictLast);
-      }
-      pdl_wait();
-      for (int kb = 0; kb < kFbStages; ++kb)
-        tma_load_2d(ring + kb * kStageBytes, &tmap_ao, &full_bar[kb], kb * kBlockK, m0, kEvictNormal);
-    }
-  } else if (warp == 1) {
-    tmem_alloc<512>(tmem_slot);
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-  const bool tr = s_trace != 0;
-  pdl_wait();
-  if (threadIdx.x == 0) trace_point(tr, 1);
-
-  if (warp == 0) {
-    if (elect_one()) {
-      producer_rest<kFbStages>(sv, &tmap_ao, &tmap_wo, kNkb, m0, n0);
-      // stages 4 and 5 are the W1 / W2 regions: load the feed-forward weights as soon as the out-proj MMAs have read them
-      mbar_wait(&empty_bar[kFbRing], 0, 1);
-      mbar_arrive_expect_tx(w1_full, 2 * kBBytes);
-      for (int j = 0; j < 2; ++j) tma_load_2d(w1_smem + j * kBBytes, &tmap_w1, w1_full, (static_cast<int>(crank) * 2 + j) * kBlockK, 0, kEvictLast);
-      mbar_wait(&empty_bar[kFbRing + 1], 0, 1);
-      mbar_arrive_expect_tx(w2_full, 2 * kBBytes);
-      tma_load_2d(w2_smem, &tmap_w2, w2_full, 0, n0, kEvictLast);
-      tma_load_2d(w2_smem + kBBytes, &tmap_w2, w2_full, kBlockK, n0, kEvictLast);
-    }
-  } else if (warp == 1) {
-    if (elect_one()) mma_mainloop<kFbStages>(sv, tmem_base, kNkb, false);      // acc0 -> TMEM columns [0, 128)
-  }
-
-  // ---- phase A epilogue: residual + accumulator, LN2 statistics
-  const bool is_epi = warp >= 2;
-  const int ew = warp - 2;
-  const int quad = warp & 3;
-  const int half = ew >> 2;
-  const int row_in_tile = quad * 32 + lane;
-  const int row = m0 + row_in_tile;
-  const int c0 = coff + half * kRowCols;
-  const uint32_t tmem_lane = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
-  float r[kRowCols];
-  auto add_acc_and_stats = [&](uint32_t acc_col) {
-    float sum = 0.f, sumsq = 0.f;
-#pragma unroll
-    for (int c = 0; c < kRowCols / 16; ++c) {
-      float v[16];
-      tmem_ld_32x16(tmem_lane + acc_col + half * kRowCols + c * 16, v);
-#pragma unroll
-      for (int j = 0; j < 16; ++j) {
-        const float t = r[c * 16 + j] + v[j];
-        r[c * 16 + j] = t;
-        sum += t;
-        sumsq = fmaf(t, t, sumsq);
-      }
-    }
-    s_stats[half * 128 + row_in_tile] = make_float2(sum, sumsq);
-  };
-  auto gather_stats = [&](float& mean, float& rstd) {
-    float2 part[kRowCluster * 2];
-#pragma unroll
-    for (uint32_t pr = 0; pr < kRowCluster; ++pr) {
-#pragma unroll
-      for (int hh = 0; hh < 2; ++hh) part[pr * 2 + hh] = dsmem_ld_f32x2_addr(dsmem_addr(&s_stats[hh * 128 + row_in_tile], pr));
-    }
-    float sum = 0.f, sumsq = 0.f;
-#pragma unroll
-    for (int i = 0; i < kRowCluster * 2; ++i) { sum += part[i].x; sumsq += part[i].y; }
-    mean = sum * (1.0f / kE);
-    rstd = rsqrtf(fmaxf(sumsq * (1.0f / kE) - mean * mean, 0.f) + ep.eps);
-  };
-  if (is_epi) {
-    if (ew < 4) {
-      s_gain_mid[threadIdx.x - 64] = __ldg(ep.gain_mid + coff + (threadIdx.x - 64));
-      s_gain_out[threadIdx.x - 64] = __ldg(ep.gain_out + coff + (threadIdx.x - 64));
-    }
-    if (row < M) {
-#pragma unroll
-      for (int q = 0; q < kRowCols / 4; ++q) {
-        const float4 t = *reinterpret_cast<const float4*>(ep.x + xblk_off(row, (c0 >> 2) + q));
-        r[q * 4] = t.x; r[q * 4 + 1] = t.y; r[q * 4 + 2] = t.z; r[q * 4 + 3] = t.w;
-      }
-    } else {
-#pragma unroll
-      for (int i = 0; i < kRowCols; ++i) r[i] = 0.f;
-    }
-    mbar_wait(tmem_full0, 0, 3);
-    if (threadIdx.x == 64) trace_point(tr, 2);
-    tc_fence_after_sync();
-    add_acc_and_stats(0);
-    if (threadIdx.x == 64) trace_point(tr, 3);
-  }
-  __syncthreads();          // s_gain visible to all epilogue warps
-  cluster_sync_all();       // #1: LN2 partials visible; every CTA's phase-A MMAs have completed (their accumulators were read)
-  if (threadIdx.x == 64) trace_point(tr, 4);
-
-  // ---- LN2 rows of this CTA's 128 columns -> the two k-block tiles of ITS FFN1 operand (ring slots 0 and 1); nothing leaves the CTA
-  if (is_epi) {
-    float mean = 0.f, rstd = 0.f;
-    if (row < M) gather_stats(mean, rstd);
-    const int kb = half;                                                     // this thread's 64 columns = one row of that k-block
-    uint8_t* arow = ring + kb * kABytes + row_in_tile * 128;
-#pragma unroll
-    for (int q = 0; q < kRowCols / 8; ++q) {
-      float y[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) y[i] = (r[q * 8 + i] - mean) * rstd * s_gain_mid[half * kRowCols + q * 8 + i];
-      *reinterpret_cast<uint4*>(arow + ((q ^ (row_in_tile & 7)) << 4)) =
-          make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
-    }
-    fence_proxy_async_smem();      // generic-proxy writes -> visible to the async proxy (the bulk copies and this CTA's own MMAs)
-    if (threadIdx.x == 64) trace_point(tr, 5);
-  }
-  __syncthreads();
-  if (threadIdx.x == 64) trace_point(tr, 6);
-
-  // ---- phase B: partial products of ALL 128 hidden columns over this CTA's 128 columns of K (acc1 -> TMEM columns [128, 256))
-  if (warp == 1) {
-    if (elect_one()) {
-      mbar_wait(w1_full, 0, 6);
-      tc_fence_after_sync();
-      const uint32_t sa = smem_u32(ring), sb = smem_u32(w1_smem);
-#pragma unroll
-      for (int kb = 0; kb < 2; ++kb)
-#pragma unroll
-        for (int k = 0; k < kBlockK / kUmmaK; ++k)
-          umma_bf16_ss(tmem_base + 128, umma_desc_sw128_kmajor(sa + kb * kABytes + k * (kUmmaK * 2)),
-                       umma_desc_sw128_kmajor(sb + kb * kBBytes + k * (kUmmaK * 2)), kIdesc, (kb | k) != 0 ? 1u : 0u);
-      umma_commit(tmem_full1);
-    }
-  }
-  __syncwarp();
-  // reduce-scatter of the partial sums: the 32 hidden columns that CTA p owns go to p (16 KB per peer: [128 rows][32 floats], 16-byte units
-  // XOR-swizzled by the row); a thread stages the columns of destinations 2 * half and 2 * half + 1
-  uint8_t* send_buf = ring + 2 * kABytes;                       // [3][16 KB]: slot d - 1 holds the block for peer (rank + d) % 4
-  uint8_t* recv_buf = ring + 5 * kABytes;                       // [3][16 KB]: slot d - 1 receives the block of source (rank - d) % 4
-  if (is_epi) {
-    mbar_wait(tmem_full1, 0, 7);
-    if (threadIdx.x == 64) trace_point(tr, 7);
-    tc_fence_after_sync();
-#pragma unroll
-    for (int dd = 0; dd < 2; ++dd) {
-      const uint32_t dest = 2 * half + dd;
-      if (dest != crank) {
-        float pv[32];
-        tmem_ld_32x32(tmem_lane + 128 + dest * kHSplit, pv);
-        uint8_t* prow = send_buf + (((dest - crank) & 3u) - 1u) * kPartBytes + row_in_tile * 128;
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          *reinterpret_cast<float4*>(prow + ((q ^ (row_in_tile & 7)) << 4)) = make_float4(pv[q * 4], pv[q * 4 + 1], pv[q * 4 + 2], pv[q * 4 + 3]);
-      }
-    }
-    fence_proxy_async_smem();
-  }
-  __syncthreads();
-  if (warp == 0) {
-    if (elect_one()) {
-#pragma unroll
-      for (uint32_t d = 1; d < kRowCluster; ++d) {
-        const uint32_t pr = (crank + d) % kRowCluster;
-        dsmem_bulk_copy(dsmem_addr(recv_buf + (d - 1) * kPartBytes, pr), send_buf + (d - 1) * kPartBytes, kPartBytes, dsmem_addr(pq_full, pr));
-      }
-    }
-  }
-  __syncwarp();
-  if (threadIdx.x == 64) trace_point(tr, 15);
-  if (is_epi) {
-    // this thread's 16 hidden columns: the four partial sums added in the order of the source rank (the same in every kernel variant)
-    float own[16], v[16];
-    tmem_ld_32x16(tmem_lane + 128 + crank * kHSplit + half * 16, own);
-    mbar_wait(pq_full, 0, 5);
-#pragma unroll
-    for (uint32_t src = 0; src < kRowCluster; ++src) {
-      float t[16];
-      if (src == crank) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) t[j] = own[j];
-      } else {
-        const uint8_t* prow = recv_buf + (((crank - src) & 3u) - 1u) * kPartBytes + row_in_tile * 128;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float4 f = *reinterpret_cast<const float4*>(prow + (((half * 4 + q) ^ (row_in_tile & 7)) << 4));
-          t[q * 4] = f.x; t[q * 4 + 1] = f.y; t[q * 4 + 2] = f.z; t[q * 4 + 3] = f.w;
-        }
-      }
-#pragma unroll
-      for (int j = 0; j < 16; ++j) v[j] = src == 0 ? t[j] : v[j] + t[j];
-    }
-#pragma unroll
-    for (int j = 0; j < 16; ++j) v[j] = gelu_fast(v[j]);
-    // hidden-column exchange: the h region holds four 8 KB slices [source CTA][128 rows][64 B]; this thread's 16 columns go into the
-    // local slice, which one thread then pushes to the peers with bulk copies (per-thread st.shared::cluster stores: 4.2 k cycles)
-    uint4* mine = reinterpret_cast<uint4*>(h_smem + static_cast<int>(crank) * kHSlice + row_in_tile * 64 + half * 32);
-#pragma unroll
-    for (int q = 0; q < 2; ++q)
-      mine[q] = make_uint4(pack_bf16x2(v[q * 8 + 0], v[q * 8 + 1]), pack_bf16x2(v[q * 8 + 2], v[q * 8 + 3]),
-                           pack_bf16x2(v[q * 8 + 4], v[q * 8 + 5]), pack_bf16x2(v[q * 8 + 6], v[q * 8 + 7]));
-    fence_proxy_async_smem();
-  }
-  __syncthreads();
-  if (warp == 0) {
-    if (elect_one()) {
-      const uint8_t* src = h_smem + static_cast<int>(crank) * kHSlice;
-#pragma unroll
-      for (uint32_t d = 1; d < kRowCluster; ++d) {
-        const uint32_t pr = (crank + d) % kRowCluster;
-        dsmem_bulk_copy(dsmem_addr(src, pr), src, kHSlice, dsmem_addr(hx_full, pr));
-      }
-    }
-  }
-  __syncwarp();
-  if (threadIdx.x == 64) trace_point(tr, 8);
-  if (is_epi) {
-    // assemble the K-major swizzled A operand of FFN2 in the (now dead) W1 region: this thread's row, k-block `half` = the slices of
-    // source CTAs 2 * half and 2 * half + 1
-    mbar_wait(hx_full, 0, 10);
-    uint8_t* hrow = w1_smem + half * kABytes + row_in_tile * 128;
-#pragma unroll
-    for (int sidx = 0; sidx < 2; ++sidx) {
-      const uint4* src = reinterpret_cast<const uint4*>(h_smem + (2 * half + sidx) * kHSlice + row_in_tile * 64);
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const int chunk = sidx * 4 + c;
-        *reinterpret_cast<uint4*>(hrow + ((chunk ^ (row_in_tile & 7)) << 4)) = src[c];
-      }
-    }
-    fence_proxy_async_smem();
-    tc_fence_before_sync();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(hop_ready);
-  }
-  if (threadIdx.x == 64) trace_point(tr, 9);
-
-  // ---- phase C: second feed-forward GEMM, residual, LayerNorm
-  if (warp == 1) {
-    if (elect_one()) {
-      mbar_wait(hop_ready, 0, 11);
-      mbar_wait(w2_full, 0, 8);
-      tc_fence_after_sync();
-      const uint32_t sa = smem_u32(w1_smem), sb = smem_u32(w2_smem);
-#pragma unroll
-      for (int kb = 0; kb < kFfnDim / kBlockK; ++kb)
-#pragma unroll
-        for (int k = 0; k < kBlockK / kUmmaK; ++k)
-          umma_bf16_ss(tmem_base + 256, umma_desc_sw128_kmajor(sa + kb * kABytes + k * (kUmmaK * 2)),
-                       umma_desc_sw128_kmajor(sb + kb * kBBytes + k * (kUmmaK * 2)), kIdesc, (kb | k) != 0 ? 1u : 0u);
-      umma_commit(tmem_full2);
-    }
-  }
-  __syncwarp();
-  if (is_epi) {
-    mbar_wait(tmem_full2, 0, 9);     // FFN2 has read W2: its first 2 KB hold the second round of statistics
-    if (threadIdx.x == 64) trace_point(tr, 10);
-    tc_fence_after_sync();
-    s_stats = reinterpret_cast<float2*>(w2_smem);
-    add_acc_and_stats(256);
-    if (threadIdx.x == 64) trace_point(tr, 11);
-  }
-  __syncwarp();
-  cluster_sync_all();       // #4
-  if (threadIdx.x == 64) trace_point(tr, 12);
   if (is_epi) {
     float mean = 0.f, rstd = 0.f;
     s_stats = reinterpret_cast<float2*>(w2_smem);
@@ -2080,370 +1533,6 @@ outproj_ffn_ks_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_
   cluster_sync_relaxed();   // peers may still be reading this CTA's statistics / operand tiles
   if (threadIdx.x == 0) trace_point(tr, 14);
   if (warp == 1) tmem_dealloc<512>(tmem_base);
-}
-
-
-// ---------------------------------------------------------------------------------------------------------
-// The same block on 64-ROW tiles with TWO CTAs resident per SM (decode path, default; NOVIC_BLOCK_ROWS=128 restores the kernel above).
-// The kernel above is one serial chain per CTA - loads -> MMA -> statistics -> hand-over -> MMA -> GELU -> hand-over -> MMA ->
-// statistics -> stores, about 30 k cycles of which the tensor core works 3 k - and at 4096 rows there is exactly one 128-row tile per
-// cluster, so nothing overlaps anything.  Halving the tile doubles the clusters (256 CTAs for 4096 rows) and fits two CTAs on an SM
-// (<= 113 KB of shared memory, 256 TMEM columns, <= 170 registers x 192 threads each): one CTA's waits are the other's work.
-//   * UMMA keeps M = 128: rows 64..127 of every A operand are whatever follows the 64-row tile in shared memory (always inside the
-//     allocation); their accumulator lanes 64..127 are never read.  Rows 0..63 <-> TMEM lanes 0..63, so the four epilogue warps
-//     are the ones whose (warp % 4) is 0 or 1: warps 0, 1, 4, 5; warp 2 issues the loads and bulk copies, warp 3 the MMAs.
-//   * every operand arrives through 3-D tensor maps, two or more k-block tiles per request (the TMA unit serves ~2 requests at a time
-//     whatever their size, and two CTAs share it): 4 x 16 KB of rows + 4 x 32 KB of Wo + W1 and W2 in one 32 KB request each
-//   * shared memory: [X 64 KB | HS 16 KB | W1 32 KB].  X + HS + the first half of W1 are the two 48 KB stages (2 x (A 8 KB) + 2 x (Wo 16 KB)) of
-//     the out-proj pipeline (W1 is requested when its MMAs have completed), then X is the FFN1 A operand (8 k-block tiles of 64 rows: own two written locally, six by the peers' bulk
-//     copies), then - once this CTA's FFN1 MMAs have completed - W2 (32 KB, loaded late: it lands while GELU and the hidden-column
-//     exchange run), the second round of LayerNorm partials and the bf16 output staging.  HS receives the four 4 KB hidden slices
-//     (its first KB holds the first round of partials before that); W1 becomes the FFN2 A operand.  Accumulators: out-proj and FFN2
-//     share TMEM columns 0..127, FFN1 uses 128..159.  The LayerNorm gains are read with warp-uniform loads (no shared copy).
-// Same operands and accumulation order as the 128-row kernel: results are bit-identical.
-// ---------------------------------------------------------------------------------------------------------
-constexpr int kHbRows = 64;
-constexpr int kHbThreads = 192;
-constexpr int kHbABytes = kHbRows * kBlockK * 2;                 // 8 KB: one k-block of a 64-row A tile
-constexpr int kHbKbs = 2;                                        // k-blocks per request and stage (3-D tensor maps)
-constexpr int kHbStageBytes = kHbKbs * (kHbABytes + kBBytes);    // 48 KB: [A: 2 x 8 KB][Wo: 2 x 16 KB]
-constexpr int kHbStages = 2;
-constexpr int kHbXBytes = (kE / kBlockK) * kHbABytes;            // 64 KB
-constexpr int kHbHsBytes = kRowCluster * kHbRows * 64;           // 16 KB
-constexpr int kHbW1Bytes = (kFfnDim / kRowCluster) * kE * 2;     // 32 KB
-constexpr int kHbBarBytes = 256;
-__host__ __device__ constexpr int outproj_ffn64_smem_bytes() { return kHbXBytes + kHbHsBytes + kHbW1Bytes + kHbBarBytes + 768 /*alignment slack*/; }
-static_assert(outproj_ffn64_smem_bytes() <= 113 * 1024, "two CTAs of the 64-row block kernel must fit on an SM");
-static_assert(kHbStages * kHbStageBytes <= kHbXBytes + kHbHsBytes + kHbW1Bytes, "the out-proj stages fill X, HS and half of the W1 region");
-
-__global__ void __cluster_dims__(kRowCluster, 1, 1) __launch_bounds__(kHbThreads, 2)
-outproj_ffn64_kernel(const __grid_constant__ CUtensorMap tmap_ao, const __grid_constant__ CUtensorMap tmap_wo, const __grid_constant__ CUtensorMap tmap_w1q,
-                     const __grid_constant__ CUtensorMap tmap_w2, int M, FusedBlockParams ep) {
-  constexpr int BN = kRowBN;
-  constexpr int kHSplit = kFfnDim / kRowCluster;              // 32 hidden columns per CTA
-  constexpr int kW1kb = kHSplit * kBlockK * 2;                // 4 KB
-  constexpr uint32_t kIdesc = umma_idesc_bf16_f32(kBlockM, BN);
-  constexpr uint32_t kIdescH = umma_idesc_bf16_f32(kBlockM, kHSplit);
-  constexpr int kNkb = kE / kBlockK;                          // 8
-  constexpr int kHSlice = kHbRows * kHSplit * 2;              // one CTA's hidden columns: 64 rows x 64 B = 4 KB
-  constexpr uint32_t kTmem = 256;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* xop = smem;
-  uint8_t* hs = xop + kHbXBytes;
-  uint8_t* w1_smem = hs + kHbHsBytes;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(w1_smem + kHbW1Bytes);
-  uint64_t* empty_bar = full_bar + kHbStages;
-  uint64_t* tmem_full0 = empty_bar + kHbStages;
-  uint64_t* w1_full = tmem_full0 + 1;
-  uint64_t* w2_full = tmem_full0 + 2;
-  uint64_t* tmem_full1 = tmem_full0 + 3;
-  uint64_t* tmem_full2 = tmem_full0 + 4;
-  uint64_t* affn_full = tmem_full0 + 5;
-  uint64_t* hx_full = tmem_full0 + 6;
-  uint64_t* hop_ready = tmem_full0 + 7;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full0 + 8);
-  static_assert((2 * kHbStages + 8) * 8 + 4 <= kHbBarBytes, "barrier area");
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = static_cast<int>(lane_id());
-  const int m0 = blockIdx.y * kHbRows;
-  const uint32_t crank = cluster_ctarank();
-  const int coff = static_cast<int>(crank) * BN;
-  const int n0 = coff;
-  pdl_trigger();
-  if (threadIdx.x == 0 && static_cast<int>(smem - smem_raw) > 768) {   // the slack covers a base that is not 1 KB aligned by at most this much
-    printf("outproj_ffn64_kernel: dynamic shared memory base %u leaves no room for the 1 KB alignment\n", smem_u32(smem_raw));
-    __trap();
-  }
-
-  if (warp == 2) {
-    if (elect_one()) {
-      tma_prefetch_desc(&tmap_ao); tma_prefetch_desc(&tmap_wo); tma_prefetch_desc(&tmap_w1q); tma_prefetch_desc(&tmap_w2);
-      for (int st = 0; st < kHbStages; ++st) { mbar_init(&full_bar[st], 1); mbar_init(&empty_bar[st], 1); }
-      mbar_init(tmem_full0, 1); mbar_init(w1_full, 1); mbar_init(w2_full, 1); mbar_init(tmem_full1, 1); mbar_init(tmem_full2, 1);
-      mbar_init(affn_full, 1); mbar_init(hx_full, 1); mbar_init(hop_ready, 4);
-      fence_mbar_init();
-      mbar_arrive_expect_tx(affn_full, (kRowCluster - 1) * 2 * kHbABytes);   // the peers' copies can only start after cluster barrier #1
-      mbar_arrive_expect_tx(hx_full, (kRowCluster - 1) * kHSlice);
-      // the weights do not depend on the previous kernel: the first Wo tiles before the wait, the activation tiles after it
-      for (int i = 0; i < kHbStages; ++i) {
-        mbar_arrive_expect_tx(&full_bar[i], kHbStageBytes);
-        tma_load_3d(xop + i * kHbStageBytes + kHbKbs * kHbABytes, &tmap_wo, &full_bar[i], n0, i * kHbKbs, kEvictLast);
-      }
-      pdl_wait();
-      for (int i = 0; i < kHbStages; ++i)
-        tma_load_3d(xop + i * kHbStageBytes, &tmap_ao, &full_bar[i], m0, i * kHbKbs, kEvictNormal);
-    }
-  } else if (warp == 3) {
-    tmem_alloc<kTmem>(tmem_slot);
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-
-  if (warp == 2) {
-    if (elect_one()) {
-      for (int i = kHbStages; i < kNkb / kHbKbs; ++i) {
-        const int st = i % kHbStages;
-        mbar_wait(&empty_bar[st], ((i / kHbStages) & 1) ^ 1, 1);
-        mbar_arrive_expect_tx(&full_bar[st], kHbStageBytes);
-        tma_load_3d(xop + st * kHbStageBytes, &tmap_ao, &full_bar[st], m0, i * kHbKbs, kEvictNormal);
-        tma_load_3d(xop + st * kHbStageBytes + kHbKbs * kHbABytes, &tmap_wo, &full_bar[st], n0, i * kHbKbs, kEvictLast);
-      }
-      // the W1 slice (one request) goes into its region once the out-proj MMAs have read the stage that overlaps it
-      mbar_wait(tmem_full0, 0, 1);
-      mbar_arrive_expect_tx(w1_full, kNkb * kW1kb);
-      tma_load_3d(w1_smem, &tmap_w1q, w1_full, static_cast<int>(crank) * kHSplit, 0, kEvictLast);
-    }
-  } else if (warp == 3) {
-    if (elect_one()) {
-      for (int i = 0; i < kNkb / kHbKbs; ++i) {
-        const int st = i % kHbStages;
-        mbar_wait(&full_bar[st], (i / kHbStages) & 1, 2);
-        tc_fence_after_sync();
-        const uint32_t sa = smem_u32(xop + st * kHbStageBytes), sb = sa + kHbKbs * kHbABytes;
-#pragma unroll
-        for (int j = 0; j < kHbKbs; ++j)
-#pragma unroll
-          for (int k = 0; k < kBlockK / kUmmaK; ++k)
-            umma_bf16_ss(tmem_base, umma_desc_sw128_kmajor(sa + j * kHbABytes + k * (kUmmaK * 2)),
-                         umma_desc_sw128_kmajor(sb + j * kBBytes + k * (kUmmaK * 2)), kIdesc, (i | j | k) != 0 ? 1u : 0u);
-        umma_commit(&empty_bar[st]);
-      }
-      umma_commit(tmem_full0);                                  // acc0 -> TMEM columns [0, 128)
-    }
-  }
-  __syncwarp();
-
-  // ---- phase A epilogue: residual + accumulator, LN2 statistics
-  const bool is_epi = (warp & 2) == 0;                          // warps 0, 1, 4, 5: TMEM lane quadrants 0 and 1
-  const int quad = warp & 3;
-  const int half = warp >> 2;
-  const int row_in_tile = quad * 32 + lane;
-  const int row = m0 + row_in_tile;
-  const int c0 = coff + half * kRowCols;
-  const uint32_t tmem_lane = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
-  float2* s_stats = reinterpret_cast<float2*>(hs);              // [2 halves][64 rows]
-  float r[kRowCols];
-  auto add_acc_and_stats = [&]() {
-    float sum = 0.f, sumsq = 0.f;
-#pragma unroll
-    for (int c = 0; c < kRowCols / 16; ++c) {
-      float v[16];
-      tmem_ld_32x16(tmem_lane + half * kRowCols + c * 16, v);
-#pragma unroll
-      for (int j = 0; j < 16; ++j) {
-        const float t = r[c * 16 + j] + v[j];
-        r[c * 16 + j] = t;
-        sum += t;
-        sumsq = fmaf(t, t, sumsq);
-      }
-    }
-    s_stats[half * kHbRows + row_in_tile] = make_float2(sum, sumsq);
-  };
-  auto gather_stats = [&](float& mean, float& rstd) {
-    float2 part[kRowCluster * 2];
-#pragma unroll
-    for (uint32_t pr = 0; pr < kRowCluster; ++pr) {
-#pragma unroll
-      for (int hh = 0; hh < 2; ++hh) part[pr * 2 + hh] = dsmem_ld_f32x2_addr(dsmem_addr(&s_stats[hh * kHbRows + row_in_tile], pr));
-    }
-    float sum = 0.f, sumsq = 0.f;
-#pragma unroll
-    for (int i = 0; i < kRowCluster * 2; ++i) { sum += part[i].x; sumsq += part[i].y; }
-    mean = sum * (1.0f / kE);
-    rstd = rsqrtf(fmaxf(sumsq * (1.0f / kE) - mean * mean, 0.f) + ep.eps);
-  };
-  if (is_epi) {
-    if (row < M) {
-#pragma unroll
-      for (int q = 0; q < kRowCols / 4; ++q) {
-        const float4 t = *reinterpret_cast<const float4*>(ep.x + xblk_off(row, (c0 >> 2) + q));
-        r[q * 4] = t.x; r[q * 4 + 1] = t.y; r[q * 4 + 2] = t.z; r[q * 4 + 3] = t.w;
-      }
-    } else {
-#pragma unroll
-      for (int i = 0; i < kRowCols; ++i) r[i] = 0.f;
-    }
-    mbar_wait(tmem_full0, 0, 3);
-    tc_fence_after_sync();
-    add_acc_and_stats();
-  }
-  tc_fence_before_sync();
-  __syncwarp();
-  cluster_sync_all();       // #1: LN2 partials visible; every CTA's out-proj MMAs have completed (their accumulators were read)
-
-  // ---- hand-over: LN2 rows -> FFN1 operand of all four CTAs (local write of the CTA's two k-block tiles, one bulk copy per peer)
-  if (is_epi) {
-    float mean = 0.f, rstd = 0.f;
-    if (row < M) gather_stats(mean, rstd);
-    const int kb = static_cast<int>(crank) * 2 + half;
-    uint8_t* arow = xop + kb * kHbABytes + row_in_tile * 128;
-    const float* gm = ep.gain_mid + c0;
-#pragma unroll
-    for (int q = 0; q < kRowCols / 8; ++q) {
-      float y[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) y[i] = (r[q * 8 + i] - mean) * rstd * __ldg(gm + q * 8 + i);
-      *reinterpret_cast<uint4*>(arow + ((q ^ (row_in_tile & 7)) << 4)) =
-          make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
-    }
-    fence_proxy_async_smem();
-  }
-  __syncthreads();
-  if (warp == 2) {
-    if (elect_one()) {
-      const uint8_t* src = xop + static_cast<int>(crank) * 2 * kHbABytes;
-#pragma unroll
-      for (uint32_t d = 1; d < kRowCluster; ++d) {
-        const uint32_t pr = (crank + d) % kRowCluster;
-        dsmem_bulk_copy(dsmem_addr(src, pr), src, 2 * kHbABytes, dsmem_addr(affn_full, pr));
-      }
-      // W2 goes where the FFN1 operand lies, as soon as this CTA's FFN1 MMAs have read it
-      mbar_wait(tmem_full1, 0, 6);
-      mbar_arrive_expect_tx(w2_full, 2 * kBBytes);
-      tma_load_3d(xop, &tmap_w2, w2_full, n0, 0, kEvictLast);
-    }
-  } else if (warp == 3) {
-    // ---- phase B: this CTA's 32 hidden columns
-    if (elect_one()) {
-      mbar_wait(affn_full, 0, 5);
-      mbar_wait(w1_full, 0, 6);
-      tc_fence_after_sync();
-      const uint32_t sa = smem_u32(xop), sb = smem_u32(w1_smem);
-#pragma unroll
-      for (int kb = 0; kb < kNkb; ++kb)
-#pragma unroll
-        for (int k = 0; k < kBlockK / kUmmaK; ++k)
-          umma_bf16_ss(tmem_base + 128, umma_desc_sw128_kmajor(sa + kb * kHbABytes + k * (kUmmaK * 2)),
-                       umma_desc_sw128_kmajor(sb + kb * kW1kb + k * (kUmmaK * 2)), kIdescH, (kb | k) != 0 ? 1u : 0u);
-      umma_commit(tmem_full1);
-    }
-  }
-  __syncwarp();
-  if (is_epi) {
-    mbar_wait(tmem_full1, 0, 7);
-    tc_fence_after_sync();
-    float v[16];
-    tmem_ld_32x16(tmem_lane + 128 + half * 16, v);
-#pragma unroll
-    for (int j = 0; j < 16; ++j) v[j] = gelu_fast(v[j]);
-    // hidden-column exchange: HS holds four 4 KB slices [source CTA][64 rows][64 B]; the local one is written here and pushed to the peers
-    uint4* mine = reinterpret_cast<uint4*>(hs + static_cast<int>(crank) * kHSlice + row_in_tile * 64 + half * 32);
-#pragma unroll
-    for (int q = 0; q < 2; ++q)
-      mine[q] = make_uint4(pack_bf16x2(v[q * 8 + 0], v[q * 8 + 1]), pack_bf16x2(v[q * 8 + 2], v[q * 8 + 3]),
-                           pack_bf16x2(v[q * 8 + 4], v[q * 8 + 5]), pack_bf16x2(v[q * 8 + 6], v[q * 8 + 7]));
-    fence_proxy_async_smem();
-  }
-  __syncthreads();
-  if (warp == 2) {
-    if (elect_one()) {
-      const uint8_t* src = hs + static_cast<int>(crank) * kHSlice;
-#pragma unroll
-      for (uint32_t d = 1; d < kRowCluster; ++d) {
-        const uint32_t pr = (crank + d) % kRowCluster;
-        dsmem_bulk_copy(dsmem_addr(src, pr), src, kHSlice, dsmem_addr(hx_full, pr));
-      }
-    }
-  }
-  __syncwarp();
-  if (is_epi) {
-    // assemble the K-major swizzled A operand of FFN2 in the (dead) W1 region: this thread's row, k-block `half` = the slices of source
-    // CTAs 2 * half and 2 * half + 1
-    mbar_wait(hx_full, 0, 10);
-    uint8_t* hrow = w1_smem + half * kHbABytes + row_in_tile * 128;
-#pragma unroll
-    for (int sidx = 0; sidx < 2; ++sidx) {
-      const uint4* src = reinterpret_cast<const uint4*>(hs + (2 * half + sidx) * kHSlice + row_in_tile * 64);
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const int chunk = sidx * 4 + c;
-        *reinterpret_cast<uint4*>(hrow + ((chunk ^ (row_in_tile & 7)) << 4)) = src[c];
-      }
-    }
-    fence_proxy_async_smem();
-    tc_fence_before_sync();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(hop_ready);
-  }
-
-  // ---- phase C: second feed-forward GEMM (accumulator columns 0..127 again), residual, LayerNorm
-  if (warp == 3) {
-    if (elect_one()) {
-      mbar_wait(hop_ready, 0, 11);
-      mbar_wait(w2_full, 0, 8);
-      tc_fence_after_sync();
-      const uint32_t sa = smem_u32(w1_smem), sb = smem_u32(xop);
-#pragma unroll
-      for (int kb = 0; kb < kFfnDim / kBlockK; ++kb)
-#pragma unroll
-        for (int k = 0; k < kBlockK / kUmmaK; ++k)
-          umma_bf16_ss(tmem_base, umma_desc_sw128_kmajor(sa + kb * kHbABytes + k * (kUmmaK * 2)),
-                       umma_desc_sw128_kmajor(sb + kb * kBBytes + k * (kUmmaK * 2)), kIdesc, (kb | k) != 0 ? 1u : 0u);
-      umma_commit(tmem_full2);
-    }
-  }
-  __syncwarp();
-  s_stats = reinterpret_cast<float2*>(xop + 2 * kBBytes);      // second round of partials: behind W2 (the FFN1 operand is dead)
-  if (is_epi) {
-    mbar_wait(tmem_full2, 0, 9);
-    tc_fence_after_sync();
-    add_acc_and_stats();
-  }
-  tc_fence_before_sync();
-  __syncwarp();
-  cluster_sync_all();       // #2
-  if (is_epi) {
-    float mean = 0.f, rstd = 0.f;
-    if (row < M) gather_stats(mean, rstd);
-    const int ew = half * 2 + quad;
-    uint8_t* stage = xop + 2 * kBBytes + 2048 + ew * (32 * kRowStagePitch);
-    {
-      uint4* d = reinterpret_cast<uint4*>(stage + lane * kRowStagePitch);
-      const float* go = ep.gain_out + c0;
-#pragma unroll
-      for (int q = 0; q < kRowCols / 8; ++q) {
-        float y[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) y[i] = (r[q * 8 + i] - mean) * rstd * __ldg(go + q * 8 + i);
-        d[q] = make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
-      }
-    }
-    if (row < M) {
-#pragma unroll
-      for (int q = 0; q < kRowCols / 4; ++q)
-        *reinterpret_cast<float4*>(ep.x + xblk_off(row, (c0 >> 2) + q)) = make_float4(r[q * 4], r[q * 4 + 1], r[q * 4 + 2], r[q * 4 + 3]);
-    }
-    __syncwarp();
-    const int warp_row0 = m0 + quad * 32;
-    const int sub = lane >> 3, chunk = lane & 7;
-#pragma unroll 4
-    for (int i = 0; i < 8; ++i) {
-      const int rr = i * 4 + sub;
-      const int grow = warp_row0 + rr;
-      if (grow < M) {
-        int nrow = grow;
-        bool keep = true;
-        if (ep.remap_rows_in > 0) {
-          const int seq = grow / ep.remap_rows_in;
-          const int k = grow - seq * ep.remap_rows_in;
-          keep = k >= ep.remap_skip;
-          nrow = seq * ep.remap_rows_out + (k - ep.remap_skip);
-        }
-        if (keep)
-          *reinterpret_cast<uint4*>(ep.xn + static_cast<size_t>(nrow) * kE + c0 + chunk * 8) =
-              *reinterpret_cast<const uint4*>(stage + rr * kRowStagePitch + chunk * 16);
-      }
-    }
-  }
-  tc_fence_before_sync();
-  __syncwarp();
-  cluster_sync_relaxed();   // peers may still be reading this CTA's partials
-  if (warp == 3) tmem_dealloc<kTmem>(tmem_base);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -2606,168 +1695,6 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
   __syncthreads();
   cluster_sync_all();       // the leader's MMAs have read the peer's shared memory; the peer's arrivals have landed in the leader
   if (warp == 1) tmem_dealloc2<kAccStages * kPairTileN>(tmem_base);
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Weight-stationary GEMM on CTA pairs (the decoder's QKV projection at large batch; NOVIC_QKV_WS=2).  The phase traces of gemm_ws_kernel
-// and of its multicast variants show the same cadence - a 128 x 128 x 512 tile every ~4.5 k cycles against 2.1 k cycles of MMA - whatever
-// the request size or the L2 traffic: a TMA request takes ~2.2 k cycles from "stage released" to "landed" when every SM pulls, so the
-// tile rate is (bytes in flight) / (round trip), and with the 128 KB weight tile resident only 64 KB of activations fit in flight.
-// A CTA pair (tcgen05.mma.cta_group::2, M = 256) needs only HALF of the weight tile per CTA (64 of its 128 rows: 64 KB), which leaves
-// room for FOUR 32 KB activation stages - twice the bytes in flight for the same 128 x 128 x 512 of MMA work per CTA and tile.
-//   pair p owns column tile p % n_tiles for the whole launch and walks the 256-row blocks p / n_tiles, + npairs / n_tiles, ...;
-//   CTA r of the pair loads rows [64 r, 64 r + 64) of the weight tile once (before griddepcontrol.wait) and streams its own 128 rows
-//   of every block; barrier protocol as in gemm2_kernel (byte counts on the leader's barriers, multicast commits, the peer's epilogue
-//   warps arrive on the leader's "drained" barrier through its cluster address).  Same accumulation order: bit-identical.
-// ---------------------------------------------------------------------------------------------------------
-constexpr int kWs2AStages = 4;
-constexpr int kWs2BKb = (kTileN / 2) * kBlockK * 2;        // one k-block of a CTA's weight half: 64 rows x 128 B = 8 KB
-__host__ __device__ constexpr int gemm_ws2_smem_bytes() { return kWsKb * kWs2BKb + kWs2AStages * kWsABytes + kEpiWarps * kEpiStageBytes + 1024 + 256; }
-
-template <class Epi>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGemmThreads, 1)
-gemm_ws2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b /* 64-row boxes */, int M, int n_tiles, int b_is_static,
-                typename Epi::Params ep) {
-  constexpr int NST = kWs2AStages;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* b_smem = smem;                                   // [8 k-blocks][64 rows x 128 B]
-  uint8_t* a_ring = b_smem + kWsKb * kWs2BKb;
-  uint8_t* epi_stage = a_ring + NST * kWsABytes;
-  uint64_t* b_full = reinterpret_cast<uint64_t*>(epi_stage + kEpiWarps * kEpiStageBytes);   // [4] used in the leader only
-  uint64_t* a_full = b_full + kWsKb / 2;                    // used in the leader only
-  uint64_t* a_empty = a_full + NST;
-  uint64_t* tmem_full_bar = a_empty + NST;
-  uint64_t* tmem_empty_bar = tmem_full_bar + kAccStages;    // used in the leader only: 2 x kEpiWarps arrivals
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty_bar + kAccStages);
-  static_assert((kWsKb / 2 + 2 * NST + 2 * kAccStages) * 8 + 4 <= 256, "barrier area");
-  __shared__ int s_trace;
-
-  const int warp = threadIdx.x >> 5;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int pair = blockIdx.x >> 1, npairs = gridDim.x >> 1;
-  const int m_tiles = (M + 2 * kBlockM - 1) / (2 * kBlockM);
-  const int nt = pair % n_tiles, g0 = pair / n_tiles, gstep = npairs / n_tiles;
-  const int n0 = nt * kTileN;
-  pdl_trigger();
-  if (threadIdx.x == 0) { s_trace = (leader && trace_begin()) ? 1 : 0; trace_point(s_trace != 0, 0); }
-
-  if (warp == 0) {
-    if (elect_one()) {
-      tma_prefetch_desc(&tmap_a);
-      tma_prefetch_desc(&tmap_b);
-      for (int j = 0; j < kWsKb / 2; ++j) mbar_init(&b_full[j], 1);
-      for (int s = 0; s < NST; ++s) { mbar_init(&a_full[s], 1); mbar_init(&a_empty[s], 1); }
-      for (int a = 0; a < kAccStages; ++a) { mbar_init(&tmem_full_bar[a], 1); mbar_init(&tmem_empty_bar[a], 2 * kEpiWarps); }
-      fence_mbar_init();
-    }
-  } else if (warp == 1) {
-    tmem_alloc2<kAccStages * kTileN>(tmem_slot);
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();       // the peer's barriers are initialised before anything arrives on them
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-  const bool tr = s_trace != 0;
-  const uint32_t leader_bfull0 = dsmem_addr(&b_full[0], 0);
-  const uint32_t leader_afull0 = dsmem_addr(&a_full[0], 0);
-
-  if (warp == 0) {
-    if (elect_one()) {
-      auto load_b = [&]() {
-        for (int j = 0; j < kWsKb / 2; ++j) {
-          if (leader) mbar_arrive_expect_tx(&b_full[j], 2 * 2 * kWs2BKb);
-          tma_load_3d_2sm(b_smem + j * 2 * kWs2BKb, &tmap_b, leader_bfull0 + j * 8, n0 + static_cast<int>(rank) * (kTileN / 2), 2 * j, kEvictLast);
-        }
-      };
-      if (b_is_static && g0 < m_tiles) load_b();
-      pdl_wait();
-      if (threadIdx.x == 0) trace_point(tr, 1);
-      if (!b_is_static && g0 < m_tiles) load_b();
-      int stage = 0; uint32_t phase = 0;
-      for (int rp = g0; rp < m_tiles; rp += gstep) {
-        const int m0 = rp * (2 * kBlockM) + static_cast<int>(rank) * kBlockM;
-        for (int j = 0; j < kWsKb / 2; ++j) {
-          mbar_wait(&a_empty[stage], phase ^ 1, 1);
-          if (leader) mbar_arrive_expect_tx(&a_full[stage], 2 * kWsABytes);
-          tma_load_3d_2sm(a_ring + stage * kWsABytes, &tmap_a, leader_afull0 + stage * 8, m0, 2 * j, kEvictNormal);
-          if (++stage == NST) { stage = 0; phase ^= 1; }
-        }
-      }
-      trace_point(tr, 3);
-    }
-  } else if (warp == 1) {
-    pdl_wait();
-    if (leader && elect_one()) {
-      constexpr uint32_t kIdesc = umma_idesc_bf16_f32(2 * kBlockM, kTileN);
-      int stage = 0; uint32_t phase = 0;
-      int i = 0;
-      for (int rp = g0; rp < m_tiles; rp += gstep, ++i) {
-        const int as = i & 1;
-        mbar_wait(&tmem_empty_bar[as], ((i >> 1) & 1) ^ 1, 9);   // both CTAs' epilogues have drained this accumulator stage
-        tc_fence_after_sync();
-        const uint32_t acc = tmem_base + as * kTileN;
-        for (int j = 0; j < kWsKb / 2; ++j) {
-          if (i == 0) mbar_wait(&b_full[j], 0, 4);
-          mbar_wait(&a_full[stage], phase, 2);
-          if (i == 0 && j == 0) trace_point(tr, 4);
-          tc_fence_after_sync();
-          const uint32_t sa = smem_u32(a_ring + stage * kWsABytes);
-          const uint32_t sb = smem_u32(b_smem + j * 2 * kWs2BKb);
-#pragma unroll
-          for (int jj = 0; jj < 2; ++jj)
-#pragma unroll
-            for (int k = 0; k < kBlockK / kUmmaK; ++k)
-              umma2_bf16_ss(acc, umma_desc_sw128_kmajor(sa + jj * kABytes + k * (kUmmaK * 2)),
-                            umma_desc_sw128_kmajor(sb + jj * kWs2BKb + k * (kUmmaK * 2)), kIdesc, (j | jj | k) != 0 ? 1u : 0u);
-          umma2_commit_mc(&a_empty[stage], 0x3);
-          if (++stage == NST) { stage = 0; phase ^= 1; }
-        }
-        umma2_commit_mc(&tmem_full_bar[as], 0x3);
-        if (i == 0) trace_point(tr, 5);
-      }
-    }
-    __syncwarp();
-  } else {
-    pdl_wait();
-    const int ew = warp - 2;
-    const int quad = warp & 3;
-    const int half = ew >> 2;
-    const int lane = static_cast<int>(lane_id());
-    const uint32_t leader_tmem_empty0 = dsmem_addr(&tmem_empty_bar[0], 0);
-    int i = 0;
-    for (int rp = g0; rp < m_tiles; rp += gstep, ++i) {
-      const int as = i & 1;
-      const int m0 = rp * (2 * kBlockM) + static_cast<int>(rank) * kBlockM;
-      mbar_wait(&tmem_full_bar[as], (i >> 1) & 1, 3);
-      if (i < 8 && threadIdx.x == 64) trace_point(tr, 16 + 2 * i);
-      tc_fence_after_sync();
-      EpiCtx c;
-      c.tmem_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + as * kTileN + half * (kTileN / 2);
-      c.warp_row0 = m0 + quad * 32;
-      c.row = c.warp_row0 + lane;
-      c.n0 = n0 + half * (kTileN / 2);
-      c.ncols = kTileN / 2;
-      c.M = M;
-      c.part = nt * 2 + half;
-      c.stage = epi_stage + ew * kEpiStageBytes;
-      const uint32_t rel = leader_tmem_empty0 + as * 8;
-      Epi::run(ep, c, [rel, lane]() {
-        tc_fence_before_sync();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(rel);
-      });
-      if (i < 8 && threadIdx.x == 64) trace_point(tr, 17 + 2 * i);
-    }
-  }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();       // the leader's MMAs have read the peer's shared memory; the peer's arrivals have landed in the leader
-  if (threadIdx.x == 0) trace_point(tr, 10);
-  if (warp == 1) tmem_dealloc2<kAccStages * kTileN>(tmem_base);
 }
 
 

@@ -122,7 +122,7 @@ struct AttnParams {
   const unsigned char* anc;     // optional [nseq, anc_ld]
   int nseq, nq, q0, smax, P, beams, slot_mul, prefix_bidir, keypad_ld, anc_ld;
   int early_loads;              // stream kernel: request chunks of older rows before griddepcontrol.wait
-  int stream_hint;              // stream kernel: K/V rows are requested with an evict-first L2 policy (NOVIC_ATTN_HINT)
+  int stream_hint;              // stream kernel: K/V rows are requested with an evict-first L2 policy (the decoder always sets it)
   DropCfg drop;                 // attention_tf_kernel<true> (training): dropout on the attention probabilities (thresh 0 = off)
   uint32_t drop_site;
   float scale_log2e;            // (1/sqrt(head_dim)) * log2(e)
@@ -136,85 +136,9 @@ __device__ __forceinline__ void bf16x8_to_f32(const uint4& u, float* f) {
   t = unpack_bf16x2(u.w); f[6] = t.x; f[7] = t.y;
 }
 
-__global__ void __launch_bounds__(kWarpsPerBlock * 32) attention_kernel(const AttnParams p) {
-  const int w = blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
-  if (w >= p.nseq * p.nq) return;
-  const int lane = lane_id();
-  const int a = w / p.nq;
-  const int qpos = p.q0 + (w - a * p.nq);
-  const int nkeys = (p.prefix_bidir && qpos < p.P) ? p.P : qpos + 1;
-  const int own_slot = a * p.slot_mul;
-  const int group0 = (own_slot / p.beams) * p.beams;
-
-  float qf[16];
-  {
-    const uint4* q4 = reinterpret_cast<const uint4*>(p.q + static_cast<size_t>(w) * kE) + lane * 2;
-    const uint4 u0 = __ldg(q4), u1 = __ldg(q4 + 1);
-    bf16x8_to_f32(u0, qf);
-    bf16x8_to_f32(u1, qf + 8);
-#pragma unroll
-    for (int i = 0; i < 16; ++i) qf[i] *= p.scale_log2e;
-  }
-  float m = -INFINITY, l = 0.f, acc[16];
-#pragma unroll
-  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
-
-  constexpr int UNR = 4;
-  for (int j0 = 0; j0 < nkeys; j0 += UNR) {
-    uint4 kr[UNR][2], vr[UNR][2];
-    bool valid[UNR];
-#pragma unroll
-    for (int u = 0; u < UNR; ++u) {
-      const int j = j0 + u;
-      valid[u] = j < nkeys;
-      if (valid[u] && p.keypad != nullptr && j > 0 && p.keypad[static_cast<size_t>(a) * p.keypad_ld + j]) valid[u] = false;
-      if (valid[u]) {
-        int slot;
-        if (j < p.P) slot = group0;
-        else if (p.anc != nullptr && j < qpos) slot = group0 + p.anc[static_cast<size_t>(a) * p.anc_ld + (j - p.P)];
-        else slot = own_slot;
-        const size_t off = (static_cast<size_t>(slot) * p.smax + j) * kE;
-        const uint4* k4 = reinterpret_cast<const uint4*>(p.kcache + off) + lane * 2;
-        const uint4* v4 = reinterpret_cast<const uint4*>(p.vcache + off) + lane * 2;
-        kr[u][0] = k4[0]; kr[u][1] = k4[1];
-        vr[u][0] = v4[0]; vr[u][1] = v4[1];
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < UNR; ++u) {
-      if (!valid[u]) continue;  // warp-uniform
-      float kf[16];
-      bf16x8_to_f32(kr[u][0], kf);
-      bf16x8_to_f32(kr[u][1], kf + 8);
-      float s = 0.f;
-#pragma unroll
-      for (int i = 0; i < 16; ++i) s = fmaf(qf[i], kf[i], s);
-      s += __shfl_xor_sync(0xffffffffu, s, 1);
-      s += __shfl_xor_sync(0xffffffffu, s, 2);
-      const float m_new = fmaxf(m, s);
-      const float corr = exp2f(m - m_new);
-      const float pj = exp2f(s - m_new);
-      l = l * corr + pj;
-      float vf[16];
-      bf16x8_to_f32(vr[u][0], vf);
-      bf16x8_to_f32(vr[u][1], vf + 8);
-#pragma unroll
-      for (int i = 0; i < 16; ++i) acc[i] = fmaf(acc[i], corr, pj * vf[i]);
-      m = m_new;
-    }
-  }
-  const float inv = 1.0f / l;
-  uint32_t o[8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i) o[i] = pack_bf16x2(acc[2 * i] * inv, acc[2 * i + 1] * inv);
-  uint4* d = reinterpret_cast<uint4*>(p.out + static_cast<size_t>(w) * kE) + lane * 2;
-  d[0] = make_uint4(o[0], o[1], o[2], o[3]);
-  d[1] = make_uint4(o[4], o[5], o[6], o[7]);
-}
-
 // ---------------------------------------------------------------------------------------------------------
-// Attention, bulk-async version (the one the decoder uses).  The kernel above keeps too few bytes in flight
-// (register-staged loads, 12 warps/SM): ncu showed 40 % of HBM peak.  Here a persistent CTA runs one producer warp
+// Attention, bulk-async version.  A warp-per-query kernel with register-staged loads (12 warps/SM; removed, see the history)
+// kept too few bytes in flight: ncu showed 40 % of HBM peak.  Here a persistent CTA runs one producer warp
 // that streams each sequence's K and V pages into a shared-memory ring with cp.async.bulk (TMA engine, no
 // registers, completion on an mbarrier) while 8 consumer warps compute from shared memory: up to ~190 KB per SM
 // are in flight at all times.  One ring stage = all the K rows then all the V rows one sequence needs
@@ -366,8 +290,7 @@ constexpr int kAsThreads = kAsWarps * 32;
 constexpr int kAsSmemBytes = kAsWarps * kAsSlots * kAsSlotBytes + kAsWarps * kAsSlots * 8 + 128;
 __host__ __device__ constexpr int as_smem_bytes(int warps, int slots, int chunk) { return warps * slots * chunk * 1024 + warps * slots * 8 + 128; }
 
-// WARPS x SLOTS x CHUNK KB of shared memory; the defaults are the configuration the decoder uses, the other instantiations
-// exist for tuning (NOVIC_ATTN_CFG).
+// WARPS x SLOTS x CHUNK KB of shared memory; the decoder instantiates <16, 3, 4> (other shapes were measured slower, DESIGN.md section 5).
 template <int WARPS, int SLOTS, int CHUNK>
 __global__ void __launch_bounds__(WARPS * 32, 1) attention_stream_kernel_t(const AttnParams p) {
   constexpr int kAsWarps = WARPS, kAsSlots = SLOTS, kAsChunk = CHUNK, kAsSlotBytes = CHUNK * 1024;

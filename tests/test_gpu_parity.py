@@ -352,103 +352,29 @@ def test_forward_without_targets_is_the_first_step(models):
 
 
 @pytest.mark.gpu
-def test_qkv_tail_of_the_block_kernel_is_bit_identical(monkeypatch):
-    """The next layer's QKV projection in the tail of the fused block kernel (opt-in, NOVIC_FUSE_QKV=1: measured slower than the
-    stand-alone launches, DESIGN.md section 5) against the stand-alone QKV GEMM launches (default): same operands, same accumulation
-    order -> bit-identical ids, scores, logits, for greedy (ragged batch: the last 128-row block is partial), beam search and the
-    teacher-forced forward.  The small graph-replayed batches are the regression case of the decode step's launch fence: with a
-    few CTAs per kernel a whole step's prologues fit on the GPU at once, and the attention kernel's early K/V requests read rows of
+def test_small_graph_replayed_decodes_match_direct_launches(monkeypatch):
+    """Greedy decodes of 1, 2, 5, 31 and 33 embeddings, each run twice under graph replay, against a handle that enqueues the same kernels
+    directly (NOVIC_NO_GRAPHS=1): bit-identical ids, padding and scores.  This is the regression case of the decode step's launch fence:
+    with a few CTAs per kernel a whole step's prologues fit on the GPU at once, and the attention kernel's early K/V requests read rows of
     the prefix pass before it had finished until select_greedy_kernel was made to wait before releasing its dependents."""
     dims = synth.DecoderDims()
     sd = weight_case("eos")
     embed = synth.synth_embeddings(300, seed=5).to(DEV)
-    tgt, pad = synth.synth_targets(40, dims, seed=3)
     outs = []
-    monkeypatch.setenv("NOVIC_FFN1_KSPLIT", "0")     # the tail lives in the block kernel that gathers the LN2 rows
-    monkeypatch.setenv("NOVIC_BLOCK_ROWS", "128")    # ... on 128-row tiles (the default row-owner kernel sums in another order)
-    for flag in ("0", "1"):                      # the switch is read when a handle is created
-        monkeypatch.setenv("NOVIC_FUSE_QKV", flag)
+    for flag in ("1", "0"):                      # the switch is read when a handle is created
+        monkeypatch.setenv("NOVIC_NO_GRAPHS", flag)
         m = default_decoder(dims, sd).to(DEV)
         with torch.inference_mode():
-            g = m.generate(embed, True, True, 0.9, 0.2, None, None, False)
-            b = m.generate_beam(embed[:64], 3, 1.0, 0.0, None, False, 0.0, None, False)
-            f = m(embed[:40], tgt.to(DEV), pad.to(DEV), None, True, True, False, None)
-            small = [m.generate(embed[:n], False, True, 1.0, 0.0, None, None, False) for n in (1, 2, 5, 31, 33) for _ in range(2)]
-        outs.append((g, b, f, small))
+            outs.append([m.generate(embed[:n], False, True, 1.0, 0.0, None, None, False) for n in (1, 2, 5, 31, 33) for _ in range(2)])
         del m
-    (g0, b0, f0, s0), (g1, b1, f1, s1) = outs
-    for a, c in zip(s0, s1):
+    for a, c in zip(*outs):
         assert torch.equal(a[0], c[0]) and torch.equal(a[1], c[1]) and torch.equal(a[5], c[5])
-    assert torch.equal(g0[0], g1[0]) and torch.equal(g0[1], g1[1]) and torch.equal(g0[2], g1[2]) and torch.equal(g0[5], g1[5])
-    assert torch.equal(b0[0], b1[0]) and torch.equal(b0[2], b1[2])
-    assert torch.equal(f0[0], f1[0]) and f0[2].item() == f1[2].item() and torch.equal(f0[4], f1[4])
-
-
-def test_block_kernel_on_64_row_tiles_is_bit_identical(monkeypatch):
-    """The fused out-proj + feed-forward block kernel on 64-row tiles (outproj_ffn64_kernel: what small row counts use, NOVIC_BLOCK_ROWS=64
-    forces it everywhere) against the 128-row kernel (NOVIC_BLOCK_ROWS=128): same operands and accumulation order -> bit-identical ids,
-    scores and logits for greedy (ragged: 300 = 4 x 64 + 44 rows per decode step, 1200 prefix rows), beam search and the
-    teacher-forced forward; and with two CTAs resident per SM (NOVIC_BLOCK64_PAD=0) as well."""
-    dims = synth.DecoderDims()
-    sd = weight_case("eos")
-    embed = synth.synth_embeddings(300, seed=5).to(DEV)
-    tgt, pad = synth.synth_targets(40, dims, seed=3)
-    outs = []
-    monkeypatch.setenv("NOVIC_FFN1_KSPLIT", "0")     # the 128-row kernel that gathers the LN2 rows, as the 64-row one does
-    for rows, extra in (("128", "16384"), ("64", "16384"), ("64", "0")):     # the switches are read when a handle is created
-        monkeypatch.setenv("NOVIC_BLOCK_ROWS", rows)
-        monkeypatch.setenv("NOVIC_BLOCK64_PAD", extra)
-        m = default_decoder(dims, sd).to(DEV)
-        with torch.inference_mode():
-            g = m.generate(embed, True, True, 0.9, 0.2, None, None, False)
-            b = m.generate_beam(embed[:64], 3, 1.0, 0.0, None, False, 0.0, None, False)
-            f = m(embed[:40], tgt.to(DEV), pad.to(DEV), None, True, True, False, None)
-            small = [m.generate(embed[:n], False, True, 1.0, 0.0, None, None, False) for n in (1, 63, 65)]
-        outs.append((g, b, f, small))
-        del m
-    g0, b0, f0, s0 = outs[0]
-    for g1, b1, f1, s1 in outs[1:]:
-        assert torch.equal(g0[0], g1[0]) and torch.equal(g0[1], g1[1]) and torch.equal(g0[2], g1[2]) and torch.equal(g0[5], g1[5])
-        assert torch.equal(b0[0], b1[0]) and torch.equal(b0[2], b1[2])
-        assert torch.equal(f0[0], f1[0]) and f0[2].item() == f1[2].item() and torch.equal(f0[4], f1[4])
-        for a, c in zip(s0, s1):
-            assert torch.equal(a[0], c[0]) and torch.equal(a[1], c[1]) and torch.equal(a[5], c[5])
-
-
-def test_block_kernel_with_k_split_ffn1_agrees_to_rounding(monkeypatch):
-    """The default 128-row block kernel (outproj_ffn_ks_kernel: every CTA multiplies its own 128 LN2 columns and the partial FFN1 sums are
-    reduce-scattered over the cluster) against the variant that gathers the whole LN2 row first (NOVIC_FFN1_KSPLIT=0).  The hidden
-    pre-activations are sums of four K = 128 partial products instead of one K = 512 accumulation, so the two agree to fp32 rounding before
-    the bf16 casts and to a few bf16 flips after six layers: teacher-forced logits within 0.01 (measured: max 3.4e-3, mean 2e-4 at a
-    logit rms of 0.18; the tolerance against the reference is 0.06), greedy ids identical on >= 98 % of the rows (a row may leave
-    the other variant's trajectory only at a near-tie)."""
-    dims = synth.DecoderDims()
-    sd = weight_case("lively")
-    embed = synth.synth_embeddings(2048, seed=5).to(DEV)       # 2048 rows per decode step: above the 64-row kernel's range
-    tgt, pad = synth.synth_targets(160, dims, seed=3)
-    outs = []
-    for flag in ("0", "1"):
-        monkeypatch.setenv("NOVIC_FFN1_KSPLIT", flag)
-        monkeypatch.setenv("NOVIC_BLOCK_ROWS", "128")
-        m = default_decoder(dims, sd).to(DEV)
-        with torch.inference_mode():
-            f = m(embed[:160], tgt.to(DEV), pad.to(DEV), None, True, True, False, None)
-            g = m.generate(embed, False, True, 1.0, 0.0, None, None, False)
-        outs.append((f[0].float().cpu(), g[0].cpu()))
-        del m
-    (f0, g0), (f1, g1) = outs
-    valid = ~pad
-    assert (f0 - f1)[valid].abs().max().item() <= 0.01
-    n = min(g0.shape[1], g1.shape[1])
-    same = (g0[:, :n] == g1[:, :n]).all(dim=1).float().mean().item()
-    print(f"rows with identical greedy ids: {same:.4f}")
-    assert same >= 0.98
 
 
 def test_row_owner_block_kernel_agrees_with_the_cluster_kernel_to_rounding(monkeypatch):
     """The default block kernel (block_rows_kernel: one CTA per 32 rows, the weights streamed as the M operand of the MMAs, LayerNorm
     statistics summed over TMEM lanes instead of over a thread's registers) against the 128-row cluster kernel that gathers the whole
-    LN2 row (NOVIC_BLOCK_ROWS=128, NOVIC_FFN1_KSPLIT=0).  Same products, K = 512 accumulated in one chain in both; the statistics are
+    LN2 row (outproj_ffn_kernel, NOVIC_BLOCK_ROWS=128).  Same products, K = 512 accumulated in one chain in both; the statistics are
     summed in a different order, so the two agree to fp32 rounding before the bf16 casts and to a few bf16 flips after six layers:
     teacher-forced logits within 0.01 (tolerance against the reference: 0.06), greedy ids identical on >= 98 % of the rows.  Ragged row
     counts: 2049 rows per decode step (64 full 32-row blocks + one row), 8196 prefix rows, 160 x 16 teacher-forced rows with the row
@@ -461,7 +387,6 @@ def test_row_owner_block_kernel_agrees_with_the_cluster_kernel_to_rounding(monke
     tgt, pad = synth.synth_targets(160, dims, seed=3)
     outs = []
     for rows, min64 in (("128", "0"), ("32", "0"), ("32", "1")):     # cluster kernel; 32 rows per CTA everywhere; 64 rows per CTA everywhere
-        monkeypatch.setenv("NOVIC_FFN1_KSPLIT", "0")
         monkeypatch.setenv("NOVIC_BLOCK_ROWS", rows)
         monkeypatch.setenv("NOVIC_BLOCK_ROWS64_MIN", min64)
         m = default_decoder(dims, sd).to(DEV)
@@ -483,33 +408,6 @@ def test_row_owner_block_kernel_agrees_with_the_cluster_kernel_to_rounding(monke
         for (t0, l0), (t1, l1) in zip(s0, s1):
             assert (l0[:, 0] - l1[:, 0]).abs().max().item() <= 0.01          # first step: same inputs, no trajectory effects
             assert torch.equal(t0[:, 0], t1[:, 0]) or (l0[:, 0].topk(2, dim=-1).values.diff(dim=-1).abs().min().item() <= 0.02)
-
-
-def test_attention_inside_the_block_kernel_is_bit_identical(monkeypatch):
-    """NOVIC_FUSE_ATTN=1: the decode-step attention of a CTA's 32 sequences runs on the epilogue warps of the row-owner block kernel
-    (block_rows_kernel<true>, K / V staged in two slots of the weight ring, the attention row written straight into the resident MMA
-    operand) instead of as a launch of its own.  Same arithmetic in the same order -> bit-identical ids, padding, scores and step
-    logits for greedy (ragged: 301 rows = 9 blocks + 13 rows, so some warps own one sequence and some none), beam search (ancestry
-    tables, per-row K / V requests) and guided decoding keeps working on the unfused kernels of its masked passes."""
-    dims = synth.DecoderDims()
-    sd = weight_case("eos")
-    embed = synth.synth_embeddings(301, seed=5).to(DEV)
-    outs = []
-    monkeypatch.setenv("NOVIC_ATTN_SPLIT", "0")  # small batches otherwise use attention_split_kernel, which sums the keys in another order
-    for flag in ("0", "1"):                      # the switch is read when a handle is created
-        monkeypatch.setenv("NOVIC_FUSE_ATTN", flag)
-        m = default_decoder(dims, sd).to(DEV)
-        with torch.inference_mode():
-            g = m.generate(embed, True, True, 0.9, 0.2, None, None, False)
-            b = m.generate_beam(embed[:70], 3, 1.0, 0.0, None, False, 0.0, None, False)
-            small = [m.generate(embed[:n], False, True, 1.0, 0.0, None, None, False) for n in (1, 17, 33)]
-        outs.append((g, b, small))
-        del m
-    (g0, b0, s0), (g1, b1, s1) = outs
-    assert torch.equal(g0[0], g1[0]) and torch.equal(g0[1], g1[1]) and torch.equal(g0[2], g1[2]) and torch.equal(g0[5], g1[5])
-    assert torch.equal(b0[0], b1[0]) and torch.equal(b0[1], b1[1]) and torch.equal(b0[2], b1[2])
-    for a, c in zip(s0, s1):
-        assert torch.equal(a[0], c[0]) and torch.equal(a[1], c[1]) and torch.equal(a[5], c[5])
 
 
 def test_beam_logits_on_wide_tiles_are_bit_identical(monkeypatch):
@@ -539,19 +437,15 @@ def test_beam_logits_on_wide_tiles_are_bit_identical(monkeypatch):
 
 
 def test_qkv_projection_variants_are_bit_identical(monkeypatch):
-    """The QKV projection of a large decode step (>= 24 row blocks) has five implementations with the same operands and accumulation order:
-    the generic persistent kernel (NOVIC_QKV_WS=0), the weight-stationary kernel (default), its cluster-multicast variants
-    (NOVIC_QKV_MC=2 / 4: activation stages requested once per cluster) and the weight-stationary CTA-pair kernel (NOVIC_QKV_WS=2,
-    tcgen05.mma.cta_group::2).  3100 embeddings = 24 full row blocks + a ragged one of 28 rows (the pair kernel's last pair has an empty
-    second CTA).  Ids, padding and scores must be bit-identical."""
+    """The QKV projection of a decode step has two implementations with the same operands and accumulation order: the generic persistent
+    kernel (NOVIC_QKV_WS=0) and the weight-stationary kernel (default).  3100 embeddings = 24 full row blocks + a ragged one of 28 rows.
+    Ids, padding and scores must be bit-identical."""
     dims = synth.DecoderDims()
     sd = weight_case("lively")
     embed = synth.synth_embeddings(3100, seed=8).to(DEV)
     outs = []
-    for ws, mc, st in (("0", "0", "2"), ("1", "0", "2"), ("1", "2", "2"), ("1", "4", "2"), ("2", "0", "2"), ("1", "0", "3")):     # the switches are read when a handle is created
+    for ws in ("0", "1"):                        # the switch is read when a handle is created
         monkeypatch.setenv("NOVIC_QKV_WS", ws)
-        monkeypatch.setenv("NOVIC_QKV_MC", mc)
-        monkeypatch.setenv("NOVIC_QKV_WS_STAGES", st)     # 3: a third activation stage instead of the staging tile, q / K / V stored with 256-bit stores
         m = default_decoder(dims, sd).to(DEV)
         with torch.inference_mode():
             g = m.generate(embed, False, True, 0.9, 0.2, None, None, False)

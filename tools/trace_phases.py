@@ -16,11 +16,9 @@ with torch.inference_mode():
     st = model._state(torch.device("cuda:0"))
     _abi.check(lib.novic_set_use_graphs(st["handle"], 0))
     model.generate(e, False, True, 1.0, 0.0, None, None, False)
-    # GEMM launches of a 1-layer greedy decode: prefix, qkv, block, logits (prefill), then qkv, block, logits per step.  With
-    # NOVIC_FUSE_BLOCK=0 the block is two row kernels (out-proj, FFN) and the ordinals are 5, 6, 7, 8 (tools/trace_fused.py traces the fused one).
-    fused = os.environ.get("NOVIC_FUSE_BLOCK", "1") != "0"
-    kinds = {4: "qkv (decode, M=4096)", 6: "logits (decode)"} if fused else \
-            {5: "qkv (decode, M=4096)", 6: "out-proj rowln (decode)", 7: "fused FFN rowln (decode)", 8: "logits (decode)"}
+    # GEMM launches of a 1-layer greedy decode: prefix, qkv, block, logits (prefill), then qkv, block, logits per step (the block kernels have
+    # their own tools: trace_fused.py, trace_blockrows.py)
+    kinds = {4: "qkv (decode, M=4096)", 6: "logits (decode)"}
     for target, label in kinds.items():
         _abi.check(lib.novic_debug_trace(None, 1 + target))
         model.generate(e, False, True, 1.0, 0.0, None, None, False)
